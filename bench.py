@@ -2,14 +2,16 @@
 """bench.py -- RTjpeg 720x576 YUV420 decoded frames/s on B200 (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W]              # this repo's CUDA path
-    python bench.py --impl reference [--gpus N] [--steps K] ...       # the reference's CPU decoder
+    python bench.py --impl reference [--gpus N] [--steps K] ...       # the reference's CPU decoder (oracle/_ref)
+    python bench.py --dump-outputs DIR ...                            # + what the last timed step decoded, as .npy
     torchrun --nproc-per-node N ... bench.py --gpus N ...             # one rank per GPU
 
 A "step" is one pass of the hot path (K1 scan -> K3 resolve -> K2 idct -> K2b hard blocks) over one batch of
 4096 synthetic 720x576 frames (BASELINE.json configs[1]: intra-only, Q=128).  The batch is produced once, outside
-every timed region, by the reference's own RTjpeg_compress (oracle/_ref, as north_star prescribes for the synthetic
-streams) from the seeded source in oracle/ref_driver.c.  The headline is weak scaling: every rank decodes its own
-4096-frame batch (its own seed); batches are independent, there is no data-path collective.
+every timed region, by RTjpeg_compress as oracle/ restates it (tests/golden/ pins it to the reference's own packets,
+byte for byte) from the seeded source in oracle/rtjo_driver.c: the same arguments give the same batch.  The headline
+is weak scaling: every rank decodes its own 4096-frame batch (its own seed); batches are independent, there is no
+data-path collective.
 
 value     whole-job frames/s, packets and descriptors already resident in HBM, frames left in HBM; the library's
           default arrangement (rtjgpu_set_pipeline AUTO: the scan of one slice of frames beside resolve + IDCT of the
@@ -25,7 +27,10 @@ other_configs   the parity configs of BASELINE.json (inter GOP 30 at two masks, 
 config5   BASELINE.json configs[4]: ONE inter-coded 1920x1088 stream, cut at clean frames on the host
           (rtjgpu_split_shards_lead over the headers' key hints, verified with K1's skip counts), every shard decoded
           by its rank's GPU, frames left there.  Strong scaling: the stream is the same at every N.
-cpu_baseline  the unmodified reference decoder (oracle/_ref) on this box's host cores.
+cpu_baseline  the unmodified reference decoder (oracle/_ref) on this box's host cores; left out where it is not built
+          (oracle/Makefile `ref` compiles it from the reference's sources, which the repository does not hold).
+--dump-outputs DIR  after the timed steps, what the last of them left in HBM: frames.npy, a fixed seeded sample of 16
+          decoded frames (float32, frame_index.npy says which), and frame_sums.npy, the byte sum of every frame (float64).
 """
 import argparse
 import json
@@ -50,7 +55,7 @@ C5_W, C5_H, C5_Q, C5_GOP, C5_FRAMES = 1920, 1088, 128, 30, 960
 
 
 def make_workload(frames: int, seed: int, w=W, h=H, q=QUALITY, **kw):
-    """Synthetic clip -> packets by the reference compressor (not timed)."""
+    """Synthetic clip -> packets by the restated compressor (not timed)."""
     from oracle import oracle as O
     kw.setdefault("noise_y", 2)
     kw.setdefault("noise_c", 0)
@@ -68,7 +73,7 @@ def config_dict(payload_per_frame: float, frames: int) -> dict:
         "payload_bytes_per_frame": payload_per_frame, "planar_bytes_per_frame": fsz,
         "l2": "inputs larger than L2: every step reads %.0f MB and writes %.0f MB"
               % (payload_per_frame * frames / 1e6, frames * fsz / 1e6),
-        "stream_source": "reference RTjpeg_compress on a seeded synthetic clip (untimed)",
+        "stream_source": "RTjpeg_compress (restated, the reference's packets byte for byte) on a seeded synthetic clip (untimed)",
     }
 
 
@@ -368,11 +373,11 @@ def run_config5(torch, dist, g, D, rank, world, local, steps, peak):
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms_step = float(t.item()) / steps
-    # bit-exactness of this rank's shard on its last GOP, against the reference decoding that GOP on the host
+    # bit-exactness of this rank's shard on its last GOP, against the oracle decoding that GOP on the host
     g0 = max(k for k in range(int(first[rank]), b_end) if hint[k]) if b_end > int(first[rank]) else b_end
     ok = True
     if b_end > g0:
-        want = O.ref_decode_seq(stream, offsets[g0:b_end + 1], w, h, keep_all=False)
+        want = O.decode_stream(stream, offsets[g0:b_end + 1], w, h, keep_all=False)
         ok = bool(np.array_equal(bt.out[b_end - a - 1].cpu().numpy(), want))
     okt = torch.tensor([1 if ok and verified else 0], dtype=torch.int64, device="cuda")
     if world > 1:
@@ -394,7 +399,7 @@ def run_config5(torch, dist, g, D, rank, world, local, steps, peak):
         "gpu_launches_this_rank": launches,
         "collectives_in_data_path": 0,
     }
-    if rank == 0:
+    if rank == 0 and O.have_ref():
         threads = host_threads()
         gops = list(range(0, F, C5_GOP)) + [F]
         sample = min(F, 240)
@@ -420,7 +425,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-other-configs", action="store_true")
     ap.add_argument("--no-config5", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step decoded to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -435,6 +443,7 @@ def main():
 
     import gmerlin_avdecoder_b200 as g
     from gmerlin_avdecoder_b200 import device as D
+    from oracle import oracle as O
 
     if not torch.cuda.is_available():
         raise SystemExit("bench.py: no CUDA device -- the decoder has no CPU path")
@@ -467,6 +476,8 @@ def main():
     assert info.bad_frames == 0
     ms, launches = time_steps(torch, D, ctx, batch, args.steps, barrier)
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, batch.out)
 
     t_ms = torch.tensor([ms], dtype=torch.float64, device="cuda")
     if world > 1:
@@ -552,7 +563,7 @@ def main():
                 },
             },
         }
-        if world == 1 and not args.no_cpu_baseline:
+        if world == 1 and not args.no_cpu_baseline and O.have_ref():
             threads = host_threads()
             sample = min(F, args.cpu_sample)
             reference_decode_fps(stream, offsets, sample, threads, 2)             # warm the threads and the caches
@@ -595,6 +606,20 @@ def main():
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
+
+
+def dump_outputs(out_dir: str, frames) -> None:
+    """What a caller of the device path receives, the decoded frames [F, w*h*3/2] in HBM, sampled to 16 frames chosen by a
+    fixed seed (40 MB as float32) plus the byte sum of every frame, so that two builds can be compared output for output."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    F = frames.shape[0]
+    idx = np.sort(np.random.default_rng(0).choice(F, size=min(F, 16), replace=False))
+    np.save(os.path.join(out_dir, "frame_index.npy"), idx.astype(np.float64))
+    np.save(os.path.join(out_dir, "frames.npy"), frames[torch.from_numpy(idx).to(frames.device)].cpu().numpy().astype(np.float32))
+    # a few frames at a time: the int64 sum of the whole batch at once would need a temporary of 8 bytes per pixel
+    sums = torch.cat([frames[i:i + 64].sum(dim=1, dtype=torch.int64) for i in range(0, F, 64)])
+    np.save(os.path.join(out_dir, "frame_sums.npy"), sums.cpu().numpy().astype(np.float64))
 
 
 def _emit(line: dict) -> None:

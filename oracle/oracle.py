@@ -2,7 +2,8 @@
 
 Two libraries live behind this module:
 
-* ``oracle/liboracle.so``      -- the plain-C restatement (oracle/rtjpeg_oracle.c);
+* ``oracle/liboracle.so``      -- the plain-C restatement (oracle/rtjpeg_oracle.c) and what drives it:
+  the seeded synthetic clips, their streams and threaded decode (oracle/rtjo_driver.c);
 * ``oracle/_ref/librtjref.so`` -- the UNMODIFIED reference (``lib/RTjpeg.c`` compiled
   from /root/reference by ``oracle/Makefile``) plus ``oracle/ref_driver.c``.
 
@@ -83,6 +84,15 @@ def oracle_lib():
         L.rtjo_unpack_block.argtypes = [_u8p, C.c_int, _i32p, C.POINTER(C.c_int16)]
         L.rtjo_unpack_block.restype = C.c_int
         L.rtjo_idct_block.argtypes = [C.POINTER(C.c_int16), _u8p, C.c_int]
+        L.rtjo_synth_frame.argtypes = [C.c_int, C.c_int, C.c_int, C.c_uint32, C.c_int, C.c_int, C.c_int,
+                                       _u8p, _u8p, _u8p]
+        L.rtjo_packet_bound.argtypes = [C.c_int, C.c_int]
+        L.rtjo_packet_bound.restype = C.c_size_t
+        L.rtjo_encode_clip.argtypes = [C.POINTER(Clip), C.c_int, C.c_int, _u8p, C.c_size_t, _u64p, C.c_int]
+        L.rtjo_encode_clip.restype = C.c_size_t
+        L.rtjo_decode_threaded.argtypes = [_u8p, _u64p, C.POINTER(C.c_int), C.c_int, C.c_int, C.c_int, C.c_int,
+                                           C.c_int, _u8p, _u32p]
+        L.rtjo_decode_threaded.restype = C.c_int
         _oracle = L
     return _oracle
 
@@ -173,7 +183,7 @@ def idct_block(blk: np.ndarray) -> np.ndarray:
 # --------------------------------------------------------------------------
 
 class Clip(C.Structure):
-    """Mirror of refdrv_clip (oracle/ref_driver.c)."""
+    """Mirror of rtjo_clip (oracle/rtjo_driver.c) and refdrv_clip (oracle/ref_driver.c)."""
     _fields_ = [("w", C.c_int), ("h", C.c_int), ("Q", C.c_int), ("key_rate", C.c_int),
                 ("lm", C.c_int), ("cm", C.c_int), ("noise_y", C.c_int), ("noise_c", C.c_int),
                 ("dark", C.c_int), ("seed", C.c_uint32)]
@@ -196,14 +206,10 @@ def ref_lib():
                 raise FileNotFoundError(
                     f"{REF_SO} missing and {REFERENCE_ROOT} absent: build it where the reference is mounted")
         L = C.CDLL(REF_SO)
-        L.refdrv_synth_frame.argtypes = [C.c_int, C.c_int, C.c_int, C.c_uint32, C.c_int, C.c_int, C.c_int,
-                                         _u8p, _u8p, _u8p]
         L.refdrv_packet_bound.argtypes = [C.c_int, C.c_int]
         L.refdrv_packet_bound.restype = C.c_size_t
         L.refdrv_encode_frames.argtypes = [C.POINTER(Clip), _u8p, C.c_int, _u8p, C.c_size_t, _u64p, C.c_int]
         L.refdrv_encode_frames.restype = C.c_size_t
-        L.refdrv_encode_clip.argtypes = [C.POINTER(Clip), C.c_int, C.c_int, _u8p, C.c_size_t, _u64p, C.c_int]
-        L.refdrv_encode_clip.restype = C.c_size_t
         L.refdrv_decode_seq.argtypes = [_u8p, _u64p, C.c_int, C.c_int, C.c_int, _u8p, _u8p, _u8p]
         L.refdrv_encode_frames_fmt.argtypes = [C.POINTER(Clip), C.c_int, _u8p, C.c_int, _u8p, C.c_size_t, _u64p, C.c_int]
         L.refdrv_encode_frames_fmt.restype = C.c_size_t
@@ -222,26 +228,27 @@ def ref_lib():
 
 def synth_frame(w, h, t, seed=1, noise_y=2, noise_c=0, dark=0) -> np.ndarray:
     out = np.empty(w * h * 3 // 2, dtype=np.uint8)
-    ref_lib().refdrv_synth_frame(w, h, t, seed, noise_y, noise_c, dark, _ptr(out),
-                                 C.cast(out.ctypes.data + w * h, _u8p),
-                                 C.cast(out.ctypes.data + w * h * 5 // 4, _u8p))
+    oracle_lib().rtjo_synth_frame(w, h, t, seed, noise_y, noise_c, dark, _ptr(out),
+                                  C.cast(out.ctypes.data + w * h, _u8p),
+                                  C.cast(out.ctypes.data + w * h * 5 // 4, _u8p))
     return out
 
 
 def encode_clip(clip: Clip, F: int, threads: int = 0, align: int = 16):
-    """Synthesize and encode F frames with the reference encoder.
+    """Synthesize and encode F frames with the restated encoder (oracle/rtjo_driver.c), which
+    tests/golden/ pins to the reference's own packets.
 
     Returns (stream uint8[...], offsets uint64[F+1]); packet f is
     stream[offsets[f]:offsets[f]+framesize]; every start is `align`-aligned."""
-    L = ref_lib()
+    L = oracle_lib()
     threads = threads or (os.cpu_count() or 1)
-    cap = int(L.refdrv_packet_bound(clip.w, clip.h) + align) * F + 64
+    cap = int(L.rtjo_packet_bound(clip.w, clip.h) + align) * F + 64
     # worst-case capacity can be large (64 B/block); fall back to a generous typical bound first
     typical = max(1 << 20, (clip.w * clip.h * 3 // 2 + 4096) * F)
     for c in (min(cap, typical), cap):
         buf = np.zeros(c, dtype=np.uint8)
         offs = np.empty(F + 1, dtype=np.uint64)
-        used = L.refdrv_encode_clip(C.byref(clip), F, threads, _ptr(buf), c, _ptr(offs, _u64p), align)
+        used = L.rtjo_encode_clip(C.byref(clip), F, threads, _ptr(buf), c, _ptr(offs, _u64p), align)
         if used or F == 0:
             return buf[:int(used)].copy(), offs
     raise RuntimeError("encode buffer too small")
@@ -259,6 +266,20 @@ def encode_frames(clip: Clip, frames: np.ndarray, align: int = 16):
     if not used and F:
         raise RuntimeError("encode buffer too small")
     return buf[:int(used)].copy(), offs
+
+
+def ref_encode_clip(clip: Clip, F: int, align: int = 16):
+    """The clip of encode_clip coded by the reference's own RTjpeg_compress, one encoder in sequence: what the streams of
+    tests/golden/ are made with, so that they pin the restated encoder to the reference."""
+    frames = np.stack([synth_frame(clip.w, clip.h, t, clip.seed, clip.noise_y, clip.noise_c, clip.dark) for t in range(F)])
+    return encode_frames(clip, frames, align)
+
+
+def ref_encode_clip_fmt(w: int, h: int, Q: int, F: int, fmt: int, key_rate: int = -1, lm: int = 0, cm: int = 0, **kw):
+    """encode_clip_fmt with the reference doing both the round trip of the source and the coding in format fmt."""
+    s, o = ref_encode_clip(make_clip(w, h, 255, **kw), F)
+    frames = frames_in_format(ref_decode_seq(s, o, w, h), w, h, fmt)
+    return encode_frames_fmt(make_clip(w, h, Q, key_rate, lm, cm), fmt, frames)
 
 
 def ref_decode_seq(stream, offsets, w, h, init=None, keep_all=True):
@@ -462,13 +483,15 @@ def decode_stream_fmt(stream, offsets, w: int, h: int, fmt: int, init: np.ndarra
 
 
 def encode_clip_fmt(w: int, h: int, Q: int, F: int, fmt: int, key_rate: int = -1, lm: int = 0, cm: int = 0, **kw):
-    """A synthetic clip in format fmt: the seeded YUV420 source of ref_driver.c (taken through one
-    high-quality reference round trip), reshaped by frames_in_format and coded by the reference's
-    own RTjpeg_compress in that format.  Returns (stream, offsets)."""
+    """A synthetic clip in format fmt: the seeded YUV420 source of rtjo_driver.c (taken through one
+    high-quality round trip), reshaped by frames_in_format and coded in that format by the restated
+    RTjpeg_compress.  Returns (stream, offsets)."""
     src = make_clip(w, h, 255, **kw)
     s, o = encode_clip(src, F, threads=1)
-    frames = frames_in_format(ref_decode_seq(s, o, w, h), w, h, fmt)
-    return encode_frames_fmt(make_clip(w, h, Q, key_rate, lm, cm), fmt, frames)
+    frames = frames_in_format(decode_stream(s, o, w, h), w, h, fmt)
+    if fmt == 2:
+        return encode_frames_grey(frames, w, h, Q, key_rate, lm)
+    return encode_frames_oracle(frames, w, h, fmt, Q, key_rate, lm, cm)
 
 
 # ---- colour converters (RTjpeg.c:3071-3486) ---------------------------------------------------
@@ -545,3 +568,62 @@ def encode_frames_oracle(frames: np.ndarray, w: int, h: int, fmt: int, Q: int, k
         pkts.append(tmp[:n].copy())
     L.rtjo_encoder_free(C.byref(e))
     return pack_packets(pkts, align)
+
+
+def encode_frames_grey(frames: np.ndarray, w: int, h: int, Q: int, key_rate: int = 0, lm: int = 0, align: int = 16):
+    """The reference's RTjpeg_compress in the 8-bit format over grey pictures [F, w*h] (rtjo_encode_frame8): it reads
+    every picture up to 56 rows past its end, which is the next picture or, behind the last one, zeros."""
+    L = oracle_lib()
+    L.rtjo_encoder_init.argtypes = [C.POINTER(_Encoder), C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int]
+    L.rtjo_encoder_free.argtypes = [C.POINTER(_Encoder)]
+    L.rtjo_encode_frame8.argtypes = [C.POINTER(_Encoder), C.c_void_p, _u8p]
+    L.rtjo_encode_frame8.restype = C.c_long
+    frames = _np_u8(frames)
+    F = frames.shape[0]
+    padded = np.zeros(frames.size + 64 * w, dtype=np.uint8)
+    padded[:frames.size] = frames.reshape(-1)
+    e = _Encoder()
+    L.rtjo_encoder_init(C.byref(e), 2, w, h, Q, max(key_rate, 0), lm, lm)
+    tmp = np.zeros(12 + (w // 8) * (h // 8) * 64 + 64, dtype=np.uint8)
+    pkts = []
+    for f in range(F):
+        n = L.rtjo_encode_frame8(C.byref(e), padded.ctypes.data + f * w * h, _ptr(tmp))
+        pkts.append(tmp[:n].copy())
+    L.rtjo_encoder_free(C.byref(e))
+    return pack_packets(pkts, align)
+
+
+def decode_threaded(stream, offsets, segments, w: int, h: int, threads: int = 0, zero_init: bool = True,
+                    raw_tables=None) -> np.ndarray:
+    """Restatement decode of independent frame ranges on `threads` workers (segments: first frame of each range, then
+    the frame count); returns [F, w*h*3/2].  raw_tables: 128 raw entries every worker's decoder starts with, as
+    RTjpeg_set_tables leaves them (the packets then carry quality 0)."""
+    stream = _np_u8(stream)
+    offsets = np.ascontiguousarray(offsets, dtype=np.uint64)
+    seg = np.ascontiguousarray(segments, dtype=np.int32)
+    F = int(seg[-1])
+    frames = np.empty((F, w * h * 3 // 2), dtype=np.uint8)
+    raw = None if raw_tables is None else np.ascontiguousarray(raw_tables, dtype=np.uint32)
+    rc = oracle_lib().rtjo_decode_threaded(_ptr(stream), _ptr(offsets, _u64p), seg.ctypes.data_as(C.POINTER(C.c_int)),
+                                           len(seg) - 1, w, h, threads or (os.cpu_count() or 1), 1 if zero_init else 0,
+                                           _ptr(frames), None if raw is None else _ptr(raw, _u32p))
+    if rc < 0:
+        raise ValueError("truncated packet")
+    return frames
+
+
+def decode_with_tables(raw, pkt, w: int, h: int, planes: np.ndarray) -> np.ndarray:
+    """Restatement decode of one packet on a fresh decoder given raw tables first (RTjpeg_set_tables: they stay in force
+    while the packet's quality byte is 0)."""
+    d = _Decoder()
+    oracle_lib().rtjo_decoder_reset(C.byref(d))
+    raw = np.ascontiguousarray(raw, dtype=np.uint32)
+    oracle_lib().rtjo_tables_from_raw(_ptr(raw, _u32p), C.byref(d.t))
+    d.width, d.height, d.Q = w, h, 0
+    pkt = _np_u8(pkt)
+    p = np.array(planes, dtype=np.uint8).copy()
+    n = oracle_lib().rtjo_decode_packet(C.byref(d), _ptr(pkt), pkt.size, _ptr(p), C.cast(p.ctypes.data + w * h, _u8p),
+                                        C.cast(p.ctypes.data + w * h * 5 // 4, _u8p))
+    if n < 0:
+        raise ValueError("truncated packet")
+    return p

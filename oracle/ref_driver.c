@@ -7,8 +7,7 @@
  * process as the drop-in library that exports the original names).
  *
  * It provides what the reference has no tool for (SURVEY.md section 4):
- *   - a seeded synthetic YUV420 source (SURVEY.md section 8d, configs 2-4),
- *   - stream production with the reference's own RTjpeg_compress (:3488),
+ *   - packets of caller-supplied pictures from the reference's own RTjpeg_compress (:3488),
  *   - sequential and threaded decode with the reference's RTjpeg_decompress
  *     (:3565) for parity checks and for the CPU baseline timing.
  * No reference source text is reproduced here; only its public API
@@ -33,59 +32,6 @@ extern int ref_RTjpeg_compress(RTjpeg_t *, uint8_t *, uint8_t **);
 extern void ref_RTjpeg_decompress(RTjpeg_t *, uint8_t *, uint8_t **);
 extern void ref_RTjpeg_get_tables(RTjpeg_t *, uint32_t *);
 extern void ref_RTjpeg_set_tables(RTjpeg_t *, uint32_t *);
-
-/* ------------------------------------------------------------------ */
-/* synthetic source                                                    */
-/* ------------------------------------------------------------------ */
-
-static inline uint32_t xs32(uint32_t *s)
-{
-    uint32_t x = *s;
-    x ^= x << 13; x ^= x >> 17; x ^= x << 5;
-    return *s = x;
-}
-
-static inline uint8_t clip_video(int v) { return (uint8_t)(v < 16 ? 16 : (v > 235 ? 235 : v)); }
-
-/*
- * Frame t of the synthetic clip into tight planes (Y w*h, U and V (w/2)*(h/2)).
- *   Y = 128 + 60 sin((x+3t) 0.05) cos(y 0.07) + checker(40 px, +-25, phase flips
- *       every 8 frames) + uniform noise in [-noise_y, +noise_y]
- *   U,V = smooth sinusoids around 128 (+ uniform noise in [-noise_c, +noise_c])
- * dark != 0 additionally paints the left third flat Y=16 (adversarial case:
- * "key" frames that still contain skip markers, SURVEY.md section 0-5).
- */
-void refdrv_synth_frame(int w, int h, int t, uint32_t seed, int noise_y, int noise_c,
-                        int dark, uint8_t *y, uint8_t *u, uint8_t *v)
-{
-    uint32_t rng = seed * 2654435761u + (uint32_t)t * 40503u + 1u;
-    if (!rng) rng = 1;
-    float *sx = (float *)malloc(sizeof(float) * (size_t)w);
-    for (int x = 0; x < w; x++) sx[x] = sinf((float)(x + 3 * t) * 0.05f);
-    int flip = (t >> 3) & 1;
-    for (int yy = 0; yy < h; yy++) {
-        float cy = 60.0f * cosf((float)yy * 0.07f);
-        for (int x = 0; x < w; x++) {
-            int chk = (((x / 40) + (yy / 40) + flip) & 1) ? 25 : -25;
-            int n = noise_y ? (int)(xs32(&rng) % (uint32_t)(2 * noise_y + 1)) - noise_y : 0;
-            int val = 128 + (int)lrintf(sx[x] * cy) + chk + n;
-            if (dark && x < w / 3) val = 16;
-            y[(size_t)yy * w + x] = clip_video(val);
-        }
-    }
-    int cw = w / 2, ch = h / 2;
-    for (int yy = 0; yy < ch; yy++) {
-        for (int x = 0; x < cw; x++) {
-            int nu = noise_c ? (int)(xs32(&rng) % (uint32_t)(2 * noise_c + 1)) - noise_c : 0;
-            int nv = noise_c ? (int)(xs32(&rng) % (uint32_t)(2 * noise_c + 1)) - noise_c : 0;
-            int uu = 128 + (int)lrintf(40.0f * sinf((float)(x + t) * 0.03f) * cosf((float)yy * 0.02f)) + nu;
-            int vv = 128 + (int)lrintf(40.0f * cosf((float)(x - 2 * t) * 0.025f) * sinf((float)yy * 0.035f)) + nv;
-            u[(size_t)yy * cw + x] = clip_video(uu);
-            v[(size_t)yy * cw + x] = clip_video(vv);
-        }
-    }
-    free(sx);
-}
 
 /* ------------------------------------------------------------------ */
 /* encode                                                              */
@@ -142,74 +88,6 @@ size_t refdrv_encode_frames(const refdrv_clip *c, const uint8_t *frames, int F,
     free(tmp);
     ref_RTjpeg_close(e);
     return at;
-}
-
-typedef struct {
-    const refdrv_clip *c;
-    int f0, f1;                 /* synthetic frame index range */
-    uint8_t **pkts;             /* per-frame malloc'd packets */
-    uint32_t *sizes;
-} enc_job;
-
-static void *enc_worker(void *arg)
-{
-    enc_job *j = (enc_job *)arg;
-    const refdrv_clip *c = j->c;
-    RTjpeg_t *e = make_encoder(c);
-    size_t ysz = (size_t)c->w * c->h;
-    uint8_t *frame = (uint8_t *)malloc(ysz * 3 / 2);
-    uint8_t *tmp = (uint8_t *)malloc(refdrv_packet_bound(c->w, c->h));
-    uint8_t *pl[3] = { frame, frame + ysz, frame + ysz * 5 / 4 };
-    for (int f = j->f0; f < j->f1; f++) {
-        refdrv_synth_frame(c->w, c->h, f, c->seed, c->noise_y, c->noise_c, c->dark, pl[0], pl[1], pl[2]);
-        int n = ref_RTjpeg_compress(e, tmp, pl);
-        j->pkts[f] = (uint8_t *)malloc((size_t)n);
-        memcpy(j->pkts[f], tmp, (size_t)n);
-        j->sizes[f] = (uint32_t)n;
-    }
-    free(tmp); free(frame);
-    ref_RTjpeg_close(e);
-    return NULL;
-}
-
-/*
- * Synthesize + encode F frames of the clip with `threads` workers.  Each
- * worker owns a private encoder and a contiguous frame range that starts on a
- * GOP boundary (multiple of key_rate+1), so the result is byte-identical to a
- * single sequential encoder (the encoder zeroes its reference at every key
- * frame, RTjpeg.c:3504-3505, and holds no other inter-frame state).
- * Same output convention as refdrv_encode_frames.
- */
-size_t refdrv_encode_clip(const refdrv_clip *c, int F, int threads,
-                          uint8_t *out, size_t cap, uint64_t *offsets, int align)
-{
-    if (threads < 1) threads = 1;
-    int gop = c->key_rate > 0 ? c->key_rate + 1 : 1;
-    int ngop = (F + gop - 1) / gop;
-    if (threads > ngop) threads = ngop;
-    uint8_t **pkts = (uint8_t **)calloc((size_t)F, sizeof(uint8_t *));
-    uint32_t *sizes = (uint32_t *)calloc((size_t)F, sizeof(uint32_t));
-    enc_job *jobs = (enc_job *)calloc((size_t)threads, sizeof(enc_job));
-    pthread_t *th = (pthread_t *)calloc((size_t)threads, sizeof(pthread_t));
-    for (int i = 0; i < threads; i++) {
-        int g0 = (int)((long)ngop * i / threads), g1 = (int)((long)ngop * (i + 1) / threads);
-        jobs[i].c = c; jobs[i].f0 = g0 * gop; jobs[i].f1 = g1 * gop > F ? F : g1 * gop;
-        jobs[i].pkts = pkts; jobs[i].sizes = sizes;
-        pthread_create(&th[i], NULL, enc_worker, &jobs[i]);
-    }
-    for (int i = 0; i < threads; i++) pthread_join(th[i], NULL);
-    size_t at = 0;
-    int ok = 1;
-    for (int f = 0; f < F; f++) {
-        at = (at + (size_t)align - 1) / (size_t)align * (size_t)align;
-        if (ok && at + sizes[f] <= cap) memcpy(out + at, pkts[f], sizes[f]); else ok = 0;
-        offsets[f] = at;
-        at += sizes[f];
-        free(pkts[f]);
-    }
-    offsets[F] = at;
-    free(pkts); free(sizes); free(jobs); free(th);
-    return ok ? at : 0;
 }
 
 /* ------------------------------------------------------------------ */

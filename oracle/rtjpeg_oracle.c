@@ -547,9 +547,9 @@ void rtjo_encoder_free(rtjo_encoder *e) { free(e->old); e->old = NULL; }
 long rtjo_encode_frame(rtjo_encoder *e, const uint8_t *y, const uint8_t *u, const uint8_t *v, uint8_t *out)
 {
     const int w = e->width, h = e->height, cw = w >> 1, fmt = e->fmt;
-    /* The 8-bit branch of the reference is not restated: RTjpeg_compress8 / RTjpeg_mcompress8 hand RTjpeg_dctY the
-     * picture width where it expects width / 8 (:2627, :3005; dctY steps rows by rskip << 3, :337), so every block
-     * is read with a row stride of 8 * width -- outside the plane for most of the picture.  Undefined there. */
+    /* The 8-bit branch is rtjo_encode_frame8: RTjpeg_compress8 / RTjpeg_mcompress8 hand RTjpeg_dctY the picture
+     * width where it expects width / 8 (:2627, :3005; dctY steps rows by rskip << 3, :337), so every block is read
+     * with a row stride of 8 * width -- up to 56 rows past the plane, which a tight picture does not have. */
     if (fmt != 0 && fmt != 1) return -1;
     const int inter = e->key_rate != 0;
     if (inter && e->key_count == 0) memset(e->old, 0, (size_t)e->nblk * 64 * sizeof(int16_t));
@@ -586,6 +586,45 @@ long rtjo_encode_frame(rtjo_encoder *e, const uint8_t *y, const uint8_t *u, cons
                 if (skip) *sp++ = 0xFF;
                 else sp += rtjo_pack_block(blk, luma ? e->lb8 : e->cb8, sp);
             }
+    const long ds = (long)(sp - out);
+    out[0] = (uint8_t)ds; out[1] = (uint8_t)(ds >> 8); out[2] = (uint8_t)(ds >> 16); out[3] = (uint8_t)(ds >> 24);
+    out[4] = 12; out[5] = 0;
+    out[6] = (uint8_t)w; out[7] = (uint8_t)(w >> 8); out[8] = (uint8_t)h; out[9] = (uint8_t)(h >> 8);
+    out[10] = (uint8_t)e->Q;
+    out[11] = inter ? (uint8_t)e->key_count : 0;
+    if (inter && ++e->key_count > e->key_rate) e->key_count = 0;
+    return ds;
+}
+
+/* The 8-bit branch as the reference runs it (RTjpeg_compress8, RTjpeg_mcompress8), for a grey plane y that the caller
+ * follows with at least 56 * width readable bytes.  Both hand RTjpeg_dctY the picture width where it expects
+ * width / 8 (:2627, :3005), so every block is read with a row stride of 8 * width; RTjpeg_compress8 also steps one
+ * pixel row (not eight) from a row of blocks to the next, RTjpeg_mcompress8 eight.  What lies behind the plane goes
+ * into the packet: the same bytes there give the same packet.  Pinned by the grey fixtures of tests/golden/ on every
+ * picture whose reads stay inside the pictures that follow it there. */
+long rtjo_encode_frame8(rtjo_encoder *e, const uint8_t *y, uint8_t *out)
+{
+    const int w = e->width, h = e->height;
+    if (e->fmt != 2) return -1;
+    const int inter = e->key_rate != 0;
+    if (inter && e->key_count == 0) memset(e->old, 0, (size_t)e->nblk * 64 * sizeof(int16_t));
+    uint8_t *sp = out + 12;
+    int16_t blk[64];
+    int16_t *old = e->old;
+    for (int by = 0; by < (h >> 3); by++)
+        for (int bx = 0; bx < (w >> 3); bx++) {
+            rtjo_fdct_quant(y + (size_t)by * (inter ? 8 : 1) * w + bx * 8, 8 * w, e->lqt, blk);
+            int skip = 0;
+            if (inter) {
+                skip = 1;
+                for (int i = 0; i < 64; i++)
+                    if (abs(old[i] - blk[i]) > e->lmask) { skip = 0; break; }
+                if (!skip) memcpy(old, blk, sizeof(blk));
+                old += 64;
+            }
+            if (skip) *sp++ = 0xFF;
+            else sp += rtjo_pack_block(blk, e->lb8, sp);
+        }
     const long ds = (long)(sp - out);
     out[0] = (uint8_t)ds; out[1] = (uint8_t)(ds >> 8); out[2] = (uint8_t)(ds >> 16); out[3] = (uint8_t)(ds >> 24);
     out[4] = 12; out[5] = 0;

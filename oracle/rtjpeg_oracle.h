@@ -87,6 +87,8 @@ int  rtjo_pack_block(const int16_t blk[64], int bt8, uint8_t *out);
 void rtjo_encoder_init(rtjo_encoder *e, int fmt, int w, int h, int Q, int key_rate, int lm, int cm);
 void rtjo_encoder_free(rtjo_encoder *e);
 long rtjo_encode_frame(rtjo_encoder *e, const uint8_t *y, const uint8_t *u, const uint8_t *v, uint8_t *out);
+/* fmt 2 as the reference codes it, reading up to 56 rows behind the plane (see rtjpeg_oracle.c) */
+long rtjo_encode_frame8(rtjo_encoder *e, const uint8_t *y, uint8_t *out);
 
 /* Colour converters of RTjpeg.c:3071-3486 (RTjpeg_yuv420rgb32 ... RTjpeg_yuv422rgb24), see rtjpeg_oracle.c. */
 size_t rtjo_convert_bpp(int kind);

@@ -23,13 +23,3 @@ def _built():
         g.build_library()
     yield
 
-
-@pytest.fixture(autouse=True)
-def _gpu_tests_compare_with_the_compiled_reference(request):
-    """Every -m gpu test takes its expected output from oracle/_ref (the unmodified lib/RTjpeg.c compiled by
-    oracle/Makefile; it travels to the GPU box with the repository).  Without it tests/streams.py would fall back to
-    the restatement -- still pinned through the golden fixtures, but not what the parity claim says: fail loudly."""
-    if request.node.get_closest_marker("gpu"):
-        from oracle import oracle as O
-        assert O.have_ref(), "oracle/_ref/librtjref.so is missing: the GPU parity tests compare with the compiled reference itself"
-    yield

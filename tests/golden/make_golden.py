@@ -8,9 +8,11 @@ Run in the authoring container, where /root/reference is mounted:
 Every expected output in the fixtures comes from the reference's own
 RTjpeg_decompress (lib/RTjpeg.c:3565) / RTjpeg_set_quality+get_tables
 (:2408, :2371), compiled by oracle/Makefile into oracle/_ref/.  Streams come
-from the reference's own RTjpeg_compress (:3488) fed by the seeded synthetic
-source in oracle/ref_driver.c, or -- for the `random_*` cases -- from the
-grammar-only packet generator in oracle/oracle.py (no codec arithmetic).
+from the reference's own RTjpeg_compress (:3488, through oracle.ref_encode_clip
+and ref_encode_clip_fmt) fed by the seeded synthetic source in
+oracle/rtjo_driver.c, or -- for the `random_*` cases -- from the grammar-only
+packet generator in oracle/oracle.py (no codec arithmetic).  Never from the
+restated encoder: these streams are what pins it.
 The reference ships no fixtures of its own (SURVEY.md section 4); these files
 are the pin.
 """
@@ -34,7 +36,7 @@ def sha(a: np.ndarray) -> str:
 def clip_case(name, w, h, Q, F, key_rate=-1, lm=0, cm=0, noise_y=2, noise_c=0, dark=0, seed=1,
               init_fill=0, keep_planes=True):
     clip = O.make_clip(w, h, Q, key_rate, lm, cm, noise_y=noise_y, noise_c=noise_c, dark=dark, seed=seed)
-    stream, offs = O.encode_clip(clip, F, threads=1)
+    stream, offs = O.ref_encode_clip(clip, F)
     init = np.full(w * h * 3 // 2, init_fill, dtype=np.uint8)
     frames = O.ref_decode_seq(stream, offs, w, h, init=init)
     d = dict(stream=stream, offsets=offs, w=w, h=h, Q=Q, init_fill=init_fill,
@@ -121,7 +123,7 @@ def set_tables_case(seed=11):
 
 def fmt_case(name, fmt, w, h, Q, F, key_rate=-1, lm=0, cm=0, init_fill=0, **kw):
     """YUV422 (fmt 1) and 8-bit grey (fmt 2): the other two branches of RTjpeg_decompress (:3580-3585)."""
-    stream, offs = O.encode_clip_fmt(w, h, Q, F, fmt, key_rate, lm, cm, **kw)
+    stream, offs = O.ref_encode_clip_fmt(w, h, Q, F, fmt, key_rate, lm, cm, **kw)
     init = np.full(O.frame_bytes(fmt, w, h), init_fill, dtype=np.uint8)
     frames = O.ref_decode_seq_fmt(stream, offs, w, h, fmt, init=init)
     np.savez_compressed(os.path.join(OUT, name + ".npz"), stream=stream, offsets=offs, w=w, h=h, Q=Q, fmt=fmt,
@@ -145,7 +147,7 @@ def convert_case(seed=21):
 def encode_case():
     """RTjpeg_compress (lib/RTjpeg.c:3488) over a short clip in both chroma layouts: the reference's packets, byte for byte."""
     w, h, Q, kr, lm = 64, 48, 171, 3, 2
-    s, o = O.encode_clip(O.make_clip(w, h, 255, noise_y=20, noise_c=6, dark=1), 7, threads=1)
+    s, o = O.ref_encode_clip(O.make_clip(w, h, 255, noise_y=20, noise_c=6, dark=1), 7)
     yuv = O.ref_decode_seq(s, o, w, h)
     d = dict(Q=Q, key_rate=kr, lm=lm, cm=lm)
     for fmt, key in ((0, "420"), (1, "422")):

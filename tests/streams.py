@@ -25,6 +25,14 @@ def reference_frames(stream, offsets, w, h, init=None):
     return O.decode_stream(stream, offsets, w, h, init=init)
 
 
+def reference_frames_threaded(stream, offsets, segments, w, h, threads, zero_init=True, raw_tables=None):
+    """reference_frames for independent frame ranges (see oracle.decode_threaded), on `threads` host cores."""
+    if O.have_ref():
+        return O.ref_decode_threaded(stream, offsets, segments, w, h, threads, zero_init=zero_init, keep=True,
+                                     raw_tables=raw_tables)[1]
+    return O.decode_threaded(stream, offsets, segments, w, h, threads, zero_init=zero_init, raw_tables=raw_tables)
+
+
 def clip(w, h, Q, F, **kw):
     c = O.make_clip(w, h, Q, **kw)
     return O.encode_clip(c, F)

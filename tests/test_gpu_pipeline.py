@@ -14,11 +14,6 @@ from streams import clip, reference_frames
 pytestmark = pytest.mark.gpu
 
 
-@pytest.fixture(scope="module", autouse=True)
-def _reference_present():
-    assert O.have_ref(), "oracle/_ref/librtjref.so missing: these tests compare with the compiled reference itself"
-
-
 def _ctx(pipeline, slice_frames, scan=capi.SCAN_CHUNK):
     c = g.BatchContext(0)
     c.set_scan_mode(scan)                  # one CTA per frame even for these small batches: the arrangement that is sliced

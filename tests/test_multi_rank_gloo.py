@@ -85,6 +85,7 @@ def test_two_ranks_decode_disjoint_shards(tmp_path, name, w, h, Q, mask_clean):
     assert (tmp_path / "ok").exists()
 
 
+@pytest.mark.skipif(not O.have_ref(), reason="reference build absent (oracle/_ref): the arm times the reference's own decoder")
 def test_reference_arm_runs_on_rank_zero_only(tmp_path):
     """bench.py --impl reference under a multi-rank launch: rank 0 prints the line, the others exit 0."""
     import json

@@ -8,7 +8,7 @@ import gmerlin_avdecoder_b200 as g
 from gmerlin_avdecoder_b200 import capi
 from oracle import oracle as O
 from nuv_writer import frame, write_nuv
-from streams import clip
+from streams import clip, reference_frames
 
 
 def _payloads(s, o):
@@ -22,7 +22,7 @@ def _reference_frames_with_tables(raw, stream, offsets, w, h):
     out = []
     for f in range(len(offsets) - 1):
         pkt = stream[int(offsets[f]):int(offsets[f + 1])]
-        planes = O.ref_decode_with_tables(raw, pkt, w, h, planes)
+        planes = (O.ref_decode_with_tables if O.have_ref() else O.decode_with_tables)(raw, pkt, w, h, planes)
         out.append(planes.copy())
     return np.stack(out)
 
@@ -63,7 +63,7 @@ def test_reader_follows_demux_nuv():
         assert int.from_bytes(p[6:8].tobytes(), "little") == w and int.from_bytes(p[8:10].tobytes(), "little") == h
         assert p[10] == 0 and np.array_equal(p[12:12 + len(want)], want)
     # what lib/RTjpeg.c makes of them (set_tables path) is what it makes of the original stream
-    direct = O.ref_decode_seq(s, o, w, h)
+    direct = reference_frames(s, o, w, h)
     got = _reference_frames_with_tables(raw, stream, offsets, w, h)
     assert np.array_equal(got[[0, 1, 3, 4, 5, 6]], direct)
     assert np.array_equal(got[2], got[1])                      # 'L': the picture repeats
@@ -109,7 +109,7 @@ def test_config0_nuv_320x240_keyframe_only_on_gpu():
     hd = g.nuv_open(data)
     stream, offsets, tc, unsupported = g.nuv_extract_rtj0(data, hd)
     assert unsupported == 0 and len(offsets) - 1 == F
-    want = O.ref_decode_seq(s, o, w, h)                        # the reference on the original 'RTJ0' stream
+    want = reference_frames(s, o, w, h)                        # the reference on the original 'RTJ0' stream
     with g.BatchContext(0) as ctx:
         ctx.set_custom_tables(np.array(hd.tables[:], dtype=np.uint32))
         desc, _ = g.plan(stream, offsets, capi.State(w, h, capi.TABLE_CUSTOM, 0))
