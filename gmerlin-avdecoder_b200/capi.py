@@ -135,6 +135,10 @@ def load_library() -> C.CDLL:
     L.rtjgpu_decode_device.argtypes = [vp, vp, vp, C.c_int, C.c_int, C.c_int, vp, vp, vp]
     L.rtjgpu_decode_device_rgb.argtypes = [vp, vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, vp, C.c_size_t, C.c_size_t, C.c_int,
                                            vp, vp, vp]
+    L.rtjgpu_decode_device_seq.argtypes = [vp, vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_int), vp,
+                                           C.POINTER(vp), vp]
+    L.rtjgpu_decode_device_rgb_seq.argtypes = [vp, vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_int), C.c_int, vp,
+                                               C.c_size_t, C.c_size_t, C.c_int, C.POINTER(vp), C.POINTER(vp), vp]
     L.rtjgpu_decode_host.argtypes = [vp, _u8p, _u64p, C.c_int, C.POINTER(State), _u8p, _u8p, C.c_int]
     L.rtjgpu_sync.argtypes = [vp]
     L.rtjgpu_enable_timing.argtypes = [vp, C.c_int]
@@ -183,6 +187,17 @@ def _u8(a: np.ndarray):
     return a.ctypes.data_as(_u8p)
 
 
+def _int_array(v):
+    return (C.c_int * max(len(v), 1))(*[int(x) for x in v])
+
+
+def _ptr_array(v):
+    """A host array of device addresses (None entries: NULL), or NULL for v = None."""
+    if v is None:
+        return None
+    return (C.c_void_p * max(len(v), 1))(*[int(x) if x else None for x in v])
+
+
 def _check(rc: int, what: str) -> None:
     if rc != OK:
         raise RTjpegError(rc, what)
@@ -201,6 +216,35 @@ def plan(stream: np.ndarray, offsets: np.ndarray, state: State | None = None):
     _check(L.rtjgpu_plan(_u8(stream), offsets.ctypes.data_as(_u64p), F, C.byref(st),
                          C.c_void_p(desc.ctypes.data)), "rtjgpu_plan")
     return desc[:F], st
+
+
+def plan_sequences(seqs, states=None):
+    """Several independent packet sequences into one batch for rtjgpu_decode_device_seq.  seqs: list of (stream, offsets) as
+    for plan().  Every sequence's packets keep their slots and their alignment modulo 16 in one buffer; each sequence is
+    planned on its own with its own state (states: list of State advanced in place, or None = fresh ones).
+    Returns (stream, offsets[F + 1], desc[F], seq_first[S + 1], states)."""
+    if states is None:
+        states = [State(0, 0, TABLE_ZERO, 0) for _ in seqs]
+    assert len(states) == len(seqs)
+    bases, at = [], 0
+    for _, offsets in seqs:
+        lo, hi = int(offsets[0]), int(offsets[-1])
+        base = (at + 15) // 16 * 16 + lo % 16           # the packets' starts keep their place modulo 16
+        bases.append(base)
+        at = base + hi - lo
+    out = np.zeros(at, dtype=np.uint8)
+    offs, descs, seq_first = [], [], [0]
+    for (stream, offsets), base, st in zip(seqs, bases, states):
+        offsets = np.asarray(offsets, dtype=np.uint64)
+        lo, hi = int(offsets[0]), int(offsets[-1])
+        out[base:base + hi - lo] = np.asarray(stream, dtype=np.uint8)[lo:hi]
+        o = offsets - np.uint64(lo) + np.uint64(base)
+        desc, _ = plan(out, o, st)
+        offs.append(o[:-1])
+        descs.append(desc)
+        seq_first.append(seq_first[-1] + len(desc))
+    offsets = np.concatenate(offs + [np.array([at], dtype=np.uint64)])
+    return out, offsets, np.concatenate(descs), np.array(seq_first, dtype=np.int64), states
 
 
 def tables_for_quality(Q: int):
@@ -378,6 +422,25 @@ class BatchContext:
                                                 C.c_void_p(d_rgb), row_pitch, frame_pitch, alpha, C.c_void_p(d_carry or 0),
                                                 C.c_void_p(d_last_yuv or 0), C.c_void_p(cuda_stream or 0)),
                "rtjgpu_decode_device_rgb")
+
+    def decode_device_seq(self, d_stream: int, d_desc: int, F: int, w: int, h: int, seq_first, d_out: int,
+                          carries=None, cuda_stream: int | None = None) -> None:
+        """rtjgpu_decode_device_seq: seq_first[S + 1] frame indices, carries a list of S device addresses (None = zeros)
+        or None."""
+        S = len(seq_first) - 1
+        _check(self._L.rtjgpu_decode_device_seq(self._h, C.c_void_p(d_stream), C.c_void_p(d_desc), F, w, h, S,
+                                                _int_array(seq_first), C.c_void_p(d_out), _ptr_array(carries),
+                                                C.c_void_p(cuda_stream or 0)), "rtjgpu_decode_device_seq")
+
+    def decode_device_rgb_seq(self, d_stream: int, d_desc: int, F: int, w: int, h: int, seq_first, kind: int, d_rgb: int,
+                              row_pitch: int, frame_pitch: int, alpha: int = 0, carries=None, last_yuv=None,
+                              cuda_stream: int | None = None) -> None:
+        """rtjgpu_decode_device_rgb_seq: last_yuv a list of S device addresses (None = not wanted) or None."""
+        S = len(seq_first) - 1
+        _check(self._L.rtjgpu_decode_device_rgb_seq(self._h, C.c_void_p(d_stream), C.c_void_p(d_desc), F, w, h, S,
+                                                    _int_array(seq_first), kind, C.c_void_p(d_rgb), row_pitch, frame_pitch,
+                                                    alpha, _ptr_array(carries), _ptr_array(last_yuv),
+                                                    C.c_void_p(cuda_stream or 0)), "rtjgpu_decode_device_rgb_seq")
 
     def decode_host(self, stream: np.ndarray, offsets: np.ndarray, out: np.ndarray, state: State | None = None,
                     carry: np.ndarray | None = None, flags: int = 0) -> State:

@@ -44,6 +44,8 @@ struct Workspace {
     /* K2's position table, rebuilt when the geometry changes */
     void         *d_lut = nullptr;       size_t lut_cap = 0;     /* bytes */
     int           lut_fmt = -1, lut_w = 0, lut_h = 0;
+    /* the sequence layout of a batch of several sequences (seq_upload) */
+    uint8_t      *d_seq = nullptr;       size_t seq_cap = 0;     /* bytes */
 };
 
 constexpr int HOST_SLOTS = 3;
@@ -122,6 +124,12 @@ struct rtjgpu_ctx {
     uint64_t       host_bad = 0;              /* overrun frames seen by the current rtjgpu_decode_host call */
     uint32_t      *h_host_skips = nullptr;    size_t host_skips_cap = 0;   /* pinned: per-frame skip counts of that call */
     int            host_F = 0;
+    /* pinned staging of the sequence layouts of rtjgpu_decode_device[_rgb]_seq: two buffers taken in turn, each reused only
+     * when its last copy to the device is done */
+    uint8_t       *h_seq[2] = {};             size_t h_seq_cap[2] = {};
+    cudaEvent_t    seq_copied[2] = {};
+    bool           seq_pending[2] = {};
+    int            seq_turn = 0;
 };
 
 namespace {
@@ -291,6 +299,7 @@ void ws_release(Workspace *ws)
     if (ws->d_seg_gentry) cudaFree(ws->d_seg_gentry);
     if (ws->d_seg_gbase) cudaFree(ws->d_seg_gbase);
     if (ws->d_lut) cudaFree(ws->d_lut);
+    if (ws->d_seq) cudaFree(ws->d_seq);
     *ws = Workspace();
 }
 
@@ -348,6 +357,24 @@ int plan_slices(const rtjgpu_ctx *ctx, int F, int *first)
  * K2's short-lived CTAs retire.  The last writer of a skipped block lies in an earlier frame, i.e. in a slice
  * that is already scanned, so nothing else has to be ordered.
  */
+/* The sequences of a device batch as the caller gave them: host arrays.  first == NULL: rtjgpu_decode_device[_rgb], one
+ * sequence whose carry and last_yuv are carries[0] / last_yuv[0]. */
+struct SeqIn {
+    int                   S = 1;
+    const int            *first = nullptr;       /* [S + 1] */
+    const uint8_t *const *carries = nullptr;     /* [S], or NULL: zeros */
+    uint8_t *const       *last_yuv = nullptr;    /* [S], or NULL */
+    const uint8_t *carry(int s) const { return carries ? carries[s] : nullptr; }
+    uint8_t *last(int s) const { return last_yuv ? last_yuv[s] : nullptr; }
+};
+
+/* ... and its device copy (S > 1; all NULL for one sequence: the kernels take the one-stream path) */
+struct SeqDev {
+    const uint32_t       *seq = nullptr;         /* [F] RTJ_SEQ(first, index) */
+    const uint8_t *const *carries = nullptr;     /* [S] */
+    uint8_t *const       *last_yuvs = nullptr;   /* [S] */
+};
+
 /* where K2's pixels go when they leave as packed RGB (rtjgpu_decode_device_rgb) */
 struct RgbOut {
     uint8_t *d_rgb = nullptr;
@@ -359,7 +386,7 @@ struct RgbOut {
 
 int run_kernels(rtjgpu_ctx *ctx, Workspace *ws, const uint8_t *d_stream, const rtjgpu_frame_desc *d_desc,
                 int F, int w, int h, uint8_t *d_out, const uint8_t *d_carry, cudaStream_t st, cudaEvent_t *ev,
-                bool allow_pipe, const RgbOut *rgb = nullptr)
+                bool allow_pipe, const RgbOut *rgb = nullptr, const SeqDev *seq = nullptr)
 {
     rtj_launch_args a;
     a.d_stream = d_stream; a.d_desc = d_desc; a.d_tables = ctx->d_tables;
@@ -383,6 +410,7 @@ int run_kernels(rtjgpu_ctx *ctx, Workspace *ws, const uint8_t *d_stream, const r
     a.d_rgb = rgb ? rgb->d_rgb : nullptr;
     a.rgb_row_pitch = rgb ? rgb->row_pitch : 0; a.rgb_frame_pitch = rgb ? rgb->frame_pitch : 0;
     a.rgb_kind = rgb ? rgb->kind : 0; a.rgb_alpha = rgb ? rgb->alpha : 0; a.d_last_yuv = rgb ? rgb->d_last_yuv : nullptr;
+    a.d_seq = seq ? seq->seq : nullptr; a.d_carries = seq ? seq->carries : nullptr; a.d_last_yuvs = seq ? seq->last_yuvs : nullptr;
     a.scan_mode = ctx->scan_mode;
     const int nblk = RTJ_FMT_NBLK(ctx->format, w, h);
     {
@@ -495,6 +523,122 @@ int grow_pinned(rtjgpu_ctx *ctx, T **p, size_t *cap, size_t need)
     return RTJGPU_OK;
 }
 
+/* The checks of the _seq calls that the one-stream calls do not have. */
+int seq_check(int F, const SeqIn &q)
+{
+    if (q.S < 1 || q.S > F || !q.first || q.first[0] != 0 || q.first[q.S] != F) return RTJGPU_E_ARG;
+    for (int s = 0; s < q.S; s++) {
+        if (q.first[s + 1] <= q.first[s]) return RTJGPU_E_ARG;              /* no empty sequence */
+        if (((uintptr_t)q.carry(s) & 7) || ((uintptr_t)q.last(s) & 15)) return RTJGPU_E_ARG;
+    }
+    return RTJGPU_OK;
+}
+
+/* The device copy of a layout of S > 1 sequences, in the workspace: [F] RTJ_SEQ words, then [S] carry pointers, then
+ * [S] last_yuv pointers.  It goes up with cudaMemcpyAsync on the launch stream, staged in one of two pinned buffers taken
+ * in turn; a buffer is written again only once its previous copy is done, and the caller's arrays are not read after
+ * this returns. */
+int seq_upload(rtjgpu_ctx *ctx, Workspace *ws, int F, const SeqIn &q, cudaStream_t st, SeqDev *out)
+{
+    const size_t words = ((size_t)F * sizeof(uint32_t) + 7) & ~(size_t)7, ptrs = (size_t)q.S * sizeof(void *);
+    const size_t bytes = words + 2 * ptrs;
+    const int t = ctx->seq_turn;
+    if (!ctx->seq_copied[t]) CK(ctx, cudaEventCreateWithFlags(&ctx->seq_copied[t], cudaEventDisableTiming));
+    if (ctx->seq_pending[t]) {
+        CK(ctx, cudaEventSynchronize(ctx->seq_copied[t]));
+        ctx->seq_pending[t] = false;
+    }
+    int rc = grow_pinned(ctx, &ctx->h_seq[t], &ctx->h_seq_cap[t], bytes);
+    if (rc) return rc;
+    if ((rc = grow_device(ctx, &ws->d_seq, &ws->seq_cap, bytes))) return rc;
+    uint32_t *hw = reinterpret_cast<uint32_t *>(ctx->h_seq[t]);
+    for (int s = 0; s < q.S; s++)
+        for (int f = q.first[s]; f < q.first[s + 1]; f++) hw[f] = RTJ_SEQ(q.first[s], s);
+    const uint8_t **hc = reinterpret_cast<const uint8_t **>(ctx->h_seq[t] + words);
+    uint8_t **hl = reinterpret_cast<uint8_t **>(ctx->h_seq[t] + words + ptrs);
+    for (int s = 0; s < q.S; s++) { hc[s] = q.carry(s); hl[s] = q.last(s); }
+    CK(ctx, cudaMemcpyAsync(ws->d_seq, ctx->h_seq[t], bytes, cudaMemcpyHostToDevice, st));
+    CK(ctx, cudaEventRecord(ctx->seq_copied[t], st));
+    ctx->seq_pending[t] = true;
+    ctx->seq_turn = t ^ 1;
+    out->seq = reinterpret_cast<const uint32_t *>(ws->d_seq);
+    out->carries = reinterpret_cast<const uint8_t *const *>(ws->d_seq + words);
+    out->last_yuvs = reinterpret_cast<uint8_t *const *>(ws->d_seq + words + ptrs);
+    return RTJGPU_OK;
+}
+
+/* rtjgpu_decode_device and rtjgpu_decode_device_seq: the former is the latter's one-sequence case. */
+int decode_device(rtjgpu_ctx *ctx, const uint8_t *d_stream, const rtjgpu_frame_desc *d_desc, int F, int w, int h,
+                  const SeqIn &q, uint8_t *d_out, void *cuda_stream)
+{
+    if (!ctx || F < 0) return RTJGPU_E_ARG;
+    if (q.first) {
+        const int rc = seq_check(F, q);
+        if (rc) return rc;
+    }
+    if (F == 0) { ctx->last_F = 0; return RTJGPU_OK; }
+    if (!d_stream || !d_desc || !d_out) return RTJGPU_E_ARG;
+    /* K1 reads the stream as 32-bit words, K2 leaves its strips as 16-byte bulk stores and reads the carry as 8-byte rows */
+    if (((uintptr_t)d_stream & 3) || ((uintptr_t)d_desc & 7) || ((uintptr_t)d_out & 15) || ((uintptr_t)q.carry(0) & 7)) return RTJGPU_E_ARG;
+    if (w <= 0 || h <= 0 || (w & 15) || (h & 15) || w > 65535 || h > 65535) return RTJGPU_E_SIZE;
+    if (F > RTJGPU_MAX_FRAMES_PER_BATCH) return RTJGPU_E_TOOBIG;
+    CK(ctx, cudaSetDevice(ctx->device));
+    const int nblk = RTJ_FMT_NBLK(ctx->format, w, h);
+    if ((uint64_t)F * (uint64_t)nblk >= (1ull << 32)) return RTJGPU_E_TOOBIG;   /* block indices are 32 bit */
+    if ((uint64_t)RTJ_FMT_FRAME_BYTES(ctx->format, w, h) >= (1ull << 32)) return RTJGPU_E_TOOBIG;   /* and so are offsets inside a frame */
+    int rc = ws_reserve(ctx, &ctx->ws, F, nblk);
+    if (rc) return rc;
+    SeqDev sd;
+    if (q.S > 1 && (rc = seq_upload(ctx, &ctx->ws, F, q, (cudaStream_t)cuda_stream, &sd))) return rc;
+    cudaEvent_t *ev = ctx->timing ? ctx->ev[ctx->timed_calls % TIMING_RING] : nullptr;
+    rc = run_kernels(ctx, &ctx->ws, d_stream, d_desc, F, w, h, d_out, q.S > 1 ? nullptr : q.carry(0), (cudaStream_t)cuda_stream, ev,
+                     true, nullptr, q.S > 1 ? &sd : nullptr);
+    if (ev && rc == RTJGPU_OK) ctx->timed_calls++;
+    ctx->last_F = F;
+    ctx->last_stream = cuda_stream;
+    return rc;
+}
+
+/* rtjgpu_decode_device_rgb and rtjgpu_decode_device_rgb_seq */
+int decode_device_rgb(rtjgpu_ctx *ctx, const uint8_t *d_stream, const rtjgpu_frame_desc *d_desc, int F, int w, int h,
+                      const SeqIn &q, int kind, uint8_t *d_rgb, size_t row_pitch, size_t frame_pitch, int alpha, void *cuda_stream)
+{
+    if (!ctx || F < 0) return RTJGPU_E_ARG;
+    if (ctx->format != RTJ_YUV420) return RTJGPU_E_FORMAT;                     /* the reference's converters are yuv420 ones */
+    if (kind != RTJ_CONV_RGB32 && kind != RTJ_CONV_BGR32 && kind != RTJ_CONV_RGB24 && kind != RTJ_CONV_BGR24 && kind != RTJ_CONV_RGB16)
+        return RTJGPU_E_FORMAT;
+    if (q.first) {
+        const int rc = seq_check(F, q);
+        if (rc) return rc;
+    }
+    if (F == 0) { ctx->last_F = 0; return RTJGPU_OK; }
+    if (!d_stream || !d_desc || !d_rgb) return RTJGPU_E_ARG;
+    if (w <= 0 || h <= 0 || (w & 15) || (h & 15) || w > 65535 || h > 65535) return RTJGPU_E_SIZE;
+    if (F > RTJGPU_MAX_FRAMES_PER_BATCH) return RTJGPU_E_TOOBIG;
+    const int bpp = rtj_convert_bpp(kind);
+    if (((uintptr_t)d_stream & 3) || ((uintptr_t)d_desc & 7) || ((uintptr_t)d_rgb & 15) || ((uintptr_t)q.carry(0) & 7)
+        || ((uintptr_t)q.last(0) & 15) || (row_pitch & 15) || (frame_pitch & 15) || row_pitch < (size_t)w * bpp
+        || frame_pitch < row_pitch * (size_t)h)
+        return RTJGPU_E_ARG;
+    CK(ctx, cudaSetDevice(ctx->device));
+    const int nblk = RTJ_FMT_NBLK(ctx->format, w, h);
+    if ((uint64_t)F * (uint64_t)nblk >= (1ull << 32)) return RTJGPU_E_TOOBIG;
+    int rc = ws_reserve(ctx, &ctx->ws, F, nblk);
+    if (rc) return rc;
+    SeqDev sd;
+    if (q.S > 1 && (rc = seq_upload(ctx, &ctx->ws, F, q, (cudaStream_t)cuda_stream, &sd))) return rc;
+    RgbOut o;
+    o.d_rgb = d_rgb; o.row_pitch = row_pitch; o.frame_pitch = frame_pitch; o.kind = kind; o.alpha = (unsigned)alpha & 0xFFu;
+    o.d_last_yuv = q.S > 1 ? nullptr : q.last(0);
+    cudaEvent_t *ev = ctx->timing ? ctx->ev[ctx->timed_calls % TIMING_RING] : nullptr;
+    rc = run_kernels(ctx, &ctx->ws, d_stream, d_desc, F, w, h, nullptr, q.S > 1 ? nullptr : q.carry(0), (cudaStream_t)cuda_stream, ev,
+                     true, &o, q.S > 1 ? &sd : nullptr);
+    if (ev && rc == RTJGPU_OK) ctx->timed_calls++;
+    ctx->last_F = F;
+    ctx->last_stream = cuda_stream;
+    return rc;
+}
+
 } // namespace
 
 extern "C" {
@@ -603,6 +747,10 @@ void rtjgpu_destroy(rtjgpu_ctx *ctx)
     if (ctx->h_info_reset) cudaFreeHost(ctx->h_info_reset);
     if (ctx->h_info) cudaFreeHost(ctx->h_info);
     if (ctx->h_skips_seen) cudaFreeHost(ctx->h_skips_seen);
+    for (int i = 0; i < 2; i++) {
+        if (ctx->h_seq[i]) cudaFreeHost(ctx->h_seq[i]);
+        if (ctx->seq_copied[i]) cudaEventDestroy(ctx->seq_copied[i]);
+    }
     for (int i = 0; i < TIMING_RING * 4; i++) if (ctx->ev[i / 4][i % 4]) cudaEventDestroy(ctx->ev[i / 4][i % 4]);
     delete ctx;
 }
@@ -856,58 +1004,37 @@ int rtjgpu_plan_n(const uint8_t *stream, const uint64_t *offsets, const uint32_t
 int rtjgpu_decode_device(rtjgpu_ctx *ctx, const uint8_t *d_stream, const rtjgpu_frame_desc *d_desc, int F,
                          int w, int h, uint8_t *d_out, const uint8_t *d_carry, void *cuda_stream)
 {
-    if (!ctx || F < 0) return RTJGPU_E_ARG;
-    if (F == 0) { ctx->last_F = 0; return RTJGPU_OK; }
-    if (!d_stream || !d_desc || !d_out) return RTJGPU_E_ARG;
-    /* K1 reads the stream as 32-bit words, K2 leaves its strips as 16-byte bulk stores and reads the carry as 8-byte rows */
-    if (((uintptr_t)d_stream & 3) || ((uintptr_t)d_desc & 7) || ((uintptr_t)d_out & 15) || ((uintptr_t)d_carry & 7)) return RTJGPU_E_ARG;
-    if (w <= 0 || h <= 0 || (w & 15) || (h & 15) || w > 65535 || h > 65535) return RTJGPU_E_SIZE;
-    if (F > RTJGPU_MAX_FRAMES_PER_BATCH) return RTJGPU_E_TOOBIG;
-    CK(ctx, cudaSetDevice(ctx->device));
-    const int nblk = RTJ_FMT_NBLK(ctx->format, w, h);
-    if ((uint64_t)F * (uint64_t)nblk >= (1ull << 32)) return RTJGPU_E_TOOBIG;   /* block indices are 32 bit */
-    if ((uint64_t)RTJ_FMT_FRAME_BYTES(ctx->format, w, h) >= (1ull << 32)) return RTJGPU_E_TOOBIG;   /* and so are offsets inside a frame */
-    int rc = ws_reserve(ctx, &ctx->ws, F, nblk);
-    if (rc) return rc;
-    cudaEvent_t *ev = ctx->timing ? ctx->ev[ctx->timed_calls % TIMING_RING] : nullptr;
-    rc = run_kernels(ctx, &ctx->ws, d_stream, d_desc, F, w, h, d_out, d_carry, (cudaStream_t)cuda_stream, ev, true);
-    if (ev && rc == RTJGPU_OK) ctx->timed_calls++;
-    ctx->last_F = F;
-    ctx->last_stream = cuda_stream;
-    return rc;
+    SeqIn q;
+    q.carries = &d_carry;
+    return decode_device(ctx, d_stream, d_desc, F, w, h, q, d_out, cuda_stream);
+}
+
+int rtjgpu_decode_device_seq(rtjgpu_ctx *ctx, const uint8_t *d_stream, const rtjgpu_frame_desc *d_desc, int F, int w, int h,
+                             int S, const int *seq_first, uint8_t *d_out, const uint8_t *const *carries, void *cuda_stream)
+{
+    SeqIn q;
+    q.S = S; q.first = seq_first; q.carries = carries;
+    if (!seq_first) return RTJGPU_E_ARG;
+    return decode_device(ctx, d_stream, d_desc, F, w, h, q, d_out, cuda_stream);
 }
 
 int rtjgpu_decode_device_rgb(rtjgpu_ctx *ctx, const uint8_t *d_stream, const rtjgpu_frame_desc *d_desc, int F,
                              int w, int h, int kind, uint8_t *d_rgb, size_t row_pitch, size_t frame_pitch, int alpha,
                              const uint8_t *d_carry, uint8_t *d_last_yuv, void *cuda_stream)
 {
-    if (!ctx || F < 0) return RTJGPU_E_ARG;
-    if (ctx->format != RTJ_YUV420) return RTJGPU_E_FORMAT;                     /* the reference's converters are yuv420 ones */
-    if (kind != RTJ_CONV_RGB32 && kind != RTJ_CONV_BGR32 && kind != RTJ_CONV_RGB24 && kind != RTJ_CONV_BGR24 && kind != RTJ_CONV_RGB16)
-        return RTJGPU_E_FORMAT;
-    if (F == 0) { ctx->last_F = 0; return RTJGPU_OK; }
-    if (!d_stream || !d_desc || !d_rgb) return RTJGPU_E_ARG;
-    if (w <= 0 || h <= 0 || (w & 15) || (h & 15) || w > 65535 || h > 65535) return RTJGPU_E_SIZE;
-    if (F > RTJGPU_MAX_FRAMES_PER_BATCH) return RTJGPU_E_TOOBIG;
-    const int bpp = rtj_convert_bpp(kind);
-    if (((uintptr_t)d_stream & 3) || ((uintptr_t)d_desc & 7) || ((uintptr_t)d_rgb & 15) || ((uintptr_t)d_carry & 7)
-        || ((uintptr_t)d_last_yuv & 15) || (row_pitch & 15) || (frame_pitch & 15) || row_pitch < (size_t)w * bpp
-        || frame_pitch < row_pitch * (size_t)h)
-        return RTJGPU_E_ARG;
-    CK(ctx, cudaSetDevice(ctx->device));
-    const int nblk = RTJ_FMT_NBLK(ctx->format, w, h);
-    if ((uint64_t)F * (uint64_t)nblk >= (1ull << 32)) return RTJGPU_E_TOOBIG;
-    int rc = ws_reserve(ctx, &ctx->ws, F, nblk);
-    if (rc) return rc;
-    RgbOut o;
-    o.d_rgb = d_rgb; o.row_pitch = row_pitch; o.frame_pitch = frame_pitch; o.kind = kind; o.alpha = (unsigned)alpha & 0xFFu;
-    o.d_last_yuv = d_last_yuv;
-    cudaEvent_t *ev = ctx->timing ? ctx->ev[ctx->timed_calls % TIMING_RING] : nullptr;
-    rc = run_kernels(ctx, &ctx->ws, d_stream, d_desc, F, w, h, nullptr, d_carry, (cudaStream_t)cuda_stream, ev, true, &o);
-    if (ev && rc == RTJGPU_OK) ctx->timed_calls++;
-    ctx->last_F = F;
-    ctx->last_stream = cuda_stream;
-    return rc;
+    SeqIn q;
+    q.carries = &d_carry; q.last_yuv = &d_last_yuv;
+    return decode_device_rgb(ctx, d_stream, d_desc, F, w, h, q, kind, d_rgb, row_pitch, frame_pitch, alpha, cuda_stream);
+}
+
+int rtjgpu_decode_device_rgb_seq(rtjgpu_ctx *ctx, const uint8_t *d_stream, const rtjgpu_frame_desc *d_desc, int F, int w, int h,
+                                 int S, const int *seq_first, int kind, uint8_t *d_rgb, size_t row_pitch, size_t frame_pitch,
+                                 int alpha, const uint8_t *const *carries, uint8_t *const *last_yuv, void *cuda_stream)
+{
+    SeqIn q;
+    q.S = S; q.first = seq_first; q.carries = carries; q.last_yuv = last_yuv;
+    if (!seq_first) return RTJGPU_E_ARG;
+    return decode_device_rgb(ctx, d_stream, d_desc, F, w, h, q, kind, d_rgb, row_pitch, frame_pitch, alpha, cuda_stream);
 }
 
 int rtjgpu_sync(rtjgpu_ctx *ctx)

@@ -51,6 +51,13 @@ extern "C" {
  * coded the block, or RTJ_SRC_CARRY when none has yet. */
 #define RTJ_SRC_CARRY 0xFFFFu
 
+/* Per-frame word of a batch of several sequences: the frame where f's sequence starts and that sequence's index
+ * (both below 2^16: F <= RTJGPU_MAX_FRAMES_PER_BATCH).  A last writer before RTJ_SEQ_FIRST(...) belongs to another
+ * sequence and does not count. */
+#define RTJ_SEQ(first, index) ((uint32_t)(first) | (uint32_t)(index) << 16)
+#define RTJ_SEQ_FIRST(v) ((v) & 0xFFFFu)
+#define RTJ_SEQ_INDEX(v) ((v) >> 16)
+
 #define RTJ_NUM_TABLES 257
 
 /* Dequantisation tables as the kernels read them: zig-zag order (entry k is
@@ -156,6 +163,11 @@ typedef struct rtj_launch_args {
     int                      rgb_kind;      /* RTJ_CONV_RGB32 / BGR32 / RGB24 / BGR24 / RGB16 */
     unsigned                 rgb_alpha;
     uint8_t                 *d_last_yuv;    /* the batch's last frame as planes too, or NULL */
+    /* a batch of several independent sequences (rtjgpu_decode_device_seq); all NULL for one sequence, which takes
+     * d_carry / d_last_yuv instead */
+    const uint32_t          *d_seq;         /* [F] RTJ_SEQ(first frame of f's sequence, index of that sequence) */
+    const uint8_t *const    *d_carries;     /* [S] picture before each sequence, entries NULL = zeros */
+    uint8_t *const          *d_last_yuvs;   /* [S] RGB: where each sequence's last frame leaves as planes, entries may be NULL */
     int                      scan_mode;     /* RTJGPU_SCAN_* */
     rtj_seg_plan             seg;           /* workspace of the segment-parallel scan (sum == NULL: not available) */
 } rtj_launch_args;

@@ -514,6 +514,11 @@ struct K2Params {
     int rgb_kind;                    /* RTJ_CONV_RGB32 / BGR32 / RGB24 / BGR24 / RGB16 */
     unsigned rgb_alpha;
     uint8_t *last_yuv;               /* RGB: the batch's last frame as planes as well (the next batch's carry), or NULL */
+    /* several independent sequences in the batch (NULL: one, which takes carry / last_yuv): per frame RTJ_SEQ(first frame
+     * of its sequence, sequence index); per sequence its carry and, RGB, where its last frame leaves as planes */
+    const uint32_t *seq;
+    const uint8_t *const *carries;
+    uint8_t *const *last_yuvs;
     int ahead;                       /* frames between a CTA and the one that follows it on the same SM slot */
     int wq;                          /* slots of one warp's queue */
 };
@@ -638,6 +643,8 @@ rtj_idct_kernel(const K2Params P)
     unsigned valid = 0;              /* bit r: the strip holds the picture's pixels at this thread's position of round r */
 
     for (unsigned f = f_first; f < f_last; f++) {
+    /* a frame that starts a sequence of its own holds nothing of the frame before: like the run's first frame, it keeps nothing */
+    if (runs && P.seq && RTJ_SEQ_FIRST(P.seq[f]) == f) valid = 0u;
     const unsigned frame_blk0 = f * (unsigned)P.nblk + strip_blk0;   /* F * nblk < 2^32 (checked by the host) */
     const uint32_t *my_ent = P.ent + frame_blk0;
     /* A CTA lives a few microseconds, of which the first read of its entries from DRAM -- under the write traffic of
@@ -855,9 +862,10 @@ rtj_idct_kernel(const K2Params P)
             }
             if (live && !hard) {
                 uint32_t px[16];
-                if (P.carry) {
+                const uint8_t *carry = P.seq ? P.carries[RTJ_SEQ_INDEX(P.seq[f])] : P.carry;    /* the picture before f's sequence */
+                if (carry) {
                     int pitch;
-                    const uint8_t *cp = G::carry_src(P.carry, bi, my, mx0, w, h, pitch);
+                    const uint8_t *cp = G::carry_src(carry, bi, my, mx0, w, h, pitch);
 #pragma unroll
                     for (int r = 0; r < 8; r++) {
                         const uint2 v = *reinterpret_cast<const uint2 *>(cp + (size_t)r * pitch);
@@ -879,6 +887,7 @@ rtj_idct_kernel(const K2Params P)
     __syncthreads();
     const int lw = G::UNIT_W * mbs;                              /* luma bytes per strip row */
     bool planes_leave = true, luma_leaves = true;
+    uint8_t *last_planes = P.last_yuv;                          /* RGB: where the frame leaves as planes too, if it does */
     if (RGB) {
         /* The strip -- 16 luma rows, 8 rows of Cb and of Cr: exactly what the reference's converters read for 16 output
          * rows (lib/RTjpeg.c:3123-3190) -- leaves as packed pixels.  A thread takes 8 pixels of two rows (one chroma row):
@@ -907,7 +916,12 @@ rtj_idct_kernel(const K2Params P)
             default:             row8<RTJ_CONV_RGB16>(y0, ct, P.rgb_alpha, o); row8<RTJ_CONV_RGB16>(y1, ct, P.rgb_alpha, o + P.rgb_row_pitch); break;
             }
         }
-        if (!P.last_yuv || f + 1u != (unsigned)P.F) planes_leave = false;      /* the last frame also leaves as planes: the next batch's carry */
+        /* the last frame also leaves as planes: the next batch's carry -- with several sequences, the last frame of each */
+        if (P.seq) {
+            const unsigned nx = f + 1u;
+            last_planes = nx == (unsigned)P.F || RTJ_SEQ_FIRST(P.seq[nx]) == nx ? P.last_yuvs[RTJ_SEQ_INDEX(P.seq[f])] : nullptr;
+        } else if (f + 1u != (unsigned)P.F) last_planes = nullptr;
+        if (!last_planes) planes_leave = false;
     } else {
         /* What rtj_idct_hard*_kernel patch need not be written here first.  All blocks HARD: nothing leaves; all luma blocks
          * (a quality above 170, where every luma block carries ten coefficients or more): the chroma rows only. */
@@ -918,7 +932,7 @@ rtj_idct_kernel(const K2Params P)
     if (planes_leave) {
     const size_t fsz = RTJ_FMT_FRAME_BYTES(FMT, w, h);
     const int cw = w >> 1;
-    uint8_t *const planes = RGB ? P.last_yuv : P.out + (size_t)f * fsz;
+    uint8_t *const planes = RGB ? last_planes : P.out + (size_t)f * fsz;
     uint8_t *oy = planes + (size_t)(my * G::LUMA_ROWS) * w + mx0 * G::UNIT_W;
     uint8_t *ou = planes + (size_t)w * h + (size_t)(my * 8) * cw + mx0 * 8;
     uint8_t *ov = ou + (FMT == 0 ? (size_t)cw * (h >> 1) : (size_t)cw * h);
@@ -1396,6 +1410,7 @@ extern "C" int rtj_launch_idct(const rtj_launch_args *a, void *stream)
     const int nf = a->f1 - a->f0;
     P.rgb = a->d_rgb; P.rgb_row_pitch = a->rgb_row_pitch; P.rgb_frame_pitch = a->rgb_frame_pitch;
     P.rgb_kind = a->rgb_kind; P.rgb_alpha = a->rgb_alpha & 0xFFu; P.last_yuv = a->d_last_yuv;
+    P.seq = a->d_seq; P.carries = a->d_carries; P.last_yuvs = a->d_last_yuvs;
     if (a->d_rgb) {
         if (fmt != 0) return (int)cudaErrorInvalidValue;
         switch (a->rgb_kind) {

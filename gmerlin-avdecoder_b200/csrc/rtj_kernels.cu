@@ -329,6 +329,9 @@ rtj_scan_lane_kernel(const uint8_t *__restrict__ stream, const rtjgpu_frame_desc
  * before them -- hold no skip marker has nothing to resolve: every position was written by frame f1 - 1.
  * (slice_skips[0 .. slice] are final when K3 of that slice runs; the batch-wide count is not, K1 of later
  * slices may be running.)
+ * A batch of several independent sequences (rtjgpu_decode_device_seq) changes nothing but rtj_resolve_kernel's walk:
+ * a last writer in front of the frame's own sequence is taken as none.  rtj_resolve_last_kernel's running maximum and
+ * the shortcut above stay exact -- the nearest writer before a frame is the only one that can lie in its sequence.
  */
 constexpr int RESOLVE_T = RTJ_RESOLVE_T;
 
@@ -404,11 +407,13 @@ rtj_resolve_last_kernel(const uint32_t *__restrict__ ent, uint16_t *__restrict__
     }
 }
 
-extern "C" __global__ void __launch_bounds__(128)
+/* (seven CTAs an SM: 72 registers, what the kernel held before the sequence check -- registers are allocated in eights) */
+extern "C" __global__ void __launch_bounds__(128, 7)
 rtj_resolve_kernel(uint32_t *__restrict__ ent, const uint16_t *__restrict__ chunk_last, const uint32_t *__restrict__ chunk_mask,
                    uint16_t *__restrict__ src, int f0, int f1, int nblk, const rtj_dev_info *__restrict__ info, int slice,
                    const uint16_t *__restrict__ carry_in, uint16_t *__restrict__ carry_out,
-                   const rtjgpu_frame_desc *__restrict__ desc, unsigned long long *__restrict__ skips_seen)
+                   const rtjgpu_frame_desc *__restrict__ desc, unsigned long long *__restrict__ skips_seen,
+                   const uint32_t *__restrict__ seq)
 {
     const int b = blockIdx.x * blockDim.x + threadIdx.x;
     /* how many blocks the batch skipped, left where the host sees it without asking (pinned memory): the next batch's
@@ -430,6 +435,15 @@ rtj_resolve_kernel(uint32_t *__restrict__ ent, const uint16_t *__restrict__ chun
         const int fa = c0 * RESOLVE_T, fb = min(f1, fa + RESOLVE_T);
         unsigned last = c0 > c_lo ? chunk_last[(size_t)(c0 - 1) * nblk + b] : RTJ_SRC_CARRY;   /* rtj_resolve_last_kernel's running maximum */
         if (last == RTJ_SRC_CARRY && carry_in) last = carry_in[b];
+        /* Several sequences in the batch (seq != NULL): a last writer in front of the frame's own sequence is none -- the block
+         * comes from that sequence's carry.  One comparison at the chunk's first frame covers the running maximum and carry_in
+         * (RTJ_SRC_CARRY is above every frame index); behind it, a frame that starts a sequence starts from none. */
+        uint32_t starts = 0;                                         /* bit j: frame fa + j starts a sequence */
+        if (seq) {
+            if (RTJ_SEQ_FIRST(seq[fa]) > last) last = RTJ_SRC_CARRY;
+#pragma unroll 1
+            for (int j = 1; j < fb - fa; j++) starts |= (RTJ_SEQ_FIRST(seq[fa + j]) == (unsigned)(fa + j) ? 1u : 0u) << j;
+        }
         /* the last writer's entry, when it is an inline one (the block travels in it), and the tables it was written under:
          * a skipped block of a frame with the same tables gets a copy of it (RTJ_ENT_COPY_BIT) in the place of its marker */
         uint32_t last_e = 0;
@@ -453,6 +467,7 @@ rtj_resolve_kernel(uint32_t *__restrict__ ent, const uint16_t *__restrict__ chun
             }
 #pragma unroll
             for (int j = 0; j < 8; j++) {
+                if ((starts >> (f + j - fa)) & 1u) { last = RTJ_SRC_CARRY; last_e = 0; }
                 if (RTJ_ENT_IS_SKIP(e[j])) {
                     if (last_e && tab[j] == last_tab) ent[(size_t)(f + j) * nblk + b] = last_e;
                     else src[(size_t)(f + j) * nblk + b] = (uint16_t)last;
@@ -466,6 +481,7 @@ rtj_resolve_kernel(uint32_t *__restrict__ ent, const uint16_t *__restrict__ chun
         for (; f < fb; f++) {
             const uint32_t ee = (skipped >> (f - fa)) & 1u ? RTJ_ENT_SKIP : ent[(size_t)f * nblk + b];
             const unsigned tb = desc[f].table;
+            if ((starts >> (f - fa)) & 1u) { last = RTJ_SRC_CARRY; last_e = 0; }
             if (RTJ_ENT_IS_SKIP(ee)) {
                 if (last_e && tb == last_tab) ent[(size_t)f * nblk + b] = last_e;
                 else src[(size_t)f * nblk + b] = (uint16_t)last;
@@ -719,7 +735,7 @@ extern "C" int rtj_launch_resolve(const rtj_launch_args *a, void *stream)
     cfg.numAttrs = 1;
     const cudaError_t e = cudaLaunchKernelEx(&cfg, rtj_resolve_kernel, a->d_ent, (const uint16_t *)a->d_chunk_last, (const uint32_t *)a->d_chunk_mask,
                                              a->d_src, a->f0, a->f1, nblk, (const rtj_dev_info *)a->d_info, a->slice, a->d_k3_in, a->d_k3_out,
-                                             a->d_desc, a->h_skips_seen);
+                                             a->d_desc, a->h_skips_seen, a->d_seq);
     if (e != cudaSuccess) return (int)e;
     return (int)cudaGetLastError();
 }

@@ -52,3 +52,21 @@ def decode(ctx: capi.BatchContext, b: DeviceBatch, carry: torch.Tensor | None = 
     ctx.set_format(b.fmt)
     ctx.decode_device(b.stream.data_ptr(), b.desc.data_ptr(), b.F, b.w, b.h, b.out.data_ptr(),
                       None if carry is None else carry.data_ptr(), st.cuda_stream)
+
+
+def upload_sequences(seqs, w: int, h: int, device: int | str = 0, fmt: int = 0, states=None):
+    """Several independent packet sequences [(stream, offsets), ...] as one batch (capi.plan_sequences): each is planned
+    with its own state (states: list of capi.State, advanced in place, or None).  Returns (DeviceBatch, seq_first[S + 1])."""
+    stream, _, desc, seq_first, _ = capi.plan_sequences(seqs, states)
+    return upload(stream, desc, w, h, device=device, fmt=fmt), seq_first
+
+
+def decode_sequences(ctx: capi.BatchContext, b: DeviceBatch, seq_first, carries=None,
+                     stream: torch.cuda.Stream | None = None) -> None:
+    """rtjgpu_decode_device_seq over a batch of upload_sequences: carries is a list of S tensors (the picture before each
+    sequence) or None entries (zeros), or None."""
+    st = stream if stream is not None else torch.cuda.current_stream(b.out.device)
+    ctx.set_format(b.fmt)
+    ptrs = None if carries is None else [None if c is None else c.data_ptr() for c in carries]
+    ctx.decode_device_seq(b.stream.data_ptr(), b.desc.data_ptr(), b.F, b.w, b.h, list(seq_first), b.out.data_ptr(), ptrs,
+                          st.cuda_stream)

@@ -311,6 +311,23 @@ int  rtjgpu_decode_device_rgb(rtjgpu_ctx *ctx, const uint8_t *d_stream, const rt
                               int w, int h, int kind, uint8_t *d_rgb, size_t row_pitch, size_t frame_pitch, int alpha,
                               const uint8_t *d_carry, uint8_t *d_last_yuv, void *cuda_stream);
 
+/* MANY INDEPENDENT STREAMS IN ONE CALL.  F frames = S independent sequences laid end to end in d_desc: sequence s is frames
+ * [seq_first[s], seq_first[s + 1]).  A skipped block whose position no earlier frame OF THE SAME SEQUENCE coded is taken from
+ * carries[s] (w*h*bytes-per-format picture, 8-byte aligned, device memory), or zeros where carries == NULL or carries[s] ==
+ * NULL.  seq_first and carries are HOST arrays (S + 1 and S entries), read before the call returns.  Everything else as
+ * rtjgpu_decode_device: d_out receives F frames, asynchronous on cuda_stream, every format.  Every sequence has the batch's
+ * picture size and format; RTJGPU_TABLE_CUSTOM frames of any sequence use the context's one custom set.  Plan each sequence
+ * with its own rtjgpu_state (rtjgpu_plan over its own offsets).  RTJGPU_E_ARG, before anything is launched, for S < 1 or
+ * S > F, seq_first[0] != 0, seq_first[S] != F, seq_first not strictly increasing (no empty sequence), or a misaligned
+ * carry.  S = 1 is rtjgpu_decode_device with carries[0]. */
+int  rtjgpu_decode_device_seq(rtjgpu_ctx *ctx, const uint8_t *d_stream, const rtjgpu_frame_desc *d_desc, int F, int w, int h,
+                              int S, const int *seq_first, uint8_t *d_out, const uint8_t *const *carries, void *cuda_stream);
+/* The same with rtjgpu_decode_device_rgb's fused converter; last_yuv (host array of S device pointers, or NULL; entries may
+ * be NULL, 16-byte aligned) receives the LAST frame of each sequence as planes: that sequence's next carry.  YUV420 only. */
+int  rtjgpu_decode_device_rgb_seq(rtjgpu_ctx *ctx, const uint8_t *d_stream, const rtjgpu_frame_desc *d_desc, int F, int w, int h,
+                                  int S, const int *seq_first, int kind, uint8_t *d_rgb, size_t row_pitch, size_t frame_pitch,
+                                  int alpha, const uint8_t *const *carries, uint8_t *const *last_yuv, void *cuda_stream);
+
 /* Host-buffer decode: packets in host memory in, frames in host memory out.
  * The batch is cut into chunks that move through pinned staging buffers with
  * cudaMemcpyAsync on several streams so that copies overlap the kernels.
@@ -348,7 +365,7 @@ int  rtjgpu_get_skip_counts(rtjgpu_ctx *ctx, uint32_t *counts, int F);
  * then the coefficients at zig-zag 1 and 2); else byte offset in the frame's payload (25 bits) and end-of-block
  * bound - 1 (6 bits above them).  After rtjgpu_scan_device these are K1's entries as made; after a decode, K3 has replaced
  * the marker of every skipped block whose last writer's entry is of the second kind (and was written under the same
- * tables) by a copy of that entry with bit 30 set.  What RTjpeg_decompress uses to copy back only the blocks a frame coded, and what
+ * tables) by a copy of that entry with bit 30 set -- the last writer in the same sequence (rtjgpu_decode_device_seq).  What RTjpeg_decompress uses to copy back only the blocks a frame coded, and what
  * the parity tests compare with the reference grammar's walk.  Synchronous. */
 int  rtjgpu_get_entries(rtjgpu_ctx *ctx, uint32_t *entries, size_t n);
 
