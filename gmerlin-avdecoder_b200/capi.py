@@ -10,6 +10,7 @@ from __future__ import annotations
 import ctypes as C
 import os
 import subprocess
+import weakref
 
 import numpy as np
 
@@ -127,6 +128,17 @@ def load_library() -> C.CDLL:
     L.rtjgpu_encoder_reset.argtypes = [vp]
     L.rtjgpu_encode_device.argtypes = [vp, vp, C.c_int, C.c_int, C.c_int, vp, C.c_size_t, vp, vp]
     L.rtjgpu_get_encode_info.argtypes = [vp, C.POINTER(C.c_uint64), C.POINTER(C.c_int)]
+    L.rtjgpu_seqenc_create.argtypes = [vp, C.POINTER(vp)]
+    L.rtjgpu_seqenc_destroy.argtypes = [vp]
+    L.rtjgpu_seqenc_destroy.restype = None
+    L.rtjgpu_seqenc_set_quality.argtypes = [vp, C.c_int]
+    L.rtjgpu_seqenc_set_intra.argtypes = [vp, C.c_int, C.c_int, C.c_int]
+    L.rtjgpu_seqenc_reset.argtypes = [vp]
+    L.rtjgpu_seqenc_key_count.argtypes = [vp]
+    L.rtjgpu_encode_device_seq.argtypes = [vp, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_int), C.POINTER(vp),
+                                           C.POINTER(vp), vp, C.c_size_t, vp, vp]
+    L.rtjgpu_encode_bound.argtypes = [C.c_int, C.c_int, C.c_int, C.c_int]
+    L.rtjgpu_encode_bound.restype = C.c_size_t
     L.RTjpeg_compress.argtypes = [vp, _u8p, C.POINTER(_u8p)]
     for name in CONVERTERS:
         getattr(L, name).argtypes = [vp, C.POINTER(_u8p), C.POINTER(_u8p)]
@@ -247,6 +259,11 @@ def plan_sequences(seqs, states=None):
     return out, offsets, np.concatenate(descs), np.array(seq_first, dtype=np.int64), states
 
 
+def encode_bound(fmt: int, w: int, h: int, F: int) -> int:
+    """rtjgpu_encode_bound: the most bytes F packets of format fmt and size w x h can take (0: not encodable)."""
+    return int(load_library().rtjgpu_encode_bound(fmt, w, h, F))
+
+
 def tables_for_quality(Q: int):
     """Host-only: (scaled[128], lb8, cb8) as RTjpeg_set_quality would leave them."""
     out = np.zeros(128, dtype=np.uint32)
@@ -349,9 +366,12 @@ class BatchContext:
             raise RTjpegError(rc or E_CUDA, f"rtjgpu_create(device={device}): no usable CUDA device, and no CPU fallback")
         self._h = h
         self.device = device
+        self._encoders = weakref.WeakSet()      # SeqEncoder handles of this context, freed with it
 
     def close(self) -> None:
         if getattr(self, "_h", None) is not None and self._h.value:
+            for e in list(getattr(self, "_encoders", ())):
+                e.close()
             self._L.rtjgpu_destroy(self._h)
             self._h = C.c_void_p()
 
@@ -396,6 +416,26 @@ class BatchContext:
                       cuda_stream: int | None = None) -> None:
         _check(self._L.rtjgpu_encode_device(self._h, C.c_void_p(d_frames), F, w, h, C.c_void_p(d_stream), capacity,
                                             C.c_void_p(d_offsets), C.c_void_p(cuda_stream or 0)), "rtjgpu_encode_device")
+
+    def seq_encoder(self, quality: int | None = None, key_rate: int = 0, lm: int = 0, cm: int = 0) -> "SeqEncoder":
+        """rtjgpu_seqenc_create: an encoder state of its own for encode_device_seq; quality None leaves a fresh instance's
+        (0, zero tables)."""
+        e = SeqEncoder(self)
+        self._encoders.add(e)
+        if quality is not None:
+            e.set_quality(quality)
+        if key_rate or lm or cm:
+            e.set_intra(key_rate, lm, cm)
+        return e
+
+    def encode_device_seq(self, F: int, w: int, h: int, seq_first, frames, encoders, d_stream: int, capacity: int,
+                          d_offsets: int, cuda_stream: int | None = None) -> None:
+        """rtjgpu_encode_device_seq: frames a list of S device addresses (each sequence's first picture), encoders a list
+        of S SeqEncoder (None: NULL, which the library refuses)."""
+        S = len(seq_first) - 1
+        _check(self._L.rtjgpu_encode_device_seq(self._h, F, w, h, S, _int_array(seq_first), _ptr_array(frames),
+                                                _ptr_array([None if e is None else e._h.value for e in encoders]), C.c_void_p(d_stream), capacity,
+                                                C.c_void_p(d_offsets), C.c_void_p(cuda_stream or 0)), "rtjgpu_encode_device_seq")
 
     def encode_info(self):
         b, o = C.c_uint64(), C.c_int()
@@ -486,6 +526,36 @@ class BatchContext:
 
     def launch_count(self) -> int:
         return int(self._L.rtjgpu_launch_count(self._h))
+
+
+class SeqEncoder:
+    """rtjgpu_seqenc: one stream's encoder state (tables, key counter, blocks last sent), bound to a BatchContext."""
+
+    def __init__(self, ctx: BatchContext):
+        self._L = ctx._L
+        h = C.c_void_p()
+        _check(self._L.rtjgpu_seqenc_create(ctx._h, C.byref(h)), "rtjgpu_seqenc_create")
+        self._h = h
+
+    def close(self) -> None:
+        if getattr(self, "_h", None) is not None and self._h.value:
+            self._L.rtjgpu_seqenc_destroy(self._h)
+            self._h = C.c_void_p()
+
+    __del__ = close
+
+    def set_quality(self, quality: int) -> None:
+        _check(self._L.rtjgpu_seqenc_set_quality(self._h, quality), "rtjgpu_seqenc_set_quality")
+
+    def set_intra(self, key_rate: int, lm: int = 0, cm: int = 0) -> None:
+        _check(self._L.rtjgpu_seqenc_set_intra(self._h, key_rate, lm, cm), "rtjgpu_seqenc_set_intra")
+
+    def reset(self) -> None:
+        _check(self._L.rtjgpu_seqenc_reset(self._h), "rtjgpu_seqenc_reset")
+
+    @property
+    def key_count(self) -> int:
+        return int(self._L.rtjgpu_seqenc_key_count(self._h))
 
 
 # Level 1 ----------------------------------------------------------------------

@@ -121,6 +121,13 @@ struct rtjgpu_ctx {
     uint64_t      *d_enc_total = nullptr;
     uint64_t      *h_enc_total = nullptr;     /* pinned */
     void          *enc_stream = nullptr;
+    /* rtjgpu_encode_device_seq: the multipliers of every quality (row 0: the zero tables of a fresh instance), made at the
+     * first rtjgpu_seqenc_create; the run table, sequence records and frame words of a call (device copy) */
+    int32_t       *d_enc_qt_all = nullptr;
+    int            enc_lb8_all[256] = {}, enc_cb8_all[256] = {};
+    uint8_t       *d_enc_seq = nullptr;       size_t enc_seq_cap = 0;      /* bytes */
+    uint64_t       enc_seq_calls = 0;         /* stamps the handles of a call: one seen twice is a duplicate */
+    std::vector<rtj_enc_run> enc_runs;        /* host scratch of a call */
     uint64_t       host_bad = 0;              /* overrun frames seen by the current rtjgpu_decode_host call */
     uint32_t      *h_host_skips = nullptr;    size_t host_skips_cap = 0;   /* pinned: per-frame skip counts of that call */
     int            host_F = 0;
@@ -534,33 +541,49 @@ int seq_check(int F, const SeqIn &q)
     return RTJGPU_OK;
 }
 
-/* The device copy of a layout of S > 1 sequences, in the workspace: [F] RTJ_SEQ words, then [S] carry pointers, then
- * [S] last_yuv pointers.  It goes up with cudaMemcpyAsync on the launch stream, staged in one of two pinned buffers taken
- * in turn; a buffer is written again only once its previous copy is done, and the caller's arrays are not read after
- * this returns. */
-int seq_upload(rtjgpu_ctx *ctx, Workspace *ws, int F, const SeqIn &q, cudaStream_t st, SeqDev *out)
+/* Small per-call tables go up with cudaMemcpyAsync on the launch stream, staged in one of two pinned buffers taken in
+ * turn; a buffer is written again only once its previous copy is done, and the caller's arrays are not read after the
+ * call returns.  stage_begin hands out the buffer to fill (bytes of it), stage_end copies it to d_dst. */
+int stage_begin(rtjgpu_ctx *ctx, size_t bytes, uint8_t **h)
 {
-    const size_t words = ((size_t)F * sizeof(uint32_t) + 7) & ~(size_t)7, ptrs = (size_t)q.S * sizeof(void *);
-    const size_t bytes = words + 2 * ptrs;
     const int t = ctx->seq_turn;
     if (!ctx->seq_copied[t]) CK(ctx, cudaEventCreateWithFlags(&ctx->seq_copied[t], cudaEventDisableTiming));
     if (ctx->seq_pending[t]) {
         CK(ctx, cudaEventSynchronize(ctx->seq_copied[t]));
         ctx->seq_pending[t] = false;
     }
-    int rc = grow_pinned(ctx, &ctx->h_seq[t], &ctx->h_seq_cap[t], bytes);
-    if (rc) return rc;
-    if ((rc = grow_device(ctx, &ws->d_seq, &ws->seq_cap, bytes))) return rc;
-    uint32_t *hw = reinterpret_cast<uint32_t *>(ctx->h_seq[t]);
-    for (int s = 0; s < q.S; s++)
-        for (int f = q.first[s]; f < q.first[s + 1]; f++) hw[f] = RTJ_SEQ(q.first[s], s);
-    const uint8_t **hc = reinterpret_cast<const uint8_t **>(ctx->h_seq[t] + words);
-    uint8_t **hl = reinterpret_cast<uint8_t **>(ctx->h_seq[t] + words + ptrs);
-    for (int s = 0; s < q.S; s++) { hc[s] = q.carry(s); hl[s] = q.last(s); }
-    CK(ctx, cudaMemcpyAsync(ws->d_seq, ctx->h_seq[t], bytes, cudaMemcpyHostToDevice, st));
+    const int rc = grow_pinned(ctx, &ctx->h_seq[t], &ctx->h_seq_cap[t], bytes);
+    *h = ctx->h_seq[t];
+    return rc;
+}
+
+int stage_end(rtjgpu_ctx *ctx, void *d_dst, size_t bytes, cudaStream_t st)
+{
+    const int t = ctx->seq_turn;
+    CK(ctx, cudaMemcpyAsync(d_dst, ctx->h_seq[t], bytes, cudaMemcpyHostToDevice, st));
     CK(ctx, cudaEventRecord(ctx->seq_copied[t], st));
     ctx->seq_pending[t] = true;
     ctx->seq_turn = t ^ 1;
+    return RTJGPU_OK;
+}
+
+/* The device copy of a layout of S > 1 sequences, in the workspace: [F] RTJ_SEQ words, then [S] carry pointers, then
+ * [S] last_yuv pointers. */
+int seq_upload(rtjgpu_ctx *ctx, Workspace *ws, int F, const SeqIn &q, cudaStream_t st, SeqDev *out)
+{
+    const size_t words = ((size_t)F * sizeof(uint32_t) + 7) & ~(size_t)7, ptrs = (size_t)q.S * sizeof(void *);
+    const size_t bytes = words + 2 * ptrs;
+    uint8_t *h;
+    int rc = stage_begin(ctx, bytes, &h);
+    if (rc) return rc;
+    if ((rc = grow_device(ctx, &ws->d_seq, &ws->seq_cap, bytes))) return rc;
+    uint32_t *hw = reinterpret_cast<uint32_t *>(h);
+    for (int s = 0; s < q.S; s++)
+        for (int f = q.first[s]; f < q.first[s + 1]; f++) hw[f] = RTJ_SEQ(q.first[s], s);
+    const uint8_t **hc = reinterpret_cast<const uint8_t **>(h + words);
+    uint8_t **hl = reinterpret_cast<uint8_t **>(h + words + ptrs);
+    for (int s = 0; s < q.S; s++) { hc[s] = q.carry(s); hl[s] = q.last(s); }
+    if ((rc = stage_end(ctx, ws->d_seq, bytes, st))) return rc;
     out->seq = reinterpret_cast<const uint32_t *>(ws->d_seq);
     out->carries = reinterpret_cast<const uint8_t *const *>(ws->d_seq + words);
     out->last_yuvs = reinterpret_cast<uint8_t *const *>(ws->d_seq + words + ptrs);
@@ -637,6 +660,28 @@ int decode_device_rgb(rtjgpu_ctx *ctx, const uint8_t *d_stream, const rtjgpu_fra
     ctx->last_F = F;
     ctx->last_stream = cuda_stream;
     return rc;
+}
+
+/* The encoder's workspace for F pictures of nblk blocks, shared by rtjgpu_encode_device and rtjgpu_encode_device_seq
+ * (both on the stream of the call that uses it) */
+int enc_reserve(rtjgpu_ctx *ctx, size_t nblk, int F)
+{
+    if (!ctx->d_enc_total) {
+        CK(ctx, cudaMalloc(&ctx->d_enc_total, 2 * sizeof(uint64_t)));
+        CK(ctx, cudaMallocHost(&ctx->h_enc_total, 2 * sizeof(uint64_t)));
+    }
+    const size_t nb = nblk * (size_t)F;
+    if (nb > ctx->enc_blocks_cap) {
+        if (ctx->d_enc_slots) cudaFree(ctx->d_enc_slots);
+        if (ctx->d_enc_lens) cudaFree(ctx->d_enc_lens);
+        if (ctx->d_enc_boff) cudaFree(ctx->d_enc_boff);
+        ctx->d_enc_slots = nullptr; ctx->d_enc_lens = nullptr; ctx->d_enc_boff = nullptr; ctx->enc_blocks_cap = 0;
+        CK(ctx, cudaMalloc(&ctx->d_enc_slots, nb * 64));
+        CK(ctx, cudaMalloc(&ctx->d_enc_lens, nb));
+        CK(ctx, cudaMalloc(&ctx->d_enc_boff, nb * sizeof(uint32_t)));
+        ctx->enc_blocks_cap = nb;
+    }
+    return grow_device(ctx, &ctx->d_enc_fsize, &ctx->enc_frames_cap, (size_t)F);
 }
 
 } // namespace
@@ -743,6 +788,8 @@ void rtjgpu_destroy(rtjgpu_ctx *ctx)
     if (ctx->d_enc_fsize) cudaFree(ctx->d_enc_fsize);
     if (ctx->d_enc_total) cudaFree(ctx->d_enc_total);
     if (ctx->h_enc_total) cudaFreeHost(ctx->h_enc_total);
+    if (ctx->d_enc_qt_all) cudaFree(ctx->d_enc_qt_all);
+    if (ctx->d_enc_seq) cudaFree(ctx->d_enc_seq);
     if (ctx->d_tables) cudaFree(ctx->d_tables);
     if (ctx->h_info_reset) cudaFreeHost(ctx->h_info_reset);
     if (ctx->h_info) cudaFreeHost(ctx->h_info);
@@ -861,18 +908,7 @@ int rtjgpu_encode_device(rtjgpu_ctx *ctx, const uint8_t *d_frames, int F, int w,
         CK(ctx, cudaMemsetAsync(ctx->d_enc_total, 0, 2 * sizeof(uint64_t), st));
         return RTJGPU_OK;
     }
-    const size_t nb = nblk * (size_t)F;
-    if (nb > ctx->enc_blocks_cap) {
-        if (ctx->d_enc_slots) cudaFree(ctx->d_enc_slots);
-        if (ctx->d_enc_lens) cudaFree(ctx->d_enc_lens);
-        if (ctx->d_enc_boff) cudaFree(ctx->d_enc_boff);
-        ctx->d_enc_slots = nullptr; ctx->d_enc_lens = nullptr; ctx->d_enc_boff = nullptr; ctx->enc_blocks_cap = 0;
-        CK(ctx, cudaMalloc(&ctx->d_enc_slots, nb * 64));
-        CK(ctx, cudaMalloc(&ctx->d_enc_lens, nb));
-        CK(ctx, cudaMalloc(&ctx->d_enc_boff, nb * sizeof(uint32_t)));
-        ctx->enc_blocks_cap = nb;
-    }
-    if ((rc = grow_device(ctx, &ctx->d_enc_fsize, &ctx->enc_frames_cap, (size_t)F))) return rc;
+    if ((rc = enc_reserve(ctx, nblk, F))) return rc;
     rtj_encode_args a;
     a.d_frames = d_frames; a.F = F; a.w = w; a.h = h; a.fmt = ctx->format;
     a.d_qt = ctx->d_enc_qt; a.lb8 = ctx->enc_lb8; a.cb8 = ctx->enc_cb8; a.quality = ctx->enc_quality;
@@ -896,6 +932,193 @@ int rtjgpu_get_encode_info(rtjgpu_ctx *ctx, uint64_t *bytes, int *overflow)
     CK(ctx, cudaStreamSynchronize(st));
     if (bytes) *bytes = ctx->h_enc_total[0];
     if (overflow) *overflow = ctx->h_enc_total[1] != 0;
+    return RTJGPU_OK;
+}
+
+/* ---- encoder states of their own: rtjgpu_encode_device_seq ---------------------------------------------- */
+
+struct rtjgpu_seqenc {
+    rtjgpu_ctx *ctx = nullptr;
+    int         device = 0;                 /* ctx's, kept for rtjgpu_seqenc_destroy */
+    int         quality = 0, key_rate = 0, key_count = 0, lm = 0, cm = 0;
+    bool        cleared = true;             /* the stored blocks are zeros: a run that starts here does not read them */
+    int         w = 0, h = 0, fmt = -1;     /* geometry of the stored blocks */
+    int16_t    *d_old = nullptr;  size_t old_cap = 0;    /* [nblk][64], allocated at the first inter call */
+    uint64_t    call = 0;                   /* rtjgpu_ctx::enc_seq_calls of the last call that named it */
+};
+
+int rtjgpu_seqenc_create(rtjgpu_ctx *ctx, rtjgpu_seqenc **out)
+{
+    if (!ctx || !out) return RTJGPU_E_ARG;
+    *out = nullptr;
+    if (!ctx->d_enc_qt_all) {
+        CK(ctx, cudaSetDevice(ctx->device));
+        std::vector<int32_t> qt(256 * 128, 0);
+        for (int q = 1; q <= 255; q++) rtj_encoder_table_from_quality(q, &qt[(size_t)q * 128], &ctx->enc_lb8_all[q], &ctx->enc_cb8_all[q]);
+        int32_t *d = nullptr;
+        CK(ctx, cudaMalloc(&d, qt.size() * sizeof(int32_t)));
+        const cudaError_t e = cudaMemcpy(d, qt.data(), qt.size() * sizeof(int32_t), cudaMemcpyHostToDevice);
+        if (e != cudaSuccess) { cudaFree(d); ctx->last_cuda = (int)e; return RTJGPU_E_CUDA; }
+        ctx->d_enc_qt_all = d;
+    }
+    rtjgpu_seqenc *e = new (std::nothrow) rtjgpu_seqenc();
+    if (!e) return RTJGPU_E_NOMEM;
+    e->ctx = ctx;
+    e->device = ctx->device;
+    *out = e;
+    return RTJGPU_OK;
+}
+
+void rtjgpu_seqenc_destroy(rtjgpu_seqenc *e)
+{
+    if (!e) return;
+    if (e->d_old) {
+        cudaSetDevice(e->device);
+        cudaFree(e->d_old);                 /* waits for the work that may still read or write it */
+    }
+    delete e;
+}
+
+int rtjgpu_seqenc_set_quality(rtjgpu_seqenc *e, int quality)
+{
+    if (!e) return RTJGPU_E_ARG;
+    e->quality = quality < 1 ? 1 : quality > 255 ? 255 : quality;
+    return RTJGPU_OK;
+}
+
+int rtjgpu_seqenc_set_intra(rtjgpu_seqenc *e, int key_rate, int lm, int cm)
+{
+    if (!e) return RTJGPU_E_ARG;
+    e->key_rate = key_rate < 0 ? 0 : key_rate > 255 ? 255 : key_rate;
+    e->lm = lm < 0 ? 0 : lm > 16 ? 16 : lm;
+    e->cm = cm < 0 ? 0 : cm > 16 ? 16 : cm;
+    e->cleared = true;                      /* lib/RTjpeg.c:2488, as rtjgpu_encoder_set_intra */
+    return RTJGPU_OK;
+}
+
+int rtjgpu_seqenc_reset(rtjgpu_seqenc *e)
+{
+    if (!e) return RTJGPU_E_ARG;
+    e->key_count = 0;
+    e->cleared = true;
+    return RTJGPU_OK;
+}
+
+int rtjgpu_seqenc_key_count(const rtjgpu_seqenc *e) { return e ? e->key_count : RTJGPU_E_ARG; }
+
+size_t rtjgpu_encode_bound(int format, int w, int h, int F)
+{
+    if ((format != RTJ_YUV420 && format != RTJ_YUV422) || w <= 0 || h <= 0 || (w & 15) || (h & 15) || w > 65535 || h > 65535
+        || F < 0)
+        return 0;
+    /* a block takes at most 64 bytes (DC byte and one byte per place, RTjpeg_b2s :109-155); header and block bytes are a
+     * multiple of 4 already, so no packet needs padding */
+    return (size_t)F * (RTJPEG_B200_HEADER_BYTES + 64 * (size_t)RTJ_FMT_NBLK(format, w, h));
+}
+
+int rtjgpu_encode_device_seq(rtjgpu_ctx *ctx, int F, int w, int h, int S, const int *seq_first,
+                             const uint8_t *const *frames, rtjgpu_seqenc *const *encs,
+                             uint8_t *d_stream, size_t capacity, uint64_t *d_offsets, void *cuda_stream)
+{
+    if (!ctx) return RTJGPU_E_ARG;
+    if (ctx->format != RTJ_YUV420 && ctx->format != RTJ_YUV422) return RTJGPU_E_FORMAT;
+    if (w <= 0 || h <= 0 || (w & 15) || (h & 15) || w > 65535 || h > 65535) return RTJGPU_E_SIZE;
+    if (F > RTJGPU_MAX_FRAMES_PER_BATCH) return RTJGPU_E_TOOBIG;
+    SeqIn q;
+    q.S = S; q.first = seq_first;
+    if (F < 1 || !seq_first || seq_check(F, q) || !frames || !encs || !d_stream || !d_offsets || ((uintptr_t)d_stream & 3))
+        return RTJGPU_E_ARG;
+    const uint64_t call = ++ctx->enc_seq_calls;
+    for (int s = 0; s < S; s++) {
+        rtjgpu_seqenc *e = encs[s];
+        if (!frames[s] || ((uintptr_t)frames[s] & 7) || !e || e->ctx != ctx || e->call == call) return RTJGPU_E_ARG;
+        e->call = call;
+    }
+    CK(ctx, cudaSetDevice(ctx->device));
+    cudaStream_t st = (cudaStream_t)cuda_stream;
+    const size_t nblk = (size_t)RTJ_FMT_NBLK(ctx->format, w, h);
+    int rc = enc_reserve(ctx, nblk, F);
+    if (rc) return rc;
+    for (int s = 0; s < S; s++) {
+        rtjgpu_seqenc *e = encs[s];
+        if (e->w != w || e->h != h || e->fmt != ctx->format) { e->w = w; e->h = h; e->fmt = ctx->format; e->cleared = true; }
+        if (e->key_rate && e->old_cap < nblk * 64) {
+            if (e->d_old) cudaFree(e->d_old);
+            e->d_old = nullptr; e->old_cap = 0;
+            CK(ctx, cudaMalloc(&e->d_old, nblk * 64 * sizeof(int16_t)));
+            e->old_cap = nblk * 64;
+            e->cleared = true;
+        }
+    }
+
+    /* Runs: every sequence cut where its key counter is 0 -- there RTjpeg_compress clears the stored blocks (:3505) --,
+     * intra sequences one picture a run; the counter and the header bytes follow RTjpeg_compress picture by picture. */
+    const size_t seqs_bytes = (size_t)S * sizeof(rtj_enc_seq);
+    const size_t words_bytes = ((size_t)F * sizeof(uint32_t) + 7) & ~(size_t)7;
+    std::vector<rtj_enc_run> &runs = ctx->enc_runs;
+    runs.clear();
+    int n_intra = 0;
+    for (int s = 0; s < S; s++)
+        if (!encs[s]->key_rate) n_intra += seq_first[s + 1] - seq_first[s];
+    runs.resize((size_t)n_intra);
+    const size_t bytes_bound = seqs_bytes + words_bytes + ((size_t)F + S) * sizeof(rtj_enc_run);
+    uint8_t *hb;
+    if ((rc = stage_begin(ctx, bytes_bound, &hb))) return rc;
+    rtj_enc_seq *hs = reinterpret_cast<rtj_enc_seq *>(hb);
+    uint32_t *hw = reinterpret_cast<uint32_t *>(hb + seqs_bytes);
+    int at_intra = 0;
+    for (int s = 0; s < S; s++) {
+        const rtjgpu_seqenc *e = encs[s];
+        const int a = seq_first[s], b = seq_first[s + 1];
+        rtj_enc_seq &r = hs[s];
+        r.d_frames = frames[s]; r.d_old = e->d_old; r.first = a; r.quality = e->quality;
+        r.lb8 = ctx->enc_lb8_all[e->quality]; r.cb8 = ctx->enc_cb8_all[e->quality]; r.lmask = e->lm; r.cmask = e->cm;
+        if (!e->key_rate) {
+            for (int f = a; f < b; f++) {
+                runs[at_intra++] = rtj_enc_run{f, f + 1, (uint32_t)s};
+                hw[f] = RTJ_ENC_FRAME(e->quality, 0);
+            }
+            continue;
+        }
+        int c = e->key_count, f0 = a;
+        uint32_t flags = c != 0 && !e->cleared ? RTJ_ENC_RUN_CONT : 0u;
+        for (int f = a; f < b; f++) {
+            if (c == 0 && f > f0) {
+                runs.push_back(rtj_enc_run{f0, f, (uint32_t)s | flags});
+                f0 = f; flags = 0;
+            }
+            hw[f] = RTJ_ENC_FRAME(e->quality, c);
+            c = c + 1 > e->key_rate ? 0 : c + 1;
+        }
+        runs.push_back(rtj_enc_run{f0, b, (uint32_t)s | flags | RTJ_ENC_RUN_LAST});
+    }
+    const size_t runs_bytes = runs.size() * sizeof(rtj_enc_run);
+    const size_t bytes = seqs_bytes + words_bytes + runs_bytes;
+    memcpy(hb + seqs_bytes + words_bytes, runs.data(), runs_bytes);
+    if ((rc = grow_device(ctx, &ctx->d_enc_seq, &ctx->enc_seq_cap, bytes))) return rc;
+    if ((rc = stage_end(ctx, ctx->d_enc_seq, bytes, st))) return rc;
+
+    rtj_encode_args a;
+    memset(&a, 0, sizeof(a));
+    a.F = F; a.w = w; a.h = h; a.fmt = ctx->format; a.d_qt = ctx->d_enc_qt_all;
+    a.d_slots = ctx->d_enc_slots; a.d_lens = ctx->d_enc_lens; a.d_boff = ctx->d_enc_boff;
+    a.d_fsize = ctx->d_enc_fsize; a.d_stream = d_stream; a.capacity = capacity; a.d_offsets = d_offsets;
+    a.d_total = ctx->d_enc_total;
+    ctx->enc_stream = cuda_stream;
+    const int n = rtj_launch_encode_seq(&a, reinterpret_cast<const rtj_enc_run *>(ctx->d_enc_seq + seqs_bytes + words_bytes),
+                                        n_intra, (int)runs.size() - n_intra, reinterpret_cast<const rtj_enc_seq *>(ctx->d_enc_seq),
+                                        reinterpret_cast<const uint32_t *>(ctx->d_enc_seq + seqs_bytes), cuda_stream);
+    if (n < 0) { ctx->last_cuda = -n; return RTJGPU_E_CUDA; }
+    ctx->launches += (uint64_t)n;
+    /* the handles move on as RTjpeg_compress would have, whether the packets fit or not */
+    for (int s = 0; s < S; s++) {
+        rtjgpu_seqenc *e = encs[s];
+        if (!e->key_rate) continue;
+        int c = e->key_count;
+        for (int f = seq_first[s]; f < seq_first[s + 1]; f++) c = c + 1 > e->key_rate ? 0 : c + 1;
+        e->key_count = c;
+        e->cleared = false;
+    }
     return RTJGPU_OK;
 }
 

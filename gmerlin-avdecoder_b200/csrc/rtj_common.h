@@ -218,6 +218,30 @@ typedef struct rtj_encode_args {
     uint64_t      *d_total;        /* out: [2] bytes needed, 1 if they did not fit */
 } rtj_encode_args;
 int rtj_launch_encode(const rtj_encode_args *a, void *stream);      /* returns launches (> 0) or -cudaError */
+
+/* rtjgpu_encode_device_seq: S sequences, each with its own encoder state, laid end to end in the output frames.  E1 takes
+ * a table of runs instead of one key period: a run is frames [f0, f1) of one sequence that chain their stored blocks, cut
+ * where that sequence's key counter is 0 (intra sequences: one picture a run). */
+typedef struct rtj_enc_run {
+    int32_t  f0, f1;               /* output frames */
+    uint32_t seq;                  /* sequence index | RTJ_ENC_RUN_* */
+} rtj_enc_run;
+#define RTJ_ENC_RUN_CONT  0x80000000u   /* starts from the handle's stored blocks (else from zeros) */
+#define RTJ_ENC_RUN_LAST  0x40000000u   /* the sequence's last run: leaves its blocks in the handle */
+#define RTJ_ENC_RUN_INDEX 0x0000FFFFu
+typedef struct rtj_enc_seq {
+    const uint8_t *d_frames;       /* the sequence's first picture; its pictures are consecutive */
+    int16_t       *d_old;          /* [nblk][64] the handle's stored blocks (inter sequences) */
+    int32_t        first;          /* output frame of the first picture */
+    int32_t        quality;        /* row of the all-quality multiplier table */
+    int32_t        lb8, cb8, lmask, cmask;
+} rtj_enc_seq;
+/* Per output frame: the header's quality and key bytes (RTJ_ENC_FRAME(quality, key)). */
+#define RTJ_ENC_FRAME(q, key) ((uint32_t)(q) | (uint32_t)(key) << 8)
+/* a->d_qt: [256][128] the multipliers of every quality (row 0 zeros); a->d_frames, quality, lb8 ... unused.  Runs
+ * [0, n_intra) are intra, [n_intra, n_intra + n_inter) inter. */
+int rtj_launch_encode_seq(const rtj_encode_args *a, const rtj_enc_run *d_runs, int n_intra, int n_inter,
+                          const rtj_enc_seq *d_seqs, const uint32_t *d_frame_words, void *stream);
 int rtj_kernels_init(void);   /* one-time function attributes (dynamic shared memory opt-in) */
 
 #ifdef __cplusplus

@@ -69,10 +69,13 @@ __device__ __forceinline__ size_t block_at(int fmt, int i, int w, int h, int &pi
 
 } // namespace
 
-/* INTER: pictures are compared with the blocks last sent (key_rate != 0); false: none of that is compiled in */
-template <bool INTER>
+/* INTER: pictures are compared with the blocks last sent (key_rate != 0); false: none of that is compiled in.
+ * SEQ: rtjgpu_encode_device_seq -- run blockIdx.y is runs[blockIdx.y], and its sequence's record gives pictures, stored
+ * blocks, tables and masks; false: one sequence, runs cut by period / first_boundary, runs and seqs unused. */
+template <bool INTER, bool SEQ = false>
 __global__ void __launch_bounds__(EN_THREADS, INTER ? 3 : 4)
-rtj_encode_blocks_kernel(const rtj_encode_args A, int nblk, int nruns, int period, int first_boundary)
+rtj_encode_blocks_kernel(const rtj_encode_args A, int nblk, int nruns, int period, int first_boundary,
+                         const rtj_enc_run *__restrict__ runs, const rtj_enc_seq *__restrict__ seqs)
 {
     __shared__ int32_t s_qt[128];                           /* the quantiser's multipliers: read 64 times a block */
     /* a row a thread: the block's token values in zig-zag order, then -- in place -- its bytes (RTjpeg_b2s never writes more
@@ -81,16 +84,19 @@ rtj_encode_blocks_kernel(const rtj_encode_args A, int nblk, int nruns, int perio
     /* INTER: the quantised block itself, two values a word as the stored blocks hold them, for the comparison (kept out of
      * the registers: the transform's 64 intermediate values live there) */
     __shared__ uint32_t s_q[INTER ? EN_THREADS : 1][33];
-    s_qt[threadIdx.x] = A.d_qt[threadIdx.x];
+    const int run = blockIdx.y;
+    const rtj_enc_run R = SEQ ? runs[run] : rtj_enc_run{};
+    const rtj_enc_seq *const Q = SEQ ? seqs + (R.seq & RTJ_ENC_RUN_INDEX) : nullptr;
+    s_qt[threadIdx.x] = SEQ ? A.d_qt[Q->quality * 128 + threadIdx.x] : A.d_qt[threadIdx.x];
     static_assert(EN_THREADS == 128, "one multiplier a thread");
     __syncthreads();
     const int b = blockIdx.x * EN_THREADS + threadIdx.x;
-    const int run = blockIdx.y;
     if (b >= nblk) return;
     /* the pictures of this run: [f0, f1).  Run 0 may continue a run of the call before (key_count0 != 0). */
     constexpr bool inter = INTER;
     int f0, f1;
-    if (!inter) { f0 = run; f1 = run + 1; }
+    if (SEQ) { f0 = R.f0; f1 = R.f1; }
+    else if (!inter) { f0 = run; f1 = run + 1; }
     else if (first_boundary == 0) { f0 = run * period; f1 = min(f0 + period, A.F); }
     else if (run == 0) { f0 = 0; f1 = min(first_boundary, A.F); }
     else { f0 = first_boundary + (run - 1) * period; f1 = min(f0 + period, A.F); }
@@ -99,18 +105,22 @@ rtj_encode_blocks_kernel(const rtj_encode_args A, int nblk, int nruns, int perio
     const size_t at = block_at(A.fmt, b, A.w, A.h, pitch);
     const bool luma = A.fmt == RTJ_YUV420 ? (b % 6) < 4 : (b & 3) < 2;
     const int32_t *qt = s_qt + (luma ? 0 : 64);
-    const int bt8 = luma ? A.lb8 : A.cb8, mask = luma ? A.lmask : A.cmask;
+    const int bt8 = SEQ ? (luma ? Q->lb8 : Q->cb8) : (luma ? A.lb8 : A.cb8);
+    const int mask = SEQ ? (luma ? Q->lmask : Q->cmask) : (luma ? A.lmask : A.cmask);
+    /* SEQ: output frame f is picture f - Q->first of the sequence's pictures */
+    const uint8_t *const pics = SEQ ? Q->d_frames : nullptr;
+    const int fbase = SEQ ? Q->first : 0;
 
     /* the block last sent here, two coefficients per register */
     uint32_t old[INTER ? 32 : 1];
-    const bool continues = inter && run == 0 && A.key_count0 != 0;
+    const bool continues = inter && (SEQ ? (R.seq & RTJ_ENC_RUN_CONT) != 0 : run == 0 && A.key_count0 != 0);
     if (INTER) {
 #pragma unroll
-        for (int k = 0; k < 32; k++) old[k] = continues ? reinterpret_cast<const uint32_t *>(A.d_old + (size_t)b * 64)[k] : 0u;
+        for (int k = 0; k < 32; k++) old[k] = continues ? reinterpret_cast<const uint32_t *>((SEQ ? Q->d_old : A.d_old) + (size_t)b * 64)[k] : 0u;
     }
 
     for (int f = f0; f < f1; f++) {
-        const uint8_t *src = A.d_frames + (size_t)f * fsz + at;
+        const uint8_t *src = SEQ ? pics + (size_t)(f - fbase) * fsz + at : A.d_frames + (size_t)f * fsz + at;
         int ws[64];
 #pragma unroll
         for (int r = 0; r < 8; r++) {
@@ -194,10 +204,10 @@ rtj_encode_blocks_kernel(const rtj_encode_args A, int nblk, int nruns, int perio
         for (int k = 0; k < (co + 3) >> 2; k++) reinterpret_cast<uint32_t *>(slot)[k] = s_zz[threadIdx.x][k];
         A.d_lens[(size_t)f * nblk + b] = (uint8_t)co;
     }
-    /* the run that ends the batch leaves its blocks for the next call */
-    if (INTER && f1 == A.F) {
+    /* the run that ends the batch (SEQ: its sequence) leaves its blocks for the next call */
+    if (INTER && (SEQ ? (R.seq & RTJ_ENC_RUN_LAST) != 0 : f1 == A.F)) {
 #pragma unroll
-        for (int k = 0; k < (INTER ? 32 : 0); k++) reinterpret_cast<uint32_t *>(A.d_old + (size_t)b * 64)[k] = old[k];
+        for (int k = 0; k < (INTER ? 32 : 0); k++) reinterpret_cast<uint32_t *>((SEQ ? Q->d_old : A.d_old) + (size_t)b * 64)[k] = old[k];
     }
 }
 
@@ -266,8 +276,10 @@ rtj_encode_offsets_kernel(const uint32_t *__restrict__ fsize, int F, uint64_t *_
     }
 }
 
-extern "C" __global__ void __launch_bounds__(EN_THREADS)
-rtj_encode_gather_kernel(const rtj_encode_args A, int nblk, int period)
+/* SEQ: the header's quality and key bytes come from frame_words[f] (RTJ_ENC_FRAME) */
+template <bool SEQ = false>
+__global__ void __launch_bounds__(EN_THREADS)
+rtj_encode_gather_kernel(const rtj_encode_args A, int nblk, int period, const uint32_t *__restrict__ frame_words)
 {
     if (A.d_total[1]) return;                               /* the stream buffer is too small: nothing is written */
     const int f = blockIdx.y;
@@ -276,11 +288,13 @@ rtj_encode_gather_kernel(const rtj_encode_args A, int nblk, int period)
     if (b == 0) {
         /* RTjpeg_frameheader (include/RTjpeg.h:100-109), filled as RTjpeg_compress does (:3515-3522) */
         const uint32_t ds = A.d_fsize[f];
-        const int key = A.key_rate == 0 ? 0 : (A.key_count0 + f) % period;
+        const uint32_t fw = SEQ ? frame_words[f] : 0u;
+        const int key = SEQ ? (int)(fw >> 8) & 0xFF : A.key_rate == 0 ? 0 : (A.key_count0 + f) % period;
+        const int quality = SEQ ? (int)fw & 0xFF : A.quality;
         pkt[0] = (uint8_t)ds; pkt[1] = (uint8_t)(ds >> 8); pkt[2] = (uint8_t)(ds >> 16); pkt[3] = (uint8_t)(ds >> 24);
         pkt[4] = RTJPEG_B200_HEADER_BYTES; pkt[5] = 0;
         pkt[6] = (uint8_t)A.w; pkt[7] = (uint8_t)(A.w >> 8); pkt[8] = (uint8_t)A.h; pkt[9] = (uint8_t)(A.h >> 8);
-        pkt[10] = (uint8_t)A.quality; pkt[11] = (uint8_t)key;
+        pkt[10] = (uint8_t)quality; pkt[11] = (uint8_t)key;
         for (uint32_t k = ds; k < ((ds + 3u) & ~3u); k++) pkt[k] = 0;       /* the padding up to the next packet */
     }
     if (b >= nblk) return;
@@ -290,6 +304,25 @@ rtj_encode_gather_kernel(const rtj_encode_args A, int nblk, int period)
     const int n = A.d_lens[i];
     for (int k = 0; k < n; k++) dst[k] = slot[k];
 }
+
+namespace {
+
+/* E2, E3 and E4 behind E1: the same for both entry points but for where E4 takes its header bytes */
+template <bool SEQ>
+int launch_layout_and_gather(const rtj_encode_args *a, int nblk, int period, const uint32_t *frame_words, cudaStream_t st)
+{
+    const unsigned gx = (unsigned)((nblk + EN_THREADS - 1) / EN_THREADS);
+    cudaError_t e;
+    rtj_encode_layout_kernel<<<(unsigned)a->F, 256, 0, st>>>(a->d_lens, a->d_boff, a->d_fsize, nblk);
+    if ((e = cudaGetLastError()) != cudaSuccess) return -(int)e;
+    rtj_encode_offsets_kernel<<<1, 1024, 0, st>>>(a->d_fsize, a->F, a->d_offsets, a->d_total, a->capacity);
+    if ((e = cudaGetLastError()) != cudaSuccess) return -(int)e;
+    rtj_encode_gather_kernel<SEQ><<<dim3(gx, (unsigned)a->F), EN_THREADS, 0, st>>>(*a, nblk, period, frame_words);
+    if ((e = cudaGetLastError()) != cudaSuccess) return -(int)e;
+    return 3;
+}
+
+} // namespace
 
 extern "C" int rtj_launch_encode(const rtj_encode_args *a, void *stream)
 {
@@ -303,15 +336,33 @@ extern "C" int rtj_launch_encode(const rtj_encode_args *a, void *stream)
     else if (first_boundary == 0) nruns = (a->F + period - 1) / period;
     else nruns = 1 + (a->F > first_boundary ? (a->F - first_boundary + period - 1) / period : 0);
     const unsigned gx = (unsigned)((nblk + EN_THREADS - 1) / EN_THREADS);
-    if (inter) rtj_encode_blocks_kernel<true><<<dim3(gx, (unsigned)nruns), EN_THREADS, 0, st>>>(*a, nblk, nruns, period, first_boundary);
-    else rtj_encode_blocks_kernel<false><<<dim3(gx, (unsigned)nruns), EN_THREADS, 0, st>>>(*a, nblk, nruns, period, first_boundary);
+    if (inter) rtj_encode_blocks_kernel<true><<<dim3(gx, (unsigned)nruns), EN_THREADS, 0, st>>>(*a, nblk, nruns, period, first_boundary, nullptr, nullptr);
+    else rtj_encode_blocks_kernel<false><<<dim3(gx, (unsigned)nruns), EN_THREADS, 0, st>>>(*a, nblk, nruns, period, first_boundary, nullptr, nullptr);
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return -(int)e;
-    rtj_encode_layout_kernel<<<(unsigned)a->F, 256, 0, st>>>(a->d_lens, a->d_boff, a->d_fsize, nblk);
-    if ((e = cudaGetLastError()) != cudaSuccess) return -(int)e;
-    rtj_encode_offsets_kernel<<<1, 1024, 0, st>>>(a->d_fsize, a->F, a->d_offsets, a->d_total, a->capacity);
-    if ((e = cudaGetLastError()) != cudaSuccess) return -(int)e;
-    rtj_encode_gather_kernel<<<dim3(gx, (unsigned)a->F), EN_THREADS, 0, st>>>(*a, nblk, period);
-    if ((e = cudaGetLastError()) != cudaSuccess) return -(int)e;
-    return 4;
+    const int n = launch_layout_and_gather<false>(a, nblk, period, nullptr, st);
+    return n < 0 ? n : 1 + n;
+}
+
+extern "C" int rtj_launch_encode_seq(const rtj_encode_args *a, const rtj_enc_run *d_runs, int n_intra, int n_inter,
+                                     const rtj_enc_seq *d_seqs, const uint32_t *d_frame_words, void *stream)
+{
+    cudaStream_t st = (cudaStream_t)stream;
+    const int nblk = RTJ_FMT_NBLK(a->fmt, a->w, a->h);
+    const unsigned gx = (unsigned)((nblk + EN_THREADS - 1) / EN_THREADS);
+    int launches = 0;
+    cudaError_t e;
+    if (n_intra) {
+        rtj_encode_blocks_kernel<false, true><<<dim3(gx, (unsigned)n_intra), EN_THREADS, 0, st>>>(*a, nblk, n_intra, 0, 0, d_runs, d_seqs);
+        if ((e = cudaGetLastError()) != cudaSuccess) return -(int)e;
+        launches++;
+    }
+    if (n_inter) {
+        rtj_encode_blocks_kernel<true, true><<<dim3(gx, (unsigned)n_inter), EN_THREADS, 0, st>>>(*a, nblk, n_inter, 0, 0,
+                                                                                               d_runs + n_intra, d_seqs);
+        if ((e = cudaGetLastError()) != cudaSuccess) return -(int)e;
+        launches++;
+    }
+    const int n = launch_layout_and_gather<true>(a, nblk, 0, d_frame_words, st);
+    return n < 0 ? n : launches + n;
 }

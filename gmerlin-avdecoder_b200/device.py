@@ -70,3 +70,30 @@ def decode_sequences(ctx: capi.BatchContext, b: DeviceBatch, seq_first, carries=
     ptrs = None if carries is None else [None if c is None else c.data_ptr() for c in carries]
     ctx.decode_device_seq(b.stream.data_ptr(), b.desc.data_ptr(), b.F, b.w, b.h, list(seq_first), b.out.data_ptr(), ptrs,
                           st.cuda_stream)
+
+
+def encode_sequences(ctx: capi.BatchContext, pictures, encoders, w: int, h: int, fmt: int = 0,
+                     stream: torch.cuda.Stream | None = None):
+    """rtjgpu_encode_device_seq: pictures a list of S uint8 device tensors (or views), each one sequence's consecutive
+    tight w x h pictures of format fmt; encoders a list of S capi.SeqEncoder.  Returns (d_stream, d_offsets, seq_first,
+    nbytes): the packets in a buffer sized by capi.encode_bound (plus STREAM_SLACK_BYTES, so that it can be decoded as
+    it is), offsets[F + 1] on the device, seq_first[S + 1] and the bytes the packets take.  Waits for the encode."""
+    assert len(pictures) == len(encoders) and len(pictures) > 0
+    fsz = capi.frame_bytes(fmt, w, h)
+    counts = []
+    for p in pictures:
+        assert p.dtype == torch.uint8 and p.is_contiguous() and p.numel() % fsz == 0, "tight pictures of the format"
+        counts.append(p.numel() // fsz)
+    seq_first = np.concatenate([[0], np.cumsum(counts)]).astype(np.int64)
+    F = int(seq_first[-1])
+    dev = pictures[0].device
+    st = stream if stream is not None else torch.cuda.current_stream(dev)
+    cap = capi.encode_bound(fmt, w, h, F)
+    d_stream = torch.full((cap + capi.STREAM_SLACK_BYTES,), 0x7F, dtype=torch.uint8, device=dev)
+    d_offsets = torch.empty(F + 1, dtype=torch.int64, device=dev)
+    ctx.set_format(fmt)
+    ctx.encode_device_seq(F, w, h, list(seq_first), [p.data_ptr() for p in pictures], encoders, d_stream.data_ptr(), cap,
+                          d_offsets.data_ptr(), st.cuda_stream)
+    nbytes, overflow = ctx.encode_info()
+    assert not overflow, "rtjgpu_encode_bound was exceeded"
+    return d_stream, d_offsets, seq_first, nbytes

@@ -263,8 +263,47 @@ int  rtjgpu_encoder_reset(rtjgpu_ctx *ctx);
  * Asynchronous on cuda_stream. */
 int  rtjgpu_encode_device(rtjgpu_ctx *ctx, const uint8_t *d_frames, int F, int w, int h,
                           uint8_t *d_stream, size_t capacity, uint64_t *d_offsets, void *cuda_stream);
-/* Waits for the last rtjgpu_encode_device: bytes its packets take, and whether they did not fit. */
+/* Waits for the last rtjgpu_encode_device or rtjgpu_encode_device_seq: bytes its packets take, and whether they did not
+ * fit. */
 int  rtjgpu_get_encode_info(rtjgpu_ctx *ctx, uint64_t *bytes, int *overflow);
+
+/* MANY INDEPENDENT STREAMS ENCODED IN ONE CALL, each with an encoder state of its own.  A handle is what an RTjpeg_t
+ * carries for RTjpeg_compress -- tables, inter-frame parameters, key counter, the blocks last sent -- bound to one context
+ * (so to its device).  rtjgpu_seqenc_create: a fresh instance's encoder (quality 0 = zero tables, key_rate 0).  The
+ * setters are those of the context's encoder: set_quality clamps to 1..255 (it need not wait for the device: a handle's
+ * tables are staged per call); set_intra clamps key_rate 0..255 and the masks 0..16 and clears the stored blocks but not
+ * the key counter; reset puts counter and blocks back to a fresh instance's.  rtjgpu_seqenc_key_count: the key counter
+ * the next picture gets.  A handle is freed by rtjgpu_seqenc_destroy, which waits for the work on
+ * the device that may still use its stored blocks; it may outlive its context but is of no use then. */
+typedef struct rtjgpu_seqenc rtjgpu_seqenc;
+int  rtjgpu_seqenc_create(rtjgpu_ctx *ctx, rtjgpu_seqenc **out);
+void rtjgpu_seqenc_destroy(rtjgpu_seqenc *e);
+int  rtjgpu_seqenc_set_quality(rtjgpu_seqenc *e, int quality);
+int  rtjgpu_seqenc_set_intra(rtjgpu_seqenc *e, int key_rate, int lm, int cm);
+int  rtjgpu_seqenc_reset(rtjgpu_seqenc *e);
+int  rtjgpu_seqenc_key_count(const rtjgpu_seqenc *e);
+/* F output frames = S sequences laid end to end: sequence s is output frames [seq_first[s], seq_first[s + 1]), its
+ * pictures are read from frames[s] (consecutive tight pictures of the context's format, 8-byte aligned, device memory)
+ * and encoded with encs[s]'s state.  One pointer may serve several sequences (a rate ladder: the same pictures under
+ * handles of different qualities); a handle may serve only one.  The packets of all sequences go to d_stream back to back,
+ * each on a multiple of 4 bytes, and d_offsets[0..F] is laid out as by rtjgpu_encode_device: sequence s can be planned
+ * with rtjgpu_plan over offsets[seq_first[s] .. seq_first[s + 1]] and its own rtjgpu_state, and decoded with
+ * rtjgpu_decode_device_seq.  Sequence s's packets are byte for byte what RTjpeg_compress gives on that sequence alone
+ * with the handle's history: key counter, stored blocks, quality and intra settings carried from earlier calls.  The
+ * handles' counters advance at the call; their stored blocks are written by the device, so calls naming the same handle
+ * must be ordered (one CUDA stream, as the workspace shared with rtjgpu_encode_device requires too).  When the packets do
+ * not fit `capacity` nothing is written to d_stream, rtjgpu_get_encode_info tells, and every handle has advanced as if
+ * they had been written: size d_stream with rtjgpu_encode_bound.  seq_first, frames and encs are host arrays (S + 1, S and
+ * S entries), not read after the call returns.  Every argument is checked before anything is launched: RTJGPU_E_FORMAT for
+ * the grey format; RTJGPU_E_ARG for seq_first as rtjgpu_decode_device_seq takes it (S >= 1, 0 .. F strictly increasing),
+ * a NULL or misaligned picture pointer, a NULL handle, one of another context, or one named twice.  Asynchronous on
+ * cuda_stream. */
+int  rtjgpu_encode_device_seq(rtjgpu_ctx *ctx, int F, int w, int h, int S, const int *seq_first,
+                              const uint8_t *const *frames, rtjgpu_seqenc *const *encs,
+                              uint8_t *d_stream, size_t capacity, uint64_t *d_offsets, void *cuda_stream);
+/* The most bytes F packets of format (RTJ_YUV420 or RTJ_YUV422) and size w x h can take, padding included: a capacity
+ * that never overflows.  Host arithmetic; 0 for a format the encoder does not take or a bad size. */
+size_t rtjgpu_encode_bound(int format, int w, int h, int F);
 
 /* Raw (pre-AAN) tables for RTJGPU_TABLE_CUSTOM, the set_tables path. */
 int  rtjgpu_set_custom_tables(rtjgpu_ctx *ctx, const uint32_t raw[128]);
