@@ -17,5 +17,5 @@ from .capi import (  # noqa: F401
     BatchContext, BatchInfo, RTjpeg, RTjpegError, SeqEncoder, State, Timing,
     FRAME_DESC_DTYPE, HOST_IN_PINNED, HOST_OUT_PINNED, LIB_PATH, PLUGIN_PATH, STREAM_SLACK_BYTES,
     TABLE_CUSTOM, TABLE_ZERO, PIPELINE_AUTO, PIPELINE_SERIAL, PIPELINE_SLICED, CONV_BPP, CONVERTERS, NuvHeader, build_library, load_library, nuv_extract_rtj0, nuv_open, nuv_packets, nuv_probe,
-    encode_bound, plan, plan_sequences, raw_tables_for_quality, split_shards, split_shards_lead, tables_for_quality, tables_from_raw,
+    encode_bound, plan, plan_sequences, raw_tables_for_quality, select_frames, split_shards, split_shards_lead, tables_for_quality, tables_from_raw,
 )

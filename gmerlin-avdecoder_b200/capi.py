@@ -151,6 +151,11 @@ def load_library() -> C.CDLL:
                                            C.POINTER(vp), vp]
     L.rtjgpu_decode_device_rgb_seq.argtypes = [vp, vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_int), C.c_int, vp,
                                                C.c_size_t, C.c_size_t, C.c_int, C.POINTER(vp), C.POINTER(vp), vp]
+    L.rtjgpu_decode_device_select.argtypes = [vp, vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_int), C.POINTER(vp),
+                                              C.c_int, C.POINTER(C.c_int), vp, vp]
+    L.rtjgpu_decode_device_rgb_select.argtypes = [vp, vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_int),
+                                                  C.POINTER(vp), C.c_int, C.POINTER(C.c_int), C.c_int, vp, C.c_size_t,
+                                                  C.c_size_t, C.c_int, C.POINTER(vp), vp]
     L.rtjgpu_decode_host.argtypes = [vp, _u8p, _u64p, C.c_int, C.POINTER(State), _u8p, _u8p, C.c_int]
     L.rtjgpu_sync.argtypes = [vp]
     L.rtjgpu_enable_timing.argtypes = [vp, C.c_int]
@@ -257,6 +262,28 @@ def plan_sequences(seqs, states=None):
         seq_first.append(seq_first[-1] + len(desc))
     offsets = np.concatenate(offs + [np.array([at], dtype=np.uint64)])
     return out, offsets, np.concatenate(descs), np.array(seq_first, dtype=np.int64), states
+
+
+def select_frames(seq_first, picks) -> np.ndarray:
+    """Per-sequence frame indices -> the batch frame indices rtjgpu_decode_device_select takes.  picks: a list of S index
+    arrays, picks[s] local to sequence s (0 .. its length - 1, any order).  Returns the sorted global indices (int64); output
+    slot k of the select call is then the k-th of them.  Raises ValueError for an index outside its sequence or one named
+    twice."""
+    seq_first = np.asarray(seq_first, dtype=np.int64)
+    S = len(seq_first) - 1
+    if len(picks) != S:
+        raise ValueError(f"select_frames: {len(picks)} index arrays for {S} sequences")
+    out = []
+    for s, p in enumerate(picks):
+        p = np.asarray(p, dtype=np.int64).reshape(-1)
+        n = int(seq_first[s + 1] - seq_first[s])
+        if p.size and (p.min() < 0 or p.max() >= n):
+            raise ValueError(f"select_frames: sequence {s} has {n} frames, index out of range")
+        p = np.sort(p)
+        if p.size > 1 and (np.diff(p) == 0).any():
+            raise ValueError(f"select_frames: sequence {s}: an index named twice")
+        out.append(p + seq_first[s])
+    return np.concatenate(out) if out else np.zeros(0, dtype=np.int64)
 
 
 def encode_bound(fmt: int, w: int, h: int, F: int) -> int:
@@ -481,6 +508,28 @@ class BatchContext:
                                                     _int_array(seq_first), kind, C.c_void_p(d_rgb), row_pitch, frame_pitch,
                                                     alpha, _ptr_array(carries), _ptr_array(last_yuv),
                                                     C.c_void_p(cuda_stream or 0)), "rtjgpu_decode_device_rgb_seq")
+
+    def decode_device_select(self, d_stream: int, d_desc: int, F: int, w: int, h: int, seq_first, sel, d_out: int,
+                             carries=None, cuda_stream: int | None = None) -> None:
+        """rtjgpu_decode_device_select: the batch of decode_device_seq, only frames sel (batch indices, strictly increasing;
+        see select_frames) decoded, frame sel[k] to d_out + k * frame_bytes."""
+        S = len(seq_first) - 1
+        _check(self._L.rtjgpu_decode_device_select(self._h, C.c_void_p(d_stream), C.c_void_p(d_desc), F, w, h, S,
+                                                   _int_array(seq_first), _ptr_array(carries), len(sel), _int_array(sel),
+                                                   C.c_void_p(d_out or 0), C.c_void_p(cuda_stream or 0)),
+               "rtjgpu_decode_device_select")
+
+    def decode_device_rgb_select(self, d_stream: int, d_desc: int, F: int, w: int, h: int, seq_first, sel, kind: int,
+                                 d_rgb: int, row_pitch: int, frame_pitch: int, alpha: int = 0, carries=None, last_yuv=None,
+                                 cuda_stream: int | None = None) -> None:
+        """rtjgpu_decode_device_rgb_select: frame sel[k] to d_rgb + k * frame_pitch; last_yuv as for decode_device_rgb_seq
+        (each sequence's last frame as planes, selected or not)."""
+        S = len(seq_first) - 1
+        _check(self._L.rtjgpu_decode_device_rgb_select(self._h, C.c_void_p(d_stream), C.c_void_p(d_desc), F, w, h, S,
+                                                       _int_array(seq_first), _ptr_array(carries), len(sel), _int_array(sel),
+                                                       kind, C.c_void_p(d_rgb or 0), row_pitch, frame_pitch, alpha,
+                                                       _ptr_array(last_yuv), C.c_void_p(cuda_stream or 0)),
+               "rtjgpu_decode_device_rgb_select")
 
     def decode_host(self, stream: np.ndarray, offsets: np.ndarray, out: np.ndarray, state: State | None = None,
                     carry: np.ndarray | None = None, flags: int = 0) -> State:

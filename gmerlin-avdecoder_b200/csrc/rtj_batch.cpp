@@ -137,6 +137,7 @@ struct rtjgpu_ctx {
     cudaEvent_t    seq_copied[2] = {};
     bool           seq_pending[2] = {};
     int            seq_turn = 0;
+    std::vector<uint32_t> sel_jobs;           /* host scratch of rtjgpu_decode_device[_rgb]_select: K2's job list (RTJ_JOB) */
 };
 
 namespace {
@@ -382,6 +383,14 @@ struct SeqDev {
     uint8_t *const       *last_yuvs = nullptr;   /* [S] */
 };
 
+/* A selection of the batch's frames (rtjgpu_decode_device[_rgb]_select): K2's jobs, sorted by frame, on the device and on
+ * the host (where the slices' ranges of jobs are looked up) */
+struct SelDev {
+    const uint32_t *d_jobs = nullptr;
+    const uint32_t *h_jobs = nullptr;
+    int             njobs = 0;
+};
+
 /* where K2's pixels go when they leave as packed RGB (rtjgpu_decode_device_rgb) */
 struct RgbOut {
     uint8_t *d_rgb = nullptr;
@@ -393,9 +402,19 @@ struct RgbOut {
 
 int run_kernels(rtjgpu_ctx *ctx, Workspace *ws, const uint8_t *d_stream, const rtjgpu_frame_desc *d_desc,
                 int F, int w, int h, uint8_t *d_out, const uint8_t *d_carry, cudaStream_t st, cudaEvent_t *ev,
-                bool allow_pipe, const RgbOut *rgb = nullptr, const SeqDev *seq = nullptr)
+                bool allow_pipe, const RgbOut *rgb = nullptr, const SeqDev *seq = nullptr, const SelDev *sel = nullptr)
 {
     rtj_launch_args a;
+    a.d_jobs = sel ? sel->d_jobs : nullptr;
+    a.j0 = a.j1 = 0; a.njobs = sel ? sel->njobs : 0;
+    /* a selection: jobs [j0, j1) are those of frames [f0, f1) (K2 skips a slice that has none) */
+    auto job_range = [&](int f0, int f1) {
+        auto at = [&](int f) {
+            return (int)(std::partition_point(sel->h_jobs, sel->h_jobs + sel->njobs,
+                                              [f](uint32_t j) { return (int)RTJ_JOB_FRAME(j) < f; }) - sel->h_jobs);
+        };
+        a.j0 = at(f0); a.j1 = at(f1);
+    };
     a.d_stream = d_stream; a.d_desc = d_desc; a.d_tables = ctx->d_tables;
     a.F = F; a.w = w; a.h = h;
     a.f0 = 0; a.f1 = F; a.slice = 0;
@@ -414,6 +433,7 @@ int run_kernels(rtjgpu_ctx *ctx, Workspace *ws, const uint8_t *d_stream, const r
     a.d_k3_in = nullptr; a.d_k3_out = ws->d_k3_carry;
     a.d_k3_count = reinterpret_cast<uint32_t *>(reinterpret_cast<uint8_t *>(ws->d_k3_carry) + (((size_t)2 * ws->k3_carry_cap * sizeof(uint16_t) + 15) & ~(size_t)15));
     a.d_out = d_out; a.d_carry = d_carry;
+    a.fused_rgb = rgb != nullptr;
     a.d_rgb = rgb ? rgb->d_rgb : nullptr;
     a.rgb_row_pitch = rgb ? rgb->row_pitch : 0; a.rgb_frame_pitch = rgb ? rgb->frame_pitch : 0;
     a.rgb_kind = rgb ? rgb->kind : 0; a.rgb_alpha = rgb ? rgb->alpha : 0; a.d_last_yuv = rgb ? rgb->d_last_yuv : nullptr;
@@ -470,8 +490,11 @@ int run_kernels(rtjgpu_ctx *ctx, Workspace *ws, const uint8_t *d_stream, const r
         }
         a.f0 = 0; a.f1 = F;
         if (ev) CK(ctx, cudaEventRecord(ev[2], st));
-        LAUNCHED(rtj_launch_idct(&a, st), 1);
-        if (!rgb) LAUNCHED(rtj_launch_idct_hard(&a, st), 2);
+        if (sel) job_range(0, F);
+        if (!sel || a.j1 > a.j0) {                              /* (an empty selection: K1 and K3 only) */
+            LAUNCHED(rtj_launch_idct(&a, st), 1);
+            if (!rgb) LAUNCHED(rtj_launch_idct_hard(&a, st), 2);
+        }
         if (ev) CK(ctx, cudaEventRecord(ev[3], st));
         return RTJGPU_OK;
     }
@@ -490,14 +513,15 @@ int run_kernels(rtjgpu_ctx *ctx, Workspace *ws, const uint8_t *d_stream, const r
         CK(ctx, cudaEventRecord(p.scanned[i], p.scan));
         CK(ctx, cudaStreamWaitEvent(p.idct, p.scanned[i], 0));
         LAUNCHED(rtj_launch_resolve(&a, p.idct), 2);
-        LAUNCHED(rtj_launch_idct(&a, p.idct), 1);
+        if (sel) job_range(first[i], first[i + 1]);
+        if (!sel || a.j1 > a.j0) LAUNCHED(rtj_launch_idct(&a, p.idct), 1);     /* (a slice without a selected frame: no K2) */
     }
     if (ev) {                                                   /* stages overlap: scan = until the last slice is scanned, idct = the rest */
         CK(ctx, cudaEventRecord(ev[1], p.scan));
         CK(ctx, cudaEventRecord(ev[2], p.scan));
     }
     a.f0 = 0; a.f1 = F;
-    if (!rgb) LAUNCHED(rtj_launch_idct_hard(&a, p.idct), 2);
+    if (!rgb && (!sel || sel->njobs > 0)) LAUNCHED(rtj_launch_idct_hard(&a, p.idct), 2);
     CK(ctx, cudaEventRecord(p.join, p.idct));
     CK(ctx, cudaStreamWaitEvent(st, p.join, 0));
     if (ev) CK(ctx, cudaEventRecord(ev[3], st));
@@ -568,39 +592,90 @@ int stage_end(rtjgpu_ctx *ctx, void *d_dst, size_t bytes, cudaStream_t st)
 }
 
 /* The device copy of a layout of S > 1 sequences, in the workspace: [F] RTJ_SEQ words, then [S] carry pointers, then
- * [S] last_yuv pointers. */
-int seq_upload(rtjgpu_ctx *ctx, Workspace *ws, int F, const SeqIn &q, cudaStream_t st, SeqDev *out)
+ * [S] last_yuv pointers -- and behind them, for a selection (jobs != NULL), its ctx->sel_jobs: one copy either way.  S = 1
+ * uploads the jobs alone. */
+int seq_upload(rtjgpu_ctx *ctx, Workspace *ws, int F, const SeqIn &q, cudaStream_t st, SeqDev *out, SelDev *jobs = nullptr)
 {
-    const size_t words = ((size_t)F * sizeof(uint32_t) + 7) & ~(size_t)7, ptrs = (size_t)q.S * sizeof(void *);
-    const size_t bytes = words + 2 * ptrs;
+    const bool layout = q.S > 1;
+    const size_t words = layout ? ((size_t)F * sizeof(uint32_t) + 7) & ~(size_t)7 : 0, ptrs = layout ? (size_t)q.S * sizeof(void *) : 0;
+    const size_t jbytes = jobs ? ctx->sel_jobs.size() * sizeof(uint32_t) : 0;
+    const size_t bytes = words + 2 * ptrs + jbytes;
     uint8_t *h;
     int rc = stage_begin(ctx, bytes, &h);
     if (rc) return rc;
     if ((rc = grow_device(ctx, &ws->d_seq, &ws->seq_cap, bytes))) return rc;
-    uint32_t *hw = reinterpret_cast<uint32_t *>(h);
-    for (int s = 0; s < q.S; s++)
-        for (int f = q.first[s]; f < q.first[s + 1]; f++) hw[f] = RTJ_SEQ(q.first[s], s);
-    const uint8_t **hc = reinterpret_cast<const uint8_t **>(h + words);
-    uint8_t **hl = reinterpret_cast<uint8_t **>(h + words + ptrs);
-    for (int s = 0; s < q.S; s++) { hc[s] = q.carry(s); hl[s] = q.last(s); }
+    if (layout) {
+        uint32_t *hw = reinterpret_cast<uint32_t *>(h);
+        for (int s = 0; s < q.S; s++)
+            for (int f = q.first[s]; f < q.first[s + 1]; f++) hw[f] = RTJ_SEQ(q.first[s], s);
+        const uint8_t **hc = reinterpret_cast<const uint8_t **>(h + words);
+        uint8_t **hl = reinterpret_cast<uint8_t **>(h + words + ptrs);
+        for (int s = 0; s < q.S; s++) { hc[s] = q.carry(s); hl[s] = q.last(s); }
+    }
+    if (jbytes) memcpy(h + words + 2 * ptrs, ctx->sel_jobs.data(), jbytes);
     if ((rc = stage_end(ctx, ws->d_seq, bytes, st))) return rc;
-    out->seq = reinterpret_cast<const uint32_t *>(ws->d_seq);
-    out->carries = reinterpret_cast<const uint8_t *const *>(ws->d_seq + words);
-    out->last_yuvs = reinterpret_cast<uint8_t *const *>(ws->d_seq + words + ptrs);
+    if (layout) {
+        out->seq = reinterpret_cast<const uint32_t *>(ws->d_seq);
+        out->carries = reinterpret_cast<const uint8_t *const *>(ws->d_seq + words);
+        out->last_yuvs = reinterpret_cast<uint8_t *const *>(ws->d_seq + words + ptrs);
+    }
+    if (jobs) {
+        jobs->d_jobs = reinterpret_cast<const uint32_t *>(ws->d_seq + words + 2 * ptrs);
+        jobs->h_jobs = ctx->sel_jobs.data();
+        jobs->njobs = (int)ctx->sel_jobs.size();
+    }
     return RTJGPU_OK;
 }
 
-/* rtjgpu_decode_device and rtjgpu_decode_device_seq: the former is the latter's one-sequence case. */
+/* A selection of the batch's frames as the caller gave it: n batch frame indices, strictly increasing (host array). */
+struct SelIn {
+    int        n = 0;
+    const int *idx = nullptr;
+};
+
+int sel_check(int F, const SelIn &s)
+{
+    if (s.n < 0 || s.n > F || (s.n > 0 && !s.idx)) return RTJGPU_E_ARG;
+    for (int k = 0; k < s.n; k++)
+        if (s.idx[k] < 0 || s.idx[k] >= F || (k > 0 && s.idx[k] <= s.idx[k - 1])) return RTJGPU_E_ARG;
+    return RTJGPU_OK;
+}
+
+/* K2's jobs of a selection (into ctx->sel_jobs), sorted by frame: selected frame sel[k] to slot k; with rgb_last, also every
+ * sequence's last frame that is not selected but has a last_yuv, to planes only. */
+void sel_jobs(rtjgpu_ctx *ctx, const SeqIn &q, const SelIn &s, bool rgb_last)
+{
+    std::vector<uint32_t> &jobs = ctx->sel_jobs;
+    jobs.clear();
+    int k = 0;
+    for (int i = 0; i < q.S; i++) {
+        const int last = q.first[i + 1] - 1;
+        bool last_selected = false;
+        for (; k < s.n && s.idx[k] <= last; k++) {
+            jobs.push_back(RTJ_JOB(s.idx[k], k));
+            last_selected = s.idx[k] == last;
+        }
+        if (rgb_last && q.last(i) && !last_selected) jobs.push_back(RTJ_JOB(last, RTJ_JOB_NO_SLOT));
+    }
+}
+
+/* rtjgpu_decode_device and rtjgpu_decode_device_seq: the former is the latter's one-sequence case.  sel != NULL:
+ * rtjgpu_decode_device_select (q.first given), which is rtjgpu_decode_device_seq when it selects every frame. */
 int decode_device(rtjgpu_ctx *ctx, const uint8_t *d_stream, const rtjgpu_frame_desc *d_desc, int F, int w, int h,
-                  const SeqIn &q, uint8_t *d_out, void *cuda_stream)
+                  const SeqIn &q, uint8_t *d_out, void *cuda_stream, const SelIn *sel = nullptr)
 {
     if (!ctx || F < 0) return RTJGPU_E_ARG;
     if (q.first) {
         const int rc = seq_check(F, q);
         if (rc) return rc;
     }
+    if (sel) {
+        const int rc = sel_check(F, *sel);
+        if (rc) return rc;
+        if (sel->n == F) sel = nullptr;                      /* every frame: the full call, runs of frames included */
+    }
     if (F == 0) { ctx->last_F = 0; return RTJGPU_OK; }
-    if (!d_stream || !d_desc || !d_out) return RTJGPU_E_ARG;
+    if (!d_stream || !d_desc || (!d_out && !(sel && sel->n == 0))) return RTJGPU_E_ARG;
     /* K1 reads the stream as 32-bit words, K2 leaves its strips as 16-byte bulk stores and reads the carry as 8-byte rows */
     if (((uintptr_t)d_stream & 3) || ((uintptr_t)d_desc & 7) || ((uintptr_t)d_out & 15) || ((uintptr_t)q.carry(0) & 7)) return RTJGPU_E_ARG;
     if (w <= 0 || h <= 0 || (w & 15) || (h & 15) || w > 65535 || h > 65535) return RTJGPU_E_SIZE;
@@ -612,19 +687,23 @@ int decode_device(rtjgpu_ctx *ctx, const uint8_t *d_stream, const rtjgpu_frame_d
     int rc = ws_reserve(ctx, &ctx->ws, F, nblk);
     if (rc) return rc;
     SeqDev sd;
-    if (q.S > 1 && (rc = seq_upload(ctx, &ctx->ws, F, q, (cudaStream_t)cuda_stream, &sd))) return rc;
+    SelDev jd;
+    if (sel) sel_jobs(ctx, q, *sel, false);
+    if ((q.S > 1 || (sel && sel->n > 0)) && (rc = seq_upload(ctx, &ctx->ws, F, q, (cudaStream_t)cuda_stream, &sd, sel ? &jd : nullptr)))
+        return rc;
     cudaEvent_t *ev = ctx->timing ? ctx->ev[ctx->timed_calls % TIMING_RING] : nullptr;
     rc = run_kernels(ctx, &ctx->ws, d_stream, d_desc, F, w, h, d_out, q.S > 1 ? nullptr : q.carry(0), (cudaStream_t)cuda_stream, ev,
-                     true, nullptr, q.S > 1 ? &sd : nullptr);
+                     true, nullptr, q.S > 1 ? &sd : nullptr, sel ? &jd : nullptr);
     if (ev && rc == RTJGPU_OK) ctx->timed_calls++;
     ctx->last_F = F;
     ctx->last_stream = cuda_stream;
     return rc;
 }
 
-/* rtjgpu_decode_device_rgb and rtjgpu_decode_device_rgb_seq */
+/* rtjgpu_decode_device_rgb and rtjgpu_decode_device_rgb_seq; sel != NULL: rtjgpu_decode_device_rgb_select */
 int decode_device_rgb(rtjgpu_ctx *ctx, const uint8_t *d_stream, const rtjgpu_frame_desc *d_desc, int F, int w, int h,
-                      const SeqIn &q, int kind, uint8_t *d_rgb, size_t row_pitch, size_t frame_pitch, int alpha, void *cuda_stream)
+                      const SeqIn &q, int kind, uint8_t *d_rgb, size_t row_pitch, size_t frame_pitch, int alpha, void *cuda_stream,
+                      const SelIn *sel = nullptr)
 {
     if (!ctx || F < 0) return RTJGPU_E_ARG;
     if (ctx->format != RTJ_YUV420) return RTJGPU_E_FORMAT;                     /* the reference's converters are yuv420 ones */
@@ -634,8 +713,13 @@ int decode_device_rgb(rtjgpu_ctx *ctx, const uint8_t *d_stream, const rtjgpu_fra
         const int rc = seq_check(F, q);
         if (rc) return rc;
     }
+    if (sel) {
+        const int rc = sel_check(F, *sel);
+        if (rc) return rc;
+        if (sel->n == F) sel = nullptr;                      /* every frame: the full call, last frames as planes included */
+    }
     if (F == 0) { ctx->last_F = 0; return RTJGPU_OK; }
-    if (!d_stream || !d_desc || !d_rgb) return RTJGPU_E_ARG;
+    if (!d_stream || !d_desc || (!d_rgb && !(sel && sel->n == 0))) return RTJGPU_E_ARG;
     if (w <= 0 || h <= 0 || (w & 15) || (h & 15) || w > 65535 || h > 65535) return RTJGPU_E_SIZE;
     if (F > RTJGPU_MAX_FRAMES_PER_BATCH) return RTJGPU_E_TOOBIG;
     const int bpp = rtj_convert_bpp(kind);
@@ -649,13 +733,16 @@ int decode_device_rgb(rtjgpu_ctx *ctx, const uint8_t *d_stream, const rtjgpu_fra
     int rc = ws_reserve(ctx, &ctx->ws, F, nblk);
     if (rc) return rc;
     SeqDev sd;
-    if (q.S > 1 && (rc = seq_upload(ctx, &ctx->ws, F, q, (cudaStream_t)cuda_stream, &sd))) return rc;
+    SelDev jd;
+    if (sel) sel_jobs(ctx, q, *sel, true);
+    if ((q.S > 1 || (sel && !ctx->sel_jobs.empty())) && (rc = seq_upload(ctx, &ctx->ws, F, q, (cudaStream_t)cuda_stream, &sd, sel ? &jd : nullptr)))
+        return rc;
     RgbOut o;
     o.d_rgb = d_rgb; o.row_pitch = row_pitch; o.frame_pitch = frame_pitch; o.kind = kind; o.alpha = (unsigned)alpha & 0xFFu;
     o.d_last_yuv = q.S > 1 ? nullptr : q.last(0);
     cudaEvent_t *ev = ctx->timing ? ctx->ev[ctx->timed_calls % TIMING_RING] : nullptr;
     rc = run_kernels(ctx, &ctx->ws, d_stream, d_desc, F, w, h, nullptr, q.S > 1 ? nullptr : q.carry(0), (cudaStream_t)cuda_stream, ev,
-                     true, &o, q.S > 1 ? &sd : nullptr);
+                     true, &o, q.S > 1 ? &sd : nullptr, sel ? &jd : nullptr);
     if (ev && rc == RTJGPU_OK) ctx->timed_calls++;
     ctx->last_F = F;
     ctx->last_stream = cuda_stream;
@@ -1258,6 +1345,31 @@ int rtjgpu_decode_device_rgb_seq(rtjgpu_ctx *ctx, const uint8_t *d_stream, const
     q.S = S; q.first = seq_first; q.carries = carries; q.last_yuv = last_yuv;
     if (!seq_first) return RTJGPU_E_ARG;
     return decode_device_rgb(ctx, d_stream, d_desc, F, w, h, q, kind, d_rgb, row_pitch, frame_pitch, alpha, cuda_stream);
+}
+
+int rtjgpu_decode_device_select(rtjgpu_ctx *ctx, const uint8_t *d_stream, const rtjgpu_frame_desc *d_desc, int F, int w, int h,
+                                int S, const int *seq_first, const uint8_t *const *carries,
+                                int n, const int *sel, uint8_t *d_out, void *cuda_stream)
+{
+    SeqIn q;
+    q.S = S; q.first = seq_first; q.carries = carries;
+    SelIn s;
+    s.n = n; s.idx = sel;
+    if (!seq_first) return RTJGPU_E_ARG;
+    return decode_device(ctx, d_stream, d_desc, F, w, h, q, d_out, cuda_stream, &s);
+}
+
+int rtjgpu_decode_device_rgb_select(rtjgpu_ctx *ctx, const uint8_t *d_stream, const rtjgpu_frame_desc *d_desc, int F, int w, int h,
+                                    int S, const int *seq_first, const uint8_t *const *carries,
+                                    int n, const int *sel, int kind, uint8_t *d_rgb, size_t row_pitch, size_t frame_pitch,
+                                    int alpha, uint8_t *const *last_yuv, void *cuda_stream)
+{
+    SeqIn q;
+    q.S = S; q.first = seq_first; q.carries = carries; q.last_yuv = last_yuv;
+    SelIn s;
+    s.n = n; s.idx = sel;
+    if (!seq_first) return RTJGPU_E_ARG;
+    return decode_device_rgb(ctx, d_stream, d_desc, F, w, h, q, kind, d_rgb, row_pitch, frame_pitch, alpha, cuda_stream, &s);
 }
 
 int rtjgpu_sync(rtjgpu_ctx *ctx)

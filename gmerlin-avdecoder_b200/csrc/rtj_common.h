@@ -58,6 +58,14 @@ extern "C" {
 #define RTJ_SEQ_FIRST(v) ((v) & 0xFFFFu)
 #define RTJ_SEQ_INDEX(v) ((v) >> 16)
 
+/* One job of K2 in a call that decodes a selection of the batch's frames (rtjgpu_decode_device[_rgb]_select): the frame
+ * and the output slot it goes to, both below 2^16 (n <= F <= RTJGPU_MAX_FRAMES_PER_BATCH).  RTJ_JOB_NO_SLOT (fused RGB
+ * only): an unselected last frame of a sequence, decoded to planes for that sequence's last_yuv and nothing else. */
+#define RTJ_JOB(frame, slot) ((uint32_t)(frame) | (uint32_t)(slot) << 16)
+#define RTJ_JOB_FRAME(v) ((v) & 0xFFFFu)
+#define RTJ_JOB_SLOT(v) ((v) >> 16)
+#define RTJ_JOB_NO_SLOT 0xFFFFu
+
 #define RTJ_NUM_TABLES 257
 
 /* Dequantisation tables as the kernels read them: zig-zag order (entry k is
@@ -157,7 +165,9 @@ typedef struct rtj_launch_args {
     uint8_t                 *d_out;
     const uint8_t           *d_carry;
     const void              *d_lut;         /* K2: position table of this geometry (rtj_launch_build_lut) */
-    /* K2 with the fused colour conversion (d_rgb != NULL): packed pixels instead of planes */
+    /* K2 with the fused colour conversion (fused_rgb != 0): packed pixels instead of planes.  d_rgb may be NULL only when no
+     * frame is converted (a selection of none whose sequences' last frames still leave as planes into last_yuv) */
+    int                      fused_rgb;
     uint8_t                 *d_rgb;
     size_t                   rgb_row_pitch, rgb_frame_pitch;
     int                      rgb_kind;      /* RTJ_CONV_RGB32 / BGR32 / RGB24 / BGR24 / RGB16 */
@@ -170,6 +180,10 @@ typedef struct rtj_launch_args {
     uint8_t *const          *d_last_yuvs;   /* [S] RGB: where each sequence's last frame leaves as planes, entries may be NULL */
     int                      scan_mode;     /* RTJGPU_SCAN_* */
     rtj_seg_plan             seg;           /* workspace of the segment-parallel scan (sum == NULL: not available) */
+    /* a selection of frames (rtjgpu_decode_device[_rgb]_select; d_jobs NULL: every frame, at its own index): K2 runs one
+     * frame per CTA over jobs [j0, j1) of the batch's njobs RTJ_JOB words, sorted by frame */
+    const uint32_t          *d_jobs;
+    int                      j0, j1, njobs;
 } rtj_launch_args;
 
 int rtj_launch_scan(const rtj_launch_args *a, void *stream);          /* returns the number of launches (>0) or -cudaError */

@@ -521,6 +521,10 @@ struct K2Params {
     uint8_t *const *last_yuvs;
     int ahead;                       /* frames between a CTA and the one that follows it on the same SM slot */
     int wq;                          /* slots of one warp's queue */
+    /* SEL: blockIdx.y names job j0 + blockIdx.y of the batch's njobs RTJ_JOB words (frame, output slot), sorted by frame;
+     * `ahead` then counts jobs */
+    const uint32_t *jobs;
+    int j0, njobs;
 };
 
 /* The general decoder for one block that K2's sparse classes do not take (long blocks; blocks whose last writer used
@@ -594,21 +598,28 @@ constexpr int RGB_NONE = -1, RGB_ANY = 99;
 /* RUN: a CTA works through P.run frames in turn (below); false: one frame, and none of the run's bookkeeping is compiled in */
 /* RES: a warp reserves its places in K2b's queue with one request per row (streams in which most blocks go that way: a quality
  * above 170; chosen by the batch before, like RUN) */
-template <bool SINGLE, int FMT, int WARPS, int RGBK, bool RUN, bool RES = false>
+/* SEL: a selection of frames (rtjgpu_decode_device[_rgb]_select).  One frame per CTA, taken from job blockIdx.y of P.jobs: a
+ * frame needs only its own entries and its last writers' (K3), never the pixels of the frames before it.  Its pixels go to
+ * the job's output slot -- K2b's queue names the slot as the place they go to --; a fused-RGB job without a slot (an
+ * unselected last frame of a sequence) leaves as planes for last_yuv only. */
+template <bool SINGLE, int FMT, int WARPS, int RGBK, bool RUN, bool RES = false, bool SEL = false>
 __global__ void __launch_bounds__(WARPS * 32, WARPS == 4 ? 8 : 10)
 rtj_idct_kernel(const K2Params P)
 {
     constexpr bool RGB = RGBK != RGB_NONE;
     static_assert(!RGB || FMT == 0, "the fused converters are the reference's yuv420 ones");
+    static_assert(!SEL || (!RUN && !RES), "a selection is decoded one frame per CTA, without K2b's reservations");
     constexpr int THREADS = WARPS * 32;
     typedef Geo<FMT> G;
     extern __shared__ __align__(128) uint8_t smem[];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     asm volatile("griddepcontrol.wait;" ::: "memory");        /* resident before K3 is done (launch_pdl); K3's entries are final from here */
+    const unsigned job_at = SEL ? (unsigned)P.j0 + blockIdx.y : 0u;
+    const uint32_t job = SEL ? __ldg(P.jobs + job_at) : 0u;
     /* A CTA works through a RUN of frames of its row of units, the strip staying in shared memory from frame to frame: what a
      * frame skips (lib/RTjpeg.c:2704 -- the block keeps what the picture held) is then simply not touched, instead of being
      * decoded again from its last writer's stream for every frame it persists in.  P.run == 1: one frame per CTA. */
-    const unsigned f_first = (unsigned)P.f0 + blockIdx.y * (RUN ? (unsigned)P.run : 1u);
+    const unsigned f_first = SEL ? RTJ_JOB_FRAME(job) : (unsigned)P.f0 + blockIdx.y * (RUN ? (unsigned)P.run : 1u);
     const unsigned f_last = RUN ? min(f_first + (unsigned)P.run, (unsigned)P.f_end) : f_first + 1u;       /* one behind */
     constexpr bool runs = RUN;
     const int w = P.w, h = P.h, mbw = w / G::UNIT_W;           /* units per picture row */
@@ -650,8 +661,13 @@ rtj_idct_kernel(const K2Params P)
     /* A CTA lives a few microseconds, of which the first read of its entries from DRAM -- under the write traffic of
      * this kernel -- is a good part.  So it asks for the entries it will want next into L2 now: those of the CTA that will
      * take its place when it retires (same strip, P.ahead frames on), or, working through a run, those of its next frame. */
-    const unsigned pf = runs ? 1u : (unsigned)P.ahead;
-    const bool pf_ok = runs ? f + 1u < f_last : f + pf < (unsigned)P.F;
+    unsigned pf = runs ? 1u : (unsigned)P.ahead;
+    bool pf_ok = runs ? f + 1u < f_last : f + pf < (unsigned)P.F;
+    if (SEL) {                                                       /* ... the frame of the job P.ahead jobs on */
+        const unsigned ja = job_at + (unsigned)P.ahead;
+        pf_ok = ja < (unsigned)P.njobs;
+        pf = pf_ok ? RTJ_JOB_FRAME(__ldg(P.jobs + ja)) - f : 0u;     /* jobs are sorted by frame: pf > 0 */
+    }
     if (pf_ok && tid * 32 < nb)
         asm volatile("prefetch.global.L2 [%0];" :: "l"(my_ent + (size_t)pf * (unsigned)P.nblk + tid * 32));
 
@@ -853,7 +869,8 @@ rtj_idct_kernel(const K2Params P)
                 const unsigned below = (1u << lane) - 1u;
                 /* a queue entry: the block's place in its frame (and whether it is a chroma block), the frame the pixels
                  * go to and the frame whose stream holds the block (its last writer) */
-                const uint2 rec = make_uint2((strip_blk0 + (unsigned)bi) | (off_is_chroma<FMT>(off, mbs) ? 0x80000000u : 0u), f | (hsf << 16));
+                const uint2 rec = make_uint2((strip_blk0 + (unsigned)bi) | (off_is_chroma<FMT>(off, mbs) ? 0x80000000u : 0u),
+                                             (SEL ? RTJ_JOB_SLOT(job) : f) | (hsf << 16));
                 if (hard && !full) reinterpret_cast<uint2 *>(P.hardq)[base + __popc(mH & below)] = rec;
                 if (full) reinterpret_cast<uint2 *>(P.hardq)[P.hardq_cap - 1u - (baseF + __popc(mF & below))] = rec;
                 /* (the luma blocks among them in the upper half: a strip whose luma blocks are all HARD keeps its luma rows) */
@@ -897,8 +914,10 @@ rtj_idct_kernel(const K2Params P)
         const uint8_t *tU = tile + G::CHROMA_AT * mbs, *tV = tU + 64 * mbs;
         const int kind = RGBK == RGB_ANY ? P.rgb_kind : RGBK;
         const int bpp = (kind == RTJ_CONV_RGB32 || kind == RTJ_CONV_BGR32) ? 4 : kind == RTJ_CONV_RGB16 ? 2 : 3;
-        uint8_t *base = P.rgb + (size_t)f * P.rgb_frame_pitch + (size_t)(my * 16) * P.rgb_row_pitch + (size_t)(mx0 * 16) * bpp;
-        for (int item = tid; item < 8 * chunks; item += THREADS) {
+        uint8_t *base = P.rgb + (size_t)(SEL ? RTJ_JOB_SLOT(job) : f) * P.rgb_frame_pitch + (size_t)(my * 16) * P.rgb_row_pitch
+                        + (size_t)(mx0 * 16) * bpp;
+        const int items = SEL && RTJ_JOB_SLOT(job) == RTJ_JOB_NO_SLOT ? 0 : 8 * chunks;    /* SEL: planes for last_yuv only */
+        for (int item = tid; item < items; item += THREADS) {
             const int rp = item / chunks, c = item - rp * chunks;
             const uint2 y0 = *reinterpret_cast<const uint2 *>(tile + (2 * rp) * lw + c * 8);
             const uint2 y1 = *reinterpret_cast<const uint2 *>(tile + (2 * rp + 1) * lw + c * 8);
@@ -932,7 +951,7 @@ rtj_idct_kernel(const K2Params P)
     if (planes_leave) {
     const size_t fsz = RTJ_FMT_FRAME_BYTES(FMT, w, h);
     const int cw = w >> 1;
-    uint8_t *const planes = RGB ? last_planes : P.out + (size_t)f * fsz;
+    uint8_t *const planes = RGB ? last_planes : P.out + (size_t)(SEL ? RTJ_JOB_SLOT(job) : f) * fsz;
     uint8_t *oy = planes + (size_t)(my * G::LUMA_ROWS) * w + mx0 * G::UNIT_W;
     uint8_t *ou = planes + (size_t)w * h + (size_t)(my * 8) * cw + mx0 * 8;
     uint8_t *ov = ou + (FMT == 0 ? (size_t)cw * (h >> 1) : (size_t)cw * h);
@@ -1281,6 +1300,9 @@ cudaError_t k2_attr()
     if (RGBK == RGB_NONE && e == cudaSuccess)
         e = cudaFuncSetAttribute(rtj_idct_kernel<SINGLE, FMT, WARPS, RGB_NONE, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                  (int)idct_smem_bytes(IDCT_MAX_MB, FMT, 3));
+    if (e == cudaSuccess)
+        e = cudaFuncSetAttribute(rtj_idct_kernel<SINGLE, FMT, WARPS, RGBK, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                 (int)idct_smem_bytes(IDCT_MAX_MB, FMT, 3));
     return e;
 }
 
@@ -1315,7 +1337,16 @@ cudaError_t k2_launch(K2Params &P, int grid_x, int F, cudaStream_t st)
     P.run = P.run < 1 ? 1 : P.run;
     const dim3 grid((unsigned)grid_x, (unsigned)((F + P.run - 1) / P.run));
     cudaError_t e;
-    if (P.run > 1) {
+    if (P.jobs) {
+        /* a selection: one frame per CTA whatever P.run says (the caller sets it to 1), no reservations in K2b's queue */
+        if (P.nstrips == 1) {
+            if (warps == 4) e = launch_pdl(rtj_idct_kernel<true, FMT, 4, RGBK, false, false, true>, grid, dim3(128), smem, st, P);
+            else e = launch_pdl(rtj_idct_kernel<true, FMT, 3, RGBK, false, false, true>, grid, dim3(96), smem, st, P);
+        } else {
+            if (warps == 4) e = launch_pdl(rtj_idct_kernel<false, FMT, 4, RGBS, false, false, true>, grid, dim3(128), smem, st, P);
+            else e = launch_pdl(rtj_idct_kernel<false, FMT, 3, RGBS, false, false, true>, grid, dim3(96), smem, st, P);
+        }
+    } else if (P.run > 1) {
         if (P.nstrips == 1) {
             if (warps == 4) e = launch_pdl(rtj_idct_kernel<true, FMT, 4, RGBK, true>, grid, dim3(128), smem, st, P);
             else e = launch_pdl(rtj_idct_kernel<true, FMT, 3, RGBK, true>, grid, dim3(96), smem, st, P);
@@ -1407,11 +1438,17 @@ extern "C" int rtj_launch_idct(const rtj_launch_args *a, void *stream)
     P.f0 = a->f0; P.F = a->F; P.f_end = a->f1; P.run = a->k2_run; P.reserve = a->raw_expected;
     P.row0 = a->row0; P.rows = uy;
     const int grid_x = P.nstrips * (a->row1 - a->row0);
-    const int nf = a->f1 - a->f0;
+    int nf = a->f1 - a->f0;
+    P.jobs = a->d_jobs; P.j0 = a->j0; P.njobs = a->njobs;
+    if (a->d_jobs) {                                 /* a selection: the launch's jobs, one frame per CTA */
+        nf = a->j1 - a->j0;
+        P.run = 1;
+        if (nf <= 0) return (int)cudaErrorInvalidValue;
+    }
     P.rgb = a->d_rgb; P.rgb_row_pitch = a->rgb_row_pitch; P.rgb_frame_pitch = a->rgb_frame_pitch;
     P.rgb_kind = a->rgb_kind; P.rgb_alpha = a->rgb_alpha & 0xFFu; P.last_yuv = a->d_last_yuv;
     P.seq = a->d_seq; P.carries = a->d_carries; P.last_yuvs = a->d_last_yuvs;
-    if (a->d_rgb) {
+    if (a->fused_rgb) {
         if (fmt != 0) return (int)cudaErrorInvalidValue;
         switch (a->rgb_kind) {
         case RTJ_CONV_RGB32: return (int)k2_launch<0, RTJ_CONV_RGB32>(P, grid_x, nf, st);

@@ -54,11 +54,12 @@ def decode(ctx: capi.BatchContext, b: DeviceBatch, carry: torch.Tensor | None = 
                       None if carry is None else carry.data_ptr(), st.cuda_stream)
 
 
-def upload_sequences(seqs, w: int, h: int, device: int | str = 0, fmt: int = 0, states=None):
+def upload_sequences(seqs, w: int, h: int, device: int | str = 0, fmt: int = 0, states=None, out: torch.Tensor | None = None):
     """Several independent packet sequences [(stream, offsets), ...] as one batch (capi.plan_sequences): each is planned
-    with its own state (states: list of capi.State, advanced in place, or None).  Returns (DeviceBatch, seq_first[S + 1])."""
+    with its own state (states: list of capi.State, advanced in place, or None).  out: as for upload() (a caller that only
+    decodes selections, decode_select, may pass an empty tensor).  Returns (DeviceBatch, seq_first[S + 1])."""
     stream, _, desc, seq_first, _ = capi.plan_sequences(seqs, states)
-    return upload(stream, desc, w, h, device=device, fmt=fmt), seq_first
+    return upload(stream, desc, w, h, device=device, out=out, fmt=fmt), seq_first
 
 
 def decode_sequences(ctx: capi.BatchContext, b: DeviceBatch, seq_first, carries=None,
@@ -70,6 +71,23 @@ def decode_sequences(ctx: capi.BatchContext, b: DeviceBatch, seq_first, carries=
     ptrs = None if carries is None else [None if c is None else c.data_ptr() for c in carries]
     ctx.decode_device_seq(b.stream.data_ptr(), b.desc.data_ptr(), b.F, b.w, b.h, list(seq_first), b.out.data_ptr(), ptrs,
                           st.cuda_stream)
+
+
+def decode_select(ctx: capi.BatchContext, b: DeviceBatch, seq_first, sel, carries=None, out: torch.Tensor | None = None,
+                  stream: torch.cuda.Stream | None = None) -> torch.Tensor:
+    """rtjgpu_decode_device_select over a batch of upload_sequences: only the batch frames sel (strictly increasing; see
+    capi.select_frames) are decoded, frame sel[k] to row k of the result.  carries as for decode_sequences.  out: a
+    [n, frame_bytes] uint8 tensor to fill (default: a new one; b.out is not used).  Returns out."""
+    st = stream if stream is not None else torch.cuda.current_stream(b.stream.device)
+    sel = [int(x) for x in np.asarray(sel, dtype=np.int64).reshape(-1)]
+    if out is None:
+        out = torch.empty((len(sel), b.frame_bytes), dtype=torch.uint8, device=b.stream.device)
+    assert out.dtype == torch.uint8 and out.is_contiguous() and out.numel() >= len(sel) * b.frame_bytes
+    ctx.set_format(b.fmt)
+    ptrs = None if carries is None else [None if c is None else c.data_ptr() for c in carries]
+    ctx.decode_device_select(b.stream.data_ptr(), b.desc.data_ptr(), b.F, b.w, b.h, list(seq_first), sel,
+                             out.data_ptr() if len(sel) else None, ptrs, st.cuda_stream)
+    return out
 
 
 def encode_sequences(ctx: capi.BatchContext, pictures, encoders, w: int, h: int, fmt: int = 0,

@@ -367,6 +367,31 @@ int  rtjgpu_decode_device_rgb_seq(rtjgpu_ctx *ctx, const uint8_t *d_stream, cons
                                   int S, const int *seq_first, int kind, uint8_t *d_rgb, size_t row_pitch, size_t frame_pitch,
                                   int alpha, const uint8_t *const *carries, uint8_t *const *last_yuv, void *cuda_stream);
 
+/* ONLY THE FRAMES A CALLER ASKS FOR.  The batch (F, S, seq_first, carries) is exactly that of rtjgpu_decode_device_seq; sel is
+ * a HOST array of n batch frame indices, strictly increasing, each in [0, F), 0 <= n <= F, not read after the call returns.
+ * Frame sel[k] goes to d_out + k * frame_bytes (tight planes of the context's format), byte for byte what
+ * rtjgpu_decode_device_seq gives at row sel[k]; nothing else of d_out is written.  A frame needs only its own entries and
+ * those of its skipped blocks' last writers, never the pixels of the frames before it: every frame is still scanned (K1)
+ * and resolved (K3), only the selected ones are decoded and stored (K2).  Afterwards rtjgpu_get_batch_info and
+ * rtjgpu_get_skip_counts describe all F frames.  To continue the streams in a later call, select each sequence's last frame:
+ * its output is that sequence's next carry (selecting only the last frames is a seek).  Upload no trailing frames that no
+ * selection needs: they are scanned all the same.  n = 0: the batch is scanned and resolved and nothing is written (d_out
+ * may then be NULL).  n = F is rtjgpu_decode_device_seq; otherwise K2 decodes one frame per CTA whatever
+ * rtjgpu_set_frame_runs says.  Every argument is checked before anything is launched: rtjgpu_decode_device_seq's rules
+ * (alignment included), and RTJGPU_E_ARG for n < 0, n > F, sel == NULL with n > 0, or an index out of range, repeated or
+ * out of order.  Asynchronous on cuda_stream. */
+int  rtjgpu_decode_device_select(rtjgpu_ctx *ctx, const uint8_t *d_stream, const rtjgpu_frame_desc *d_desc, int F, int w, int h,
+                                 int S, const int *seq_first, const uint8_t *const *carries,
+                                 int n, const int *sel, uint8_t *d_out, void *cuda_stream);
+/* The same with rtjgpu_decode_device_rgb_seq's fused converter: frame sel[k] goes to d_rgb + k * frame_pitch.  last_yuv has
+ * its _rgb_seq meaning: each sequence's last frame leaves as planes (its next carry) whether or not it is selected; an
+ * unselected last frame is decoded to planes only.  n = 0 (d_rgb may then be NULL) writes those planes and nothing else:
+ * the streams advance by one batch and no picture is kept.  RTJGPU_E_FORMAT on a context that is not RTJ_YUV420. */
+int  rtjgpu_decode_device_rgb_select(rtjgpu_ctx *ctx, const uint8_t *d_stream, const rtjgpu_frame_desc *d_desc, int F, int w, int h,
+                                     int S, const int *seq_first, const uint8_t *const *carries,
+                                     int n, const int *sel, int kind, uint8_t *d_rgb, size_t row_pitch, size_t frame_pitch,
+                                     int alpha, uint8_t *const *last_yuv, void *cuda_stream);
+
 /* Host-buffer decode: packets in host memory in, frames in host memory out.
  * The batch is cut into chunks that move through pinned staging buffers with
  * cudaMemcpyAsync on several streams so that copies overlap the kernels.
