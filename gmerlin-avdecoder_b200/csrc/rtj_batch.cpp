@@ -20,32 +20,91 @@
 
 namespace {
 
+/* An owning, grow-only buffer of T in device memory (cudaMalloc) or pinned host memory (cudaMallocHost).  reserve(n)
+ * keeps what it holds when that has room for n elements; otherwise it frees it BEFORE it allocates -- a workspace can be
+ * gigabytes, and holding the old and the new one at once would double the peak while it grows -- and keeps nothing of
+ * the old contents.  The frees are the synchronous ones: they wait for work still in flight on the memory
+ * (rtjgpu_seqenc_destroy relies on that). */
+template <typename T, bool PINNED = false>
+class Buf {
+public:
+    Buf() = default;
+    Buf(const Buf &) = delete;
+    Buf &operator=(const Buf &) = delete;
+    ~Buf() { release(); }
+
+    T *get() const { return p_; }
+    size_t cap() const { return cap_; }          /* elements */
+
+    [[nodiscard]] cudaError_t reserve(size_t n)
+    {
+        if (n <= cap_) return cudaSuccess;
+        release();
+        void *p = nullptr;
+        const cudaError_t e = PINNED ? cudaMallocHost(&p, n * sizeof(T)) : cudaMalloc(&p, n * sizeof(T));
+        if (e != cudaSuccess) return e;
+        p_ = static_cast<T *>(p);
+        cap_ = n;
+        return cudaSuccess;
+    }
+    /* reserve() of memory the caller can do without: a failed allocation is no error and leaves the buffer empty */
+    [[nodiscard]] bool try_reserve(size_t n)
+    {
+        if (reserve(n) == cudaSuccess) return true;
+        cudaGetLastError();
+        return false;
+    }
+    void release()
+    {
+        if (p_) {
+            if (PINNED) cudaFreeHost(p_);
+            else cudaFree(p_);
+        }
+        p_ = nullptr;
+        cap_ = 0;
+    }
+
+private:
+    T     *p_ = nullptr;
+    size_t cap_ = 0;
+};
+
+template <typename T> using PinnedBuf = Buf<T, true>;
+
 struct Workspace {
-    uint32_t     *d_ent = nullptr;
-    uint16_t     *d_src = nullptr;
-    uint32_t     *d_hardq = nullptr;
-    uint16_t     *d_chunk_last = nullptr;
-    uint32_t     *d_chunk_mask = nullptr;     /* (owns the allocation d_chunk_last points into) */
-    size_t        cap_chunk = 0;
-    uint16_t     *d_k3_carry = nullptr;  int    k3_carry_cap = 0;    /* [2][nblk]: last writers handed from slice to slice */
-    int2         *d_walk = nullptr;      int    walk_cap = 0;        /* [F]: where every frame's walker stands between slices */
-    uint32_t     *d_frame_skips = nullptr;
-    rtj_dev_info *d_info = nullptr;
+    Buf<uint32_t>     d_ent;                 /* [F][nblk] */
+    Buf<uint16_t>     d_src;                 /* [F][nblk] */
+    Buf<uint32_t>     d_hardq;               /* [F][nblk][2] */
+    Buf<uint16_t>     d_chunk;               /* K3's notes: chunk_mask(), chunk_last() */
+    Buf<uint8_t>      d_k3;                  /* K3's hand-over: k3_carry(), k3_count(), laid out for k3_nblk positions */
+    int               k3_nblk = 0;
+    Buf<int2>         d_walk;                /* [F]: where every frame's walker stands between slices */
+    Buf<uint32_t>     d_skips;               /* frame_skips(), redo() */
+    Buf<rtj_dev_info> d_info;
     /* segment-parallel scan */
-    uint32_t     *d_seg_sum = nullptr;   size_t seg_sum_cap = 0;     /* entries */
-    uint32_t     *d_seg_entry = nullptr; size_t seg_cap = 0;         /* entries of entry / base */
-    uint32_t     *d_seg_base = nullptr;
-    int32_t      *d_seg_nbf = nullptr;   int    seg_frames_cap = 0;
-    uint8_t      *d_seg_del = nullptr;   size_t seg_del_cap = 0;     /* segments */
-    uint32_t     *d_seg_gsum = nullptr;  size_t seg_gsum_cap = 0;    /* groups */
-    uint32_t     *d_seg_gentry = nullptr, *d_seg_gbase = nullptr;
-    size_t        cap_entries = 0;
-    int           cap_frames = 0;
+    Buf<uint32_t>     d_seg_sum, d_seg_entry, d_seg_base;
+    Buf<int32_t>      d_seg_nbf;
+    Buf<uint8_t>      d_seg_del;
+    Buf<uint32_t>     d_seg_gsum, d_seg_gentry, d_seg_gbase;
     /* K2's position table, rebuilt when the geometry changes */
-    void         *d_lut = nullptr;       size_t lut_cap = 0;     /* bytes */
-    int           lut_fmt = -1, lut_w = 0, lut_h = 0;
+    Buf<uint8_t>      d_lut;
+    int               lut_fmt = -1, lut_w = 0, lut_h = 0;
     /* the sequence layout of a batch of several sequences (seq_upload) */
-    uint8_t      *d_seq = nullptr;       size_t seq_cap = 0;     /* bytes */
+    Buf<uint8_t>      d_seq;
+
+    /* K3's per-chunk notes: a 32-bit skip mask and a 16-bit last writer per (chunk of frames, position), the masks first */
+    static size_t chunk_words(size_t nchunk) { return 3 * nchunk; }
+    uint32_t *chunk_mask() const { return reinterpret_cast<uint32_t *>(d_chunk.get()); }
+    uint16_t *chunk_last() const { return d_chunk.get() + d_chunk.cap() / 3 * 2; }
+    /* [2][nblk] last writers handed from slice to slice, and behind them K3's arrival counters, one per 128 positions
+     * (zero between launches: the last arrival resets its own) */
+    static size_t k3_carry_bytes(size_t nblk) { return (2 * nblk * sizeof(uint16_t) + 15) & ~(size_t)15; }
+    static size_t k3_count_bytes(size_t nblk) { return (nblk / 128 + 1) * sizeof(uint32_t); }
+    uint16_t *k3_carry() const { return reinterpret_cast<uint16_t *>(d_k3.get()); }
+    uint32_t *k3_count() const { return reinterpret_cast<uint32_t *>(d_k3.get() + k3_carry_bytes(k3_nblk)); }
+    /* [F] skipped blocks of every frame, and behind them [F] K1's hand-over flags */
+    uint32_t *frame_skips() const { return d_skips.get(); }
+    uint32_t *redo() const { return d_skips.get() + d_skips.cap() / 2; }
 };
 
 constexpr int HOST_SLOTS = 3;
@@ -64,13 +123,11 @@ struct HostSlot {
     cudaStream_t       stream = nullptr;
     cudaEvent_t        decoded = nullptr;     /* kernels of the chunk in this slot have finished */
     Workspace          ws;
-    uint8_t           *d_in = nullptr;   size_t d_in_cap = 0;
-    uint8_t           *d_out = nullptr;  size_t d_out_cap = 0;
-    rtjgpu_frame_desc *d_desc = nullptr; int    desc_cap = 0;
-    uint8_t           *h_in = nullptr;   size_t h_in_cap = 0;    /* pinned */
-    uint8_t           *h_out = nullptr;  size_t h_out_cap = 0;   /* pinned */
-    rtjgpu_frame_desc *h_desc = nullptr; int    h_desc_cap = 0;  /* pinned */
-    rtj_dev_info      *h_info = nullptr;                         /* pinned read-back of the chunk's counters */
+    Buf<uint8_t>       d_in, d_out;
+    Buf<rtjgpu_frame_desc> d_desc;
+    PinnedBuf<uint8_t> h_in, h_out;
+    PinnedBuf<rtjgpu_frame_desc> h_desc;
+    PinnedBuf<rtj_dev_info> h_info;           /* read-back of the chunk's counters */
     /* pending drain of h_out into the caller's memory */
     uint8_t           *pending_dst = nullptr;
     size_t             pending_bytes = 0;
@@ -82,11 +139,11 @@ struct HostSlot {
 struct rtjgpu_ctx {
     int            device = 0;
     int            last_cuda = 0;
-    rtj_dev_table *d_tables = nullptr;
+    Buf<rtj_dev_table> d_tables;
     rtj_host_table h_tables[RTJ_NUM_TABLES];
     Workspace      ws;                        /* rtjgpu_decode_device */
-    rtj_dev_info  *h_info_reset = nullptr;    /* pinned template {0,0,0,-1} */
-    rtj_dev_info  *h_info = nullptr;          /* pinned read-back */
+    PinnedBuf<rtj_dev_info> h_info_reset;     /* template {0,0,0,-1} */
+    PinnedBuf<rtj_dev_info> h_info;           /* read-back */
     int            last_F = 0;
     void          *last_stream = nullptr;
     bool           timing = false;
@@ -95,8 +152,7 @@ struct rtjgpu_ctx {
     uint64_t       launches = 0;
     HostSlot       slot[HOST_SLOTS];
     bool           slots_ready = false;
-    uint8_t       *d_host_carry = nullptr;    /* carry plane of the host pipeline */
-    size_t         d_host_carry_cap = 0;
+    Buf<uint8_t>   d_host_carry;              /* carry plane of the host pipeline */
     int            scan_mode = RTJGPU_SCAN_AUTO;
     int            format = RTJ_YUV420;
     Pipeline       pipe;
@@ -104,7 +160,7 @@ struct rtjgpu_ctx {
     int            slice_frames = 1184, slice0_frames = 1184;   /* multiples of RTJ_RESOLVE_T */
     bool           scan_priority = false;
     int            frame_run = 0;             /* rtjgpu_set_frame_runs: 0 = by the batch before, 1 = off, n = forced */
-    unsigned long long *h_skips_seen = nullptr;    /* pinned: skipped blocks, raw-prefix frames of the last batch whose K3 has run; raw-prefix frames
+    PinnedBuf<unsigned long long> h_skips_seen;    /* [3] skipped blocks, raw-prefix frames of the last batch whose K3 has run; raw-prefix frames
                                                     * the self-synchronising walk gave up when it was last tried */
     bool           slices_forced = false;     /* rtjgpu_set_pipeline / the environment gave a slice size: it holds in either arrangement */
     /* encoder: configuration, state between calls, workspace */
@@ -112,28 +168,26 @@ struct rtjgpu_ctx {
     int            enc_key_rate = 0, enc_key_count = 0, enc_lm = 0, enc_cm = 0;
     bool           enc_clear_old = true;
     int            enc_w = 0, enc_h = 0, enc_fmt = -1;
-    int32_t       *d_enc_qt = nullptr;
-    int16_t       *d_enc_old = nullptr;       size_t enc_old_cap = 0;      /* blocks */
-    uint8_t       *d_enc_slots = nullptr;     size_t enc_blocks_cap = 0;   /* blocks of a batch */
-    uint8_t       *d_enc_lens = nullptr;
-    uint32_t      *d_enc_boff = nullptr;
-    uint32_t      *d_enc_fsize = nullptr;     size_t enc_frames_cap = 0;
-    uint64_t      *d_enc_total = nullptr;
-    uint64_t      *h_enc_total = nullptr;     /* pinned */
+    Buf<int32_t>   d_enc_qt;                  /* [128] */
+    Buf<int16_t>   d_enc_old;                 /* [nblk][64] */
+    Buf<uint8_t>   d_enc_slots, d_enc_lens;   /* [F][nblk][64], [F][nblk] */
+    Buf<uint32_t>  d_enc_boff, d_enc_fsize;   /* [F][nblk], [F] */
+    Buf<uint64_t>  d_enc_total;               /* [2] */
+    PinnedBuf<uint64_t> h_enc_total;          /* [2] */
     void          *enc_stream = nullptr;
     /* rtjgpu_encode_device_seq: the multipliers of every quality (row 0: the zero tables of a fresh instance), made at the
      * first rtjgpu_seqenc_create; the run table, sequence records and frame words of a call (device copy) */
-    int32_t       *d_enc_qt_all = nullptr;
+    Buf<int32_t>   d_enc_qt_all;
     int            enc_lb8_all[256] = {}, enc_cb8_all[256] = {};
-    uint8_t       *d_enc_seq = nullptr;       size_t enc_seq_cap = 0;      /* bytes */
+    Buf<uint8_t>   d_enc_seq;
     uint64_t       enc_seq_calls = 0;         /* stamps the handles of a call: one seen twice is a duplicate */
     std::vector<rtj_enc_run> enc_runs;        /* host scratch of a call */
     uint64_t       host_bad = 0;              /* overrun frames seen by the current rtjgpu_decode_host call */
-    uint32_t      *h_host_skips = nullptr;    size_t host_skips_cap = 0;   /* pinned: per-frame skip counts of that call */
+    PinnedBuf<uint32_t> h_host_skips;         /* per-frame skip counts of that call */
     int            host_F = 0;
     /* pinned staging of the sequence layouts of rtjgpu_decode_device[_rgb]_seq: two buffers taken in turn, each reused only
      * when its last copy to the device is done */
-    uint8_t       *h_seq[2] = {};             size_t h_seq_cap[2] = {};
+    PinnedBuf<uint8_t> h_seq[2];
     cudaEvent_t    seq_copied[2] = {};
     bool           seq_pending[2] = {};
     int            seq_turn = 0;
@@ -154,48 +208,22 @@ namespace {
 int ws_reserve(rtjgpu_ctx *ctx, Workspace *ws, int F, int nblk)
 {
     const size_t need = (size_t)F * (size_t)nblk;
-    if (need > ws->cap_entries) {
-        if (ws->d_ent) cudaFree(ws->d_ent);
-        if (ws->d_src) cudaFree(ws->d_src);
-        if (ws->d_hardq) cudaFree(ws->d_hardq);
-        ws->d_ent = nullptr; ws->d_src = nullptr; ws->d_hardq = nullptr; ws->cap_entries = 0;
-        CK(ctx, cudaMalloc(&ws->d_ent, need * sizeof(uint32_t)));
-        CK(ctx, cudaMalloc(&ws->d_src, need * sizeof(uint16_t)));
-        CK(ctx, cudaMalloc(&ws->d_hardq, need * 2 * sizeof(uint32_t)));       /* two words an entry: destination and source block */
-        ws->cap_entries = need;
+    CK(ctx, ws->d_ent.reserve(need));
+    CK(ctx, ws->d_src.reserve(need));
+    CK(ctx, ws->d_hardq.reserve(2 * need));          /* two words an entry: destination and source block */
+    /* (sized on their own: few frames of a large picture need more of these than many frames of a small one) */
+    CK(ctx, ws->d_chunk.reserve(Workspace::chunk_words(((size_t)F / RTJ_RESOLVE_T + 1) * (size_t)nblk)));
+    if (nblk > ws->k3_nblk) {                       /* a new layout: allocated afresh, its counters zeroed */
+        ws->d_k3.release();
+        ws->k3_nblk = 0;
+        const size_t carry = Workspace::k3_carry_bytes(nblk), count = Workspace::k3_count_bytes(nblk);
+        CK(ctx, ws->d_k3.reserve(carry + count));
+        CK(ctx, cudaMemset(ws->d_k3.get() + carry, 0, count));
+        ws->k3_nblk = nblk;
     }
-    /* K3's per-chunk notes: a 32-bit skip mask and a 16-bit last writer per (chunk of frames, position), the masks first.
-     * (Sized on its own: few frames of a large picture need more of these than many frames of a small one.) */
-    const size_t nchunk = ((size_t)F / RTJ_RESOLVE_T + 1) * (size_t)nblk;
-    if (nchunk > ws->cap_chunk) {
-        if (ws->d_chunk_mask) cudaFree(ws->d_chunk_mask);
-        ws->d_chunk_mask = nullptr; ws->d_chunk_last = nullptr; ws->cap_chunk = 0;
-        CK(ctx, cudaMalloc(&ws->d_chunk_mask, nchunk * (sizeof(uint32_t) + sizeof(uint16_t))));
-        ws->cap_chunk = nchunk;
-    }
-    ws->d_chunk_last = reinterpret_cast<uint16_t *>(ws->d_chunk_mask + ws->cap_chunk);
-    if (nblk > ws->k3_carry_cap) {
-        if (ws->d_k3_carry) cudaFree(ws->d_k3_carry);
-        ws->d_k3_carry = nullptr; ws->k3_carry_cap = 0;
-        /* ... and behind them K3's arrival counters, one per 128 positions (zero between launches: the last arrival resets its own) */
-        const size_t carry_bytes = ((size_t)2 * nblk * sizeof(uint16_t) + 15) & ~(size_t)15, count_bytes = ((size_t)nblk / 128 + 1) * sizeof(uint32_t);
-        CK(ctx, cudaMalloc(&ws->d_k3_carry, carry_bytes + count_bytes));
-        CK(ctx, cudaMemset(reinterpret_cast<uint8_t *>(ws->d_k3_carry) + carry_bytes, 0, count_bytes));
-        ws->k3_carry_cap = nblk;
-    }
-    if (F > ws->cap_frames) {
-        if (ws->d_frame_skips) cudaFree(ws->d_frame_skips);
-        ws->d_frame_skips = nullptr; ws->cap_frames = 0;
-        CK(ctx, cudaMalloc(&ws->d_frame_skips, (size_t)2 * F * sizeof(uint32_t)));      /* ... and K1's hand-over flags behind them */
-        ws->cap_frames = F;
-    }
-    if (F > ws->walk_cap) {
-        if (ws->d_walk) cudaFree(ws->d_walk);
-        ws->d_walk = nullptr; ws->walk_cap = 0;
-        CK(ctx, cudaMalloc(&ws->d_walk, (size_t)F * sizeof(int2)));
-        ws->walk_cap = F;
-    }
-    if (!ws->d_info) CK(ctx, cudaMalloc(&ws->d_info, sizeof(rtj_dev_info)));
+    CK(ctx, ws->d_skips.reserve(2 * (size_t)F));
+    CK(ctx, ws->d_walk.reserve((size_t)F));
+    CK(ctx, ws->d_info.reserve(1));
     return RTJGPU_OK;
 }
 
@@ -213,7 +241,7 @@ bool auto_wants_segments(const rtjgpu_ctx *ctx, int F, int nblk)
      * count arrives in pinned memory, like the skip count that K2's arrangement goes by). */
     /* (The self-synchronising walk takes such frames at a few us per 40 KB when their streams forget their past -- ordinary
      * material does; noise at a high quality does not, and is what the segment-parallel passes remain for.) */
-    const volatile unsigned long long *seen = ctx->h_skips_seen;
+    const volatile unsigned long long *seen = ctx->h_skips_seen.get();
     if (seen[1]) {
         if (seen[2]) return F <= 256;
         /* measured at a quality of 255 (~9 bytes a block): the walk ~21 us per 40 KB segment of a frame whatever the batch
@@ -239,76 +267,25 @@ int seg_reserve(rtjgpu_ctx *ctx, Workspace *ws, int F, int nblk, int scan_mode, 
     const size_t maxseg = ((size_t)nblk * 64 + RTJ_SEG_BYTES_MB - 1) / RTJ_SEG_BYTES_MB + 1;   /* the smaller segment size rules */
     const size_t nseg = (size_t)F * maxseg, nsum = nseg * RTJ_SEG_NE;
     if (nsum * sizeof(uint32_t) > SEG_MAX_SUM_BYTES) return RTJGPU_OK;          /* too big: one CTA per frame instead */
-    if (nsum > ws->seg_sum_cap) {
-        if (ws->d_seg_sum) cudaFree(ws->d_seg_sum);
-        ws->d_seg_sum = nullptr; ws->seg_sum_cap = 0;
-        CK(ctx, cudaMalloc(&ws->d_seg_sum, nsum * sizeof(uint32_t)));
-        ws->seg_sum_cap = nsum;
-    }
-    if (nseg > ws->seg_cap) {
-        if (ws->d_seg_entry) cudaFree(ws->d_seg_entry);
-        if (ws->d_seg_base) cudaFree(ws->d_seg_base);
-        ws->d_seg_entry = ws->d_seg_base = nullptr; ws->seg_cap = 0;
-        CK(ctx, cudaMalloc(&ws->d_seg_entry, nseg * sizeof(uint32_t)));
-        CK(ctx, cudaMalloc(&ws->d_seg_base, nseg * sizeof(uint32_t)));
-        ws->seg_cap = nseg;
-    }
-    if (F > ws->seg_frames_cap) {
-        if (ws->d_seg_nbf) cudaFree(ws->d_seg_nbf);
-        ws->d_seg_nbf = nullptr; ws->seg_frames_cap = 0;
-        CK(ctx, cudaMalloc(&ws->d_seg_nbf, (size_t)F * sizeof(int32_t)));
-        ws->seg_frames_cap = F;
-    }
-    /* the block lengths of the first pass are kept for the second when that fits (it saves the larger half of the second) */
-    if (nseg * RTJ_SEG_DEL_BYTES <= SEG_MAX_DEL_BYTES) {
-        if (nseg > ws->seg_del_cap) {
-            if (ws->d_seg_del) cudaFree(ws->d_seg_del);
-            ws->d_seg_del = nullptr; ws->seg_del_cap = 0;
-            if (cudaMalloc(&ws->d_seg_del, nseg * RTJ_SEG_DEL_BYTES) == cudaSuccess) ws->seg_del_cap = nseg;
-            else { ws->d_seg_del = nullptr; cudaGetLastError(); }         /* no room: the second pass works them out again */
-        }
-        sp->del = ws->seg_del_cap >= nseg ? ws->d_seg_del : nullptr;
-    }
+    CK(ctx, ws->d_seg_sum.reserve(nsum));
+    CK(ctx, ws->d_seg_entry.reserve(nseg));
+    CK(ctx, ws->d_seg_base.reserve(nseg));
+    CK(ctx, ws->d_seg_nbf.reserve((size_t)F));
+    /* the block lengths of the first pass are kept for the second when that fits (it saves the larger half of the second);
+     * no room: the second pass works them out again */
+    if (nseg * RTJ_SEG_DEL_BYTES <= SEG_MAX_DEL_BYTES)
+        sp->del = ws->d_seg_del.try_reserve(nseg * RTJ_SEG_DEL_BYTES) ? ws->d_seg_del.get() : nullptr;
     if (maxseg >= RTJ_SEG_GROUP_MIN_SEGS) {
         const size_t ngroups = (maxseg + RTJ_SEG_GROUP - 1) / RTJ_SEG_GROUP, ng = (size_t)F * ngroups;
-        if (ng > ws->seg_gsum_cap) {
-            if (ws->d_seg_gsum) cudaFree(ws->d_seg_gsum);
-            if (ws->d_seg_gentry) cudaFree(ws->d_seg_gentry);
-            if (ws->d_seg_gbase) cudaFree(ws->d_seg_gbase);
-            ws->d_seg_gsum = ws->d_seg_gentry = ws->d_seg_gbase = nullptr; ws->seg_gsum_cap = 0;
-            CK(ctx, cudaMalloc(&ws->d_seg_gsum, ng * RTJ_SEG_NE * sizeof(uint32_t)));
-            CK(ctx, cudaMalloc(&ws->d_seg_gentry, ng * sizeof(uint32_t)));
-            CK(ctx, cudaMalloc(&ws->d_seg_gbase, ng * sizeof(uint32_t)));
-            ws->seg_gsum_cap = ng;
-        }
-        sp->gsum = ws->d_seg_gsum; sp->gentry = ws->d_seg_gentry; sp->gbase = ws->d_seg_gbase; sp->ngroups = (int)ngroups;
+        CK(ctx, ws->d_seg_gsum.reserve(ng * RTJ_SEG_NE));
+        CK(ctx, ws->d_seg_gentry.reserve(ng));
+        CK(ctx, ws->d_seg_gbase.reserve(ng));
+        sp->gsum = ws->d_seg_gsum.get(); sp->gentry = ws->d_seg_gentry.get(); sp->gbase = ws->d_seg_gbase.get();
+        sp->ngroups = (int)ngroups;
     }
-    sp->sum = ws->d_seg_sum; sp->entry = ws->d_seg_entry; sp->base = ws->d_seg_base; sp->nbf = ws->d_seg_nbf;
+    sp->sum = ws->d_seg_sum.get(); sp->entry = ws->d_seg_entry.get(); sp->base = ws->d_seg_base.get(); sp->nbf = ws->d_seg_nbf.get();
     sp->maxseg = (int)maxseg;
     return RTJGPU_OK;
-}
-
-void ws_release(Workspace *ws)
-{
-    if (ws->d_ent) cudaFree(ws->d_ent);
-    if (ws->d_src) cudaFree(ws->d_src);
-    if (ws->d_hardq) cudaFree(ws->d_hardq);
-    if (ws->d_chunk_mask) cudaFree(ws->d_chunk_mask);
-    if (ws->d_k3_carry) cudaFree(ws->d_k3_carry);
-    if (ws->d_walk) cudaFree(ws->d_walk);
-    if (ws->d_frame_skips) cudaFree(ws->d_frame_skips);
-    if (ws->d_info) cudaFree(ws->d_info);
-    if (ws->d_seg_sum) cudaFree(ws->d_seg_sum);
-    if (ws->d_seg_entry) cudaFree(ws->d_seg_entry);
-    if (ws->d_seg_base) cudaFree(ws->d_seg_base);
-    if (ws->d_seg_nbf) cudaFree(ws->d_seg_nbf);
-    if (ws->d_seg_del) cudaFree(ws->d_seg_del);
-    if (ws->d_seg_gsum) cudaFree(ws->d_seg_gsum);
-    if (ws->d_seg_gentry) cudaFree(ws->d_seg_gentry);
-    if (ws->d_seg_gbase) cudaFree(ws->d_seg_gbase);
-    if (ws->d_lut) cudaFree(ws->d_lut);
-    if (ws->d_seq) cudaFree(ws->d_seq);
-    *ws = Workspace();
 }
 
 int pipeline_init(rtjgpu_ctx *ctx)
@@ -353,18 +330,6 @@ int plan_slices(const rtjgpu_ctx *ctx, int F, int *first)
     return n;
 }
 
-/*
- * K1 -> K3 -> K2 -> K2b.  ev != NULL brackets the stages with events.
- *
- * The batch is worked through in slices of frames.  Serial arrangement (small batches, the segment-parallel and the
- * serial scans, RTJGPU_PIPELINE_SERIAL): everything on the caller's stream -- K1 over the batch, K3 slice by slice
- * (its look-back never leaves a slice), K2 over the batch.  Pipelined arrangement (allow_pipe, two slices or more):
- * K1 of slice s + 1 runs on a second stream next to K3 / K2 of slice s.  K1 is bound by the ALU pipe and by its
- * barriers, K2 by the FMA pipe: side by side on an SM they fill each other's idle issue slots.  K1's stream has the
- * higher priority, so the CTAs of its next slice (one wave, sized by the slice) take their share of every SM as
- * K2's short-lived CTAs retire.  The last writer of a skipped block lies in an earlier frame, i.e. in a slice
- * that is already scanned, so nothing else has to be ordered.
- */
 /* The sequences of a device batch as the caller gave them: host arrays.  first == NULL: rtjgpu_decode_device[_rgb], one
  * sequence whose carry and last_yuv are carries[0] / last_yuv[0]. */
 struct SeqIn {
@@ -376,92 +341,122 @@ struct SeqIn {
     uint8_t *last(int s) const { return last_yuv ? last_yuv[s] : nullptr; }
 };
 
-/* ... and its device copy (S > 1; all NULL for one sequence: the kernels take the one-stream path) */
-struct SeqDev {
+/* A selection of the batch's frames as the caller gave it: n batch frame indices, strictly increasing (host array). */
+struct SelIn {
+    int        n;
+    const int *idx;
+};
+
+/* where K2's pixels go when they leave as packed RGB (rtjgpu_decode_device_rgb); the last frames as planes go to the
+ * sequences' last_yuv */
+struct RgbOut {
+    uint8_t *d_rgb;
+    size_t   row_pitch, frame_pitch;
+    int      kind;
+    int      alpha;              /* its low byte */
+};
+
+/* What a device decode is given: the batch, its sequences, which frames it wants and where they go -- planes to d_out, or
+ * packed pixels (rgb != NULL).  rtjgpu_scan_device gives the batch alone. */
+struct DecodeCall {
+    const uint8_t           *d_stream;
+    const rtjgpu_frame_desc *d_desc;
+    int                      F, w, h;
+    cudaStream_t             stream;
+    SeqIn                    q;
+    const SelIn             *sel = nullptr;      /* NULL: every frame, at its own index */
+    uint8_t                 *d_out = nullptr;
+    const RgbOut            *rgb = nullptr;
+
+    DecodeCall(const uint8_t *d_stream, const rtjgpu_frame_desc *d_desc, int F, int w, int h, void *stream)
+        : d_stream(d_stream), d_desc(d_desc), F(F), w(w), h(h), stream((cudaStream_t)stream) {}
+};
+
+/* The device copies of a call's tables (seq_upload): the sequence layout (S > 1; all NULL for one sequence: the kernels
+ * take the one-stream path), and a selection's K2 jobs, sorted by frame, on the device and on the host (where the slices'
+ * ranges of jobs are looked up) */
+struct CallDev {
     const uint32_t       *seq = nullptr;         /* [F] RTJ_SEQ(first, index) */
     const uint8_t *const *carries = nullptr;     /* [S] */
     uint8_t *const       *last_yuvs = nullptr;   /* [S] */
+    const uint32_t       *d_jobs = nullptr, *h_jobs = nullptr;
+    int                   njobs = 0;
 };
 
-/* A selection of the batch's frames (rtjgpu_decode_device[_rgb]_select): K2's jobs, sorted by frame, on the device and on
- * the host (where the slices' ranges of jobs are looked up) */
-struct SelDev {
-    const uint32_t *d_jobs = nullptr;
-    const uint32_t *h_jobs = nullptr;
-    int             njobs = 0;
-};
-
-/* where K2's pixels go when they leave as packed RGB (rtjgpu_decode_device_rgb) */
-struct RgbOut {
-    uint8_t *d_rgb = nullptr;
-    size_t   row_pitch = 0, frame_pitch = 0;
-    int      kind = 0;
-    unsigned alpha = 0;
-    uint8_t *d_last_yuv = nullptr;
-};
-
-int run_kernels(rtjgpu_ctx *ctx, Workspace *ws, const uint8_t *d_stream, const rtjgpu_frame_desc *d_desc,
-                int F, int w, int h, uint8_t *d_out, const uint8_t *d_carry, cudaStream_t st, cudaEvent_t *ev,
-                bool allow_pipe, const RgbOut *rgb = nullptr, const SeqDev *seq = nullptr, const SelDev *sel = nullptr)
+/* What K1 reads of rtj_launch_args, for all frames of c on ws; every other field zero */
+rtj_launch_args k1_args(const rtjgpu_ctx *ctx, const Workspace &ws, const DecodeCall &c)
 {
     rtj_launch_args a;
-    a.d_jobs = sel ? sel->d_jobs : nullptr;
-    a.j0 = a.j1 = 0; a.njobs = sel ? sel->njobs : 0;
+    memset(&a, 0, sizeof(a));
+    a.d_stream = c.d_stream; a.d_desc = c.d_desc; a.d_tables = ctx->d_tables.get();
+    a.F = c.F; a.w = c.w; a.h = c.h;
+    a.f0 = 0; a.f1 = c.F;
+    a.fmt = ctx->format;
+    a.row1 = RTJ_FMT_UNITS_Y(ctx->format, c.h);
+    a.raw_expected = ((volatile unsigned long long *)ctx->h_skips_seen.get())[1] != 0;
+    a.d_walk = ws.d_walk.get(); a.d_redo = ws.redo();
+    a.d_ent = ws.d_ent.get(); a.d_frame_skips = ws.frame_skips(); a.d_info = ws.d_info.get();
+    a.scan_mode = ctx->scan_mode;
+    return a;
+}
+
+/*
+ * K1 -> K3 -> K2 -> K2b of call c on workspace ws, with c's tables on the device in dev.  ev != NULL brackets the stages
+ * with events.
+ *
+ * The batch is worked through in slices of frames.  Serial arrangement (small batches, the segment-parallel and the
+ * serial scans, RTJGPU_PIPELINE_SERIAL): everything on the caller's stream -- K1 over the batch, K3 slice by slice
+ * (its look-back never leaves a slice), K2 over the batch.  Pipelined arrangement (allow_pipe, two slices or more):
+ * K1 of slice s + 1 runs on a second stream next to K3 / K2 of slice s.  K1 is bound by the ALU pipe and by its
+ * barriers, K2 by the FMA pipe: side by side on an SM they fill each other's idle issue slots.  K1's stream has the
+ * higher priority, so the CTAs of its next slice (one wave, sized by the slice) take their share of every SM as
+ * K2's short-lived CTAs retire.  The last writer of a skipped block lies in an earlier frame, i.e. in a slice
+ * that is already scanned, so nothing else has to be ordered.
+ */
+int run_kernels(rtjgpu_ctx *ctx, Workspace *ws, const DecodeCall &c, const CallDev &dev, cudaEvent_t *ev, bool allow_pipe)
+{
+    const int F = c.F, nblk = RTJ_FMT_NBLK(ctx->format, c.w, c.h);
+    const cudaStream_t st = c.stream;
+    const RgbOut *rgb = c.rgb;
+    const bool sel = c.sel != nullptr;
+    rtj_launch_args a = k1_args(ctx, *ws, c);
+    a.d_jobs = dev.d_jobs; a.njobs = dev.njobs;
     /* a selection: jobs [j0, j1) are those of frames [f0, f1) (K2 skips a slice that has none) */
     auto job_range = [&](int f0, int f1) {
         auto at = [&](int f) {
-            return (int)(std::partition_point(sel->h_jobs, sel->h_jobs + sel->njobs,
-                                              [f](uint32_t j) { return (int)RTJ_JOB_FRAME(j) < f; }) - sel->h_jobs);
+            return (int)(std::partition_point(dev.h_jobs, dev.h_jobs + dev.njobs,
+                                              [f](uint32_t j) { return (int)RTJ_JOB_FRAME(j) < f; }) - dev.h_jobs);
         };
         a.j0 = at(f0); a.j1 = at(f1);
     };
-    a.d_stream = d_stream; a.d_desc = d_desc; a.d_tables = ctx->d_tables;
-    a.F = F; a.w = w; a.h = h;
-    a.f0 = 0; a.f1 = F; a.slice = 0;
-    a.fmt = ctx->format;
-    a.row0 = 0; a.row1 = RTJ_FMT_UNITS_Y(ctx->format, h);
     /* K2 works through runs of frames with the strip staying on chip when the stream skips blocks -- which only the device
      * knows for this batch.  The batch before is the guide (its count arrives in pinned memory; a count that is not there yet
      * is the one before it): streams do not change their nature from batch to batch, and either arrangement is exact. */
-    a.k2_run = ctx->frame_run ? ctx->frame_run : (*(volatile unsigned long long *)ctx->h_skips_seen ? RTJ_K2_RUN_FRAMES : 1);
-    a.h_skips_seen = ctx->h_skips_seen;
-    a.raw_expected = ((volatile unsigned long long *)ctx->h_skips_seen)[1] != 0;
-    a.d_walk = ws->d_walk;
-    a.d_redo = ws->d_frame_skips + ws->cap_frames;
-    a.d_ent = ws->d_ent; a.d_src = ws->d_src; a.d_frame_skips = ws->d_frame_skips; a.d_info = ws->d_info;
-    a.d_hardq = ws->d_hardq; a.d_chunk_last = ws->d_chunk_last; a.d_chunk_mask = ws->d_chunk_mask;
-    a.d_k3_in = nullptr; a.d_k3_out = ws->d_k3_carry;
-    a.d_k3_count = reinterpret_cast<uint32_t *>(reinterpret_cast<uint8_t *>(ws->d_k3_carry) + (((size_t)2 * ws->k3_carry_cap * sizeof(uint16_t) + 15) & ~(size_t)15));
-    a.d_out = d_out; a.d_carry = d_carry;
-    a.fused_rgb = rgb != nullptr;
-    a.d_rgb = rgb ? rgb->d_rgb : nullptr;
-    a.rgb_row_pitch = rgb ? rgb->row_pitch : 0; a.rgb_frame_pitch = rgb ? rgb->frame_pitch : 0;
-    a.rgb_kind = rgb ? rgb->kind : 0; a.rgb_alpha = rgb ? rgb->alpha : 0; a.d_last_yuv = rgb ? rgb->d_last_yuv : nullptr;
-    a.d_seq = seq ? seq->seq : nullptr; a.d_carries = seq ? seq->carries : nullptr; a.d_last_yuvs = seq ? seq->last_yuvs : nullptr;
-    a.scan_mode = ctx->scan_mode;
-    const int nblk = RTJ_FMT_NBLK(ctx->format, w, h);
+    a.k2_run = ctx->frame_run ? ctx->frame_run : (*(volatile unsigned long long *)ctx->h_skips_seen.get() ? RTJ_K2_RUN_FRAMES : 1);
+    a.h_skips_seen = ctx->h_skips_seen.get();
+    a.d_src = ws->d_src.get(); a.d_hardq = ws->d_hardq.get(); a.d_chunk_last = ws->chunk_last(); a.d_chunk_mask = ws->chunk_mask();
+    a.d_k3_out = ws->k3_carry(); a.d_k3_count = ws->k3_count();
+    a.d_out = c.d_out; a.d_carry = c.q.S > 1 ? nullptr : c.q.carry(0);
+    if (rgb) {
+        a.fused_rgb = 1;
+        a.d_rgb = rgb->d_rgb; a.rgb_row_pitch = rgb->row_pitch; a.rgb_frame_pitch = rgb->frame_pitch;
+        a.rgb_kind = rgb->kind; a.rgb_alpha = (unsigned)rgb->alpha & 0xFFu; a.d_last_yuv = c.q.S > 1 ? nullptr : c.q.last(0);
+    }
+    a.d_seq = dev.seq; a.d_carries = dev.carries; a.d_last_yuvs = dev.last_yuvs;
     {
         const int rc = seg_reserve(ctx, ws, F, nblk, ctx->scan_mode, &a.seg);
         if (rc) return rc;
     }
 
-    a.d_lut = nullptr;
-    {
-        if (ws->lut_fmt != ctx->format || ws->lut_w != w || ws->lut_h != h) {
-            const size_t need = rtj_lut_bytes(ctx->format, w, h);
-            if (need > ws->lut_cap) {
-                if (ws->d_lut) cudaFree(ws->d_lut);
-                ws->d_lut = nullptr; ws->lut_cap = 0; ws->lut_fmt = -1;
-                CK(ctx, cudaMalloc(&ws->d_lut, need));
-                ws->lut_cap = need;
-            }
-            const int e0 = rtj_launch_build_lut(ctx->format, w, h, ws->d_lut, st);
-            if (e0) { ctx->last_cuda = e0; return RTJGPU_E_CUDA; }
-            ws->lut_fmt = ctx->format; ws->lut_w = w; ws->lut_h = h;
-            ctx->launches += 1;
-        }
-        a.d_lut = ws->d_lut;
+    if (ws->lut_fmt != ctx->format || ws->lut_w != c.w || ws->lut_h != c.h) {
+        ws->lut_fmt = -1;                           /* until the table of this geometry is built */
+        CK(ctx, ws->d_lut.reserve(rtj_lut_bytes(ctx->format, c.w, c.h)));
+        const int e0 = rtj_launch_build_lut(ctx->format, c.w, c.h, ws->d_lut.get(), st);
+        if (e0) { ctx->last_cuda = e0; return RTJGPU_E_CUDA; }
+        ws->lut_fmt = ctx->format; ws->lut_w = c.w; ws->lut_h = c.h;
+        ctx->launches += 1;
     }
+    a.d_lut = ws->d_lut.get();
 
     int first[RTJ_MAX_SLICES + 1];
     const int nslices = plan_slices(ctx, F, first);
@@ -469,8 +464,8 @@ int run_kernels(rtjgpu_ctx *ctx, Workspace *ws, const uint8_t *d_stream, const r
     const bool piped = allow_pipe && chunk_scan && nslices >= 2 && ctx->pipeline_mode == RTJGPU_PIPELINE_SLICED;
     auto slice_args = [&](int i) {
         a.f0 = first[i]; a.f1 = first[i + 1]; a.slice = i;
-        a.d_k3_in = i == 0 ? nullptr : ws->d_k3_carry + (size_t)(i & 1) * nblk;
-        a.d_k3_out = ws->d_k3_carry + (size_t)((i + 1) & 1) * nblk;
+        a.d_k3_in = i == 0 ? nullptr : ws->k3_carry() + (size_t)(i & 1) * nblk;
+        a.d_k3_out = ws->k3_carry() + (size_t)((i + 1) & 1) * nblk;
     };
 #define LAUNCHED(call, count)                                                  \
     do {                                                                       \
@@ -479,7 +474,7 @@ int run_kernels(rtjgpu_ctx *ctx, Workspace *ws, const uint8_t *d_stream, const r
         ctx->launches += (count) ? (uint64_t)(count) : (uint64_t)e__;          \
     } while (0)
 
-    CK(ctx, cudaMemcpyAsync(ws->d_info, ctx->h_info_reset, sizeof(rtj_dev_info), cudaMemcpyHostToDevice, st));
+    CK(ctx, cudaMemcpyAsync(ws->d_info.get(), ctx->h_info_reset.get(), sizeof(rtj_dev_info), cudaMemcpyHostToDevice, st));
     if (ev) CK(ctx, cudaEventRecord(ev[0], st));
     if (!piped) {
         LAUNCHED(rtj_launch_scan(&a, st), 0);                  /* returns its launches */
@@ -521,7 +516,7 @@ int run_kernels(rtjgpu_ctx *ctx, Workspace *ws, const uint8_t *d_stream, const r
         CK(ctx, cudaEventRecord(ev[2], p.scan));
     }
     a.f0 = 0; a.f1 = F;
-    if (!rgb && (!sel || sel->njobs > 0)) LAUNCHED(rtj_launch_idct_hard(&a, p.idct), 2);
+    if (!rgb && (!sel || dev.njobs > 0)) LAUNCHED(rtj_launch_idct_hard(&a, p.idct), 2);
     CK(ctx, cudaEventRecord(p.join, p.idct));
     CK(ctx, cudaStreamWaitEvent(st, p.join, 0));
     if (ev) CK(ctx, cudaEventRecord(ev[3], st));
@@ -532,27 +527,8 @@ int run_kernels(rtjgpu_ctx *ctx, Workspace *ws, const uint8_t *d_stream, const r
 inline uint32_t rd_u32le(const uint8_t *p) { return (uint32_t)p[0] | (uint32_t)p[1] << 8 | (uint32_t)p[2] << 16 | (uint32_t)p[3] << 24; }
 inline uint16_t rd_u16le(const uint8_t *p) { return (uint16_t)(p[0] | p[1] << 8); }
 
-template <typename T>
-int grow_device(rtjgpu_ctx *ctx, T **p, size_t *cap, size_t need)
-{
-    if (need <= *cap) return RTJGPU_OK;
-    if (*p) cudaFree(*p);
-    *p = nullptr; *cap = 0;
-    CK(ctx, cudaMalloc(p, need * sizeof(T)));
-    *cap = need;
-    return RTJGPU_OK;
-}
-
-template <typename T>
-int grow_pinned(rtjgpu_ctx *ctx, T **p, size_t *cap, size_t need)
-{
-    if (need <= *cap) return RTJGPU_OK;
-    if (*p) cudaFreeHost(*p);
-    *p = nullptr; *cap = 0;
-    CK(ctx, cudaMallocHost(p, need * sizeof(T)));
-    *cap = need;
-    return RTJGPU_OK;
-}
+/* The picture sizes the library takes: both sides positive multiples of 16 that fit the header's 16-bit fields */
+inline bool valid_size(int w, int h) { return w > 0 && h > 0 && !(w & 15) && !(h & 15) && w <= 65535 && h <= 65535; }
 
 /* The checks of the _seq calls that the one-stream calls do not have. */
 int seq_check(int F, const SeqIn &q)
@@ -576,34 +552,35 @@ int stage_begin(rtjgpu_ctx *ctx, size_t bytes, uint8_t **h)
         CK(ctx, cudaEventSynchronize(ctx->seq_copied[t]));
         ctx->seq_pending[t] = false;
     }
-    const int rc = grow_pinned(ctx, &ctx->h_seq[t], &ctx->h_seq_cap[t], bytes);
-    *h = ctx->h_seq[t];
-    return rc;
+    CK(ctx, ctx->h_seq[t].reserve(bytes));
+    *h = ctx->h_seq[t].get();
+    return RTJGPU_OK;
 }
 
 int stage_end(rtjgpu_ctx *ctx, void *d_dst, size_t bytes, cudaStream_t st)
 {
     const int t = ctx->seq_turn;
-    CK(ctx, cudaMemcpyAsync(d_dst, ctx->h_seq[t], bytes, cudaMemcpyHostToDevice, st));
+    CK(ctx, cudaMemcpyAsync(d_dst, ctx->h_seq[t].get(), bytes, cudaMemcpyHostToDevice, st));
     CK(ctx, cudaEventRecord(ctx->seq_copied[t], st));
     ctx->seq_pending[t] = true;
     ctx->seq_turn = t ^ 1;
     return RTJGPU_OK;
 }
 
-/* The device copy of a layout of S > 1 sequences, in the workspace: [F] RTJ_SEQ words, then [S] carry pointers, then
- * [S] last_yuv pointers -- and behind them, for a selection (jobs != NULL), its ctx->sel_jobs: one copy either way.  S = 1
- * uploads the jobs alone. */
-int seq_upload(rtjgpu_ctx *ctx, Workspace *ws, int F, const SeqIn &q, cudaStream_t st, SeqDev *out, SelDev *jobs = nullptr)
+/* The device copy of c's layout of S > 1 sequences, in the workspace: [F] RTJ_SEQ words, then [S] carry pointers, then
+ * [S] last_yuv pointers -- and behind them, for a selection, its ctx->sel_jobs: one copy either way.  S = 1 uploads the
+ * jobs alone. */
+int seq_upload(rtjgpu_ctx *ctx, Workspace *ws, const DecodeCall &c, CallDev *out)
 {
+    const SeqIn &q = c.q;
     const bool layout = q.S > 1;
-    const size_t words = layout ? ((size_t)F * sizeof(uint32_t) + 7) & ~(size_t)7 : 0, ptrs = layout ? (size_t)q.S * sizeof(void *) : 0;
-    const size_t jbytes = jobs ? ctx->sel_jobs.size() * sizeof(uint32_t) : 0;
+    const size_t words = layout ? ((size_t)c.F * sizeof(uint32_t) + 7) & ~(size_t)7 : 0, ptrs = layout ? (size_t)q.S * sizeof(void *) : 0;
+    const size_t jbytes = c.sel ? ctx->sel_jobs.size() * sizeof(uint32_t) : 0;
     const size_t bytes = words + 2 * ptrs + jbytes;
     uint8_t *h;
     int rc = stage_begin(ctx, bytes, &h);
     if (rc) return rc;
-    if ((rc = grow_device(ctx, &ws->d_seq, &ws->seq_cap, bytes))) return rc;
+    CK(ctx, ws->d_seq.reserve(bytes));
     if (layout) {
         uint32_t *hw = reinterpret_cast<uint32_t *>(h);
         for (int s = 0; s < q.S; s++)
@@ -613,25 +590,20 @@ int seq_upload(rtjgpu_ctx *ctx, Workspace *ws, int F, const SeqIn &q, cudaStream
         for (int s = 0; s < q.S; s++) { hc[s] = q.carry(s); hl[s] = q.last(s); }
     }
     if (jbytes) memcpy(h + words + 2 * ptrs, ctx->sel_jobs.data(), jbytes);
-    if ((rc = stage_end(ctx, ws->d_seq, bytes, st))) return rc;
+    const uint8_t *d = ws->d_seq.get();
+    if ((rc = stage_end(ctx, ws->d_seq.get(), bytes, c.stream))) return rc;
     if (layout) {
-        out->seq = reinterpret_cast<const uint32_t *>(ws->d_seq);
-        out->carries = reinterpret_cast<const uint8_t *const *>(ws->d_seq + words);
-        out->last_yuvs = reinterpret_cast<uint8_t *const *>(ws->d_seq + words + ptrs);
+        out->seq = reinterpret_cast<const uint32_t *>(d);
+        out->carries = reinterpret_cast<const uint8_t *const *>(d + words);
+        out->last_yuvs = reinterpret_cast<uint8_t *const *>(d + words + ptrs);
     }
-    if (jobs) {
-        jobs->d_jobs = reinterpret_cast<const uint32_t *>(ws->d_seq + words + 2 * ptrs);
-        jobs->h_jobs = ctx->sel_jobs.data();
-        jobs->njobs = (int)ctx->sel_jobs.size();
+    if (c.sel) {
+        out->d_jobs = reinterpret_cast<const uint32_t *>(d + words + 2 * ptrs);
+        out->h_jobs = ctx->sel_jobs.data();
+        out->njobs = (int)ctx->sel_jobs.size();
     }
     return RTJGPU_OK;
 }
-
-/* A selection of the batch's frames as the caller gave it: n batch frame indices, strictly increasing (host array). */
-struct SelIn {
-    int        n = 0;
-    const int *idx = nullptr;
-};
 
 int sel_check(int F, const SelIn &s)
 {
@@ -659,116 +631,75 @@ void sel_jobs(rtjgpu_ctx *ctx, const SeqIn &q, const SelIn &s, bool rgb_last)
     }
 }
 
-/* rtjgpu_decode_device and rtjgpu_decode_device_seq: the former is the latter's one-sequence case.  sel != NULL:
- * rtjgpu_decode_device_select (q.first given), which is rtjgpu_decode_device_seq when it selects every frame. */
-int decode_device(rtjgpu_ctx *ctx, const uint8_t *d_stream, const rtjgpu_frame_desc *d_desc, int F, int w, int h,
-                  const SeqIn &q, uint8_t *d_out, void *cuda_stream, const SelIn *sel = nullptr)
+/* The checks every device call makes once its sequences and selection are known to be consistent (decode()): pointers,
+ * alignment, geometry, batch size -- in this order, and before anything is reserved or launched.  Without `output`
+ * (rtjgpu_scan_device) the output, carry and last_yuv pointers are not looked at.  Sets the device and *nblk. */
+int check_batch(rtjgpu_ctx *ctx, const DecodeCall &c, bool output, int *nblk)
 {
-    if (!ctx || F < 0) return RTJGPU_E_ARG;
-    if (q.first) {
-        const int rc = seq_check(F, q);
-        if (rc) return rc;
-    }
-    if (sel) {
-        const int rc = sel_check(F, *sel);
-        if (rc) return rc;
-        if (sel->n == F) sel = nullptr;                      /* every frame: the full call, runs of frames included */
-    }
-    if (F == 0) { ctx->last_F = 0; return RTJGPU_OK; }
-    if (!d_stream || !d_desc || (!d_out && !(sel && sel->n == 0))) return RTJGPU_E_ARG;
+    uint8_t *const dst = c.rgb ? c.rgb->d_rgb : c.d_out;
+    if (!c.d_stream || !c.d_desc || (output && !dst && !(c.sel && c.sel->n == 0))) return RTJGPU_E_ARG;
     /* K1 reads the stream as 32-bit words, K2 leaves its strips as 16-byte bulk stores and reads the carry as 8-byte rows */
-    if (((uintptr_t)d_stream & 3) || ((uintptr_t)d_desc & 7) || ((uintptr_t)d_out & 15) || ((uintptr_t)q.carry(0) & 7)) return RTJGPU_E_ARG;
-    if (w <= 0 || h <= 0 || (w & 15) || (h & 15) || w > 65535 || h > 65535) return RTJGPU_E_SIZE;
-    if (F > RTJGPU_MAX_FRAMES_PER_BATCH) return RTJGPU_E_TOOBIG;
+    if (((uintptr_t)c.d_stream & 3) || ((uintptr_t)c.d_desc & 7)) return RTJGPU_E_ARG;
+    if (output && (((uintptr_t)dst & 15) || ((uintptr_t)c.q.carry(0) & 7) || ((uintptr_t)c.q.last(0) & 15))) return RTJGPU_E_ARG;
+    if (output && c.rgb) {
+        const RgbOut &o = *c.rgb;
+        if ((o.row_pitch & 15) || (o.frame_pitch & 15) || o.row_pitch < (size_t)c.w * rtj_convert_bpp(o.kind)
+            || o.frame_pitch < o.row_pitch * (size_t)c.h)
+            return RTJGPU_E_ARG;
+    }
+    if (!valid_size(c.w, c.h)) return RTJGPU_E_SIZE;
+    if (c.F > RTJGPU_MAX_FRAMES_PER_BATCH) return RTJGPU_E_TOOBIG;
     CK(ctx, cudaSetDevice(ctx->device));
-    const int nblk = RTJ_FMT_NBLK(ctx->format, w, h);
-    if ((uint64_t)F * (uint64_t)nblk >= (1ull << 32)) return RTJGPU_E_TOOBIG;   /* block indices are 32 bit */
-    if ((uint64_t)RTJ_FMT_FRAME_BYTES(ctx->format, w, h) >= (1ull << 32)) return RTJGPU_E_TOOBIG;   /* and so are offsets inside a frame */
-    int rc = ws_reserve(ctx, &ctx->ws, F, nblk);
-    if (rc) return rc;
-    SeqDev sd;
-    SelDev jd;
-    if (sel) sel_jobs(ctx, q, *sel, false);
-    if ((q.S > 1 || (sel && sel->n > 0)) && (rc = seq_upload(ctx, &ctx->ws, F, q, (cudaStream_t)cuda_stream, &sd, sel ? &jd : nullptr)))
-        return rc;
-    cudaEvent_t *ev = ctx->timing ? ctx->ev[ctx->timed_calls % TIMING_RING] : nullptr;
-    rc = run_kernels(ctx, &ctx->ws, d_stream, d_desc, F, w, h, d_out, q.S > 1 ? nullptr : q.carry(0), (cudaStream_t)cuda_stream, ev,
-                     true, nullptr, q.S > 1 ? &sd : nullptr, sel ? &jd : nullptr);
-    if (ev && rc == RTJGPU_OK) ctx->timed_calls++;
-    ctx->last_F = F;
-    ctx->last_stream = cuda_stream;
-    return rc;
+    *nblk = RTJ_FMT_NBLK(ctx->format, c.w, c.h);
+    if ((uint64_t)c.F * (uint64_t)*nblk >= (1ull << 32)) return RTJGPU_E_TOOBIG;   /* block indices are 32 bit */
+    if ((uint64_t)RTJ_FMT_FRAME_BYTES(ctx->format, c.w, c.h) >= (1ull << 32)) return RTJGPU_E_TOOBIG;   /* and so are offsets inside a frame */
+    return RTJGPU_OK;
 }
 
-/* rtjgpu_decode_device_rgb and rtjgpu_decode_device_rgb_seq; sel != NULL: rtjgpu_decode_device_rgb_select */
-int decode_device_rgb(rtjgpu_ctx *ctx, const uint8_t *d_stream, const rtjgpu_frame_desc *d_desc, int F, int w, int h,
-                      const SeqIn &q, int kind, uint8_t *d_rgb, size_t row_pitch, size_t frame_pitch, int alpha, void *cuda_stream,
-                      const SelIn *sel = nullptr)
+/* Every rtjgpu_decode_device* call: rtjgpu_decode_device is the one-sequence case of rtjgpu_decode_device_seq, which is
+ * rtjgpu_decode_device_select selecting every frame; the same three with packed pixels out (c.rgb) */
+int decode(rtjgpu_ctx *ctx, DecodeCall c)
 {
-    if (!ctx || F < 0) return RTJGPU_E_ARG;
-    if (ctx->format != RTJ_YUV420) return RTJGPU_E_FORMAT;                     /* the reference's converters are yuv420 ones */
-    if (kind != RTJ_CONV_RGB32 && kind != RTJ_CONV_BGR32 && kind != RTJ_CONV_RGB24 && kind != RTJ_CONV_BGR24 && kind != RTJ_CONV_RGB16)
-        return RTJGPU_E_FORMAT;
-    if (q.first) {
-        const int rc = seq_check(F, q);
-        if (rc) return rc;
+    if (!ctx || c.F < 0) return RTJGPU_E_ARG;
+    if (c.rgb) {
+        if (ctx->format != RTJ_YUV420) return RTJGPU_E_FORMAT;                 /* the reference's converters are yuv420 ones */
+        const int k = c.rgb->kind;
+        if (k != RTJ_CONV_RGB32 && k != RTJ_CONV_BGR32 && k != RTJ_CONV_RGB24 && k != RTJ_CONV_BGR24 && k != RTJ_CONV_RGB16)
+            return RTJGPU_E_FORMAT;
     }
-    if (sel) {
-        const int rc = sel_check(F, *sel);
-        if (rc) return rc;
-        if (sel->n == F) sel = nullptr;                      /* every frame: the full call, last frames as planes included */
+    int rc;
+    if (c.q.first && (rc = seq_check(c.F, c.q))) return rc;
+    if (c.sel) {
+        if ((rc = sel_check(c.F, *c.sel))) return rc;
+        if (c.sel->n == c.F) c.sel = nullptr;         /* every frame: the full call, runs of frames and last frames as planes included */
     }
-    if (F == 0) { ctx->last_F = 0; return RTJGPU_OK; }
-    if (!d_stream || !d_desc || (!d_rgb && !(sel && sel->n == 0))) return RTJGPU_E_ARG;
-    if (w <= 0 || h <= 0 || (w & 15) || (h & 15) || w > 65535 || h > 65535) return RTJGPU_E_SIZE;
-    if (F > RTJGPU_MAX_FRAMES_PER_BATCH) return RTJGPU_E_TOOBIG;
-    const int bpp = rtj_convert_bpp(kind);
-    if (((uintptr_t)d_stream & 3) || ((uintptr_t)d_desc & 7) || ((uintptr_t)d_rgb & 15) || ((uintptr_t)q.carry(0) & 7)
-        || ((uintptr_t)q.last(0) & 15) || (row_pitch & 15) || (frame_pitch & 15) || row_pitch < (size_t)w * bpp
-        || frame_pitch < row_pitch * (size_t)h)
-        return RTJGPU_E_ARG;
-    CK(ctx, cudaSetDevice(ctx->device));
-    const int nblk = RTJ_FMT_NBLK(ctx->format, w, h);
-    if ((uint64_t)F * (uint64_t)nblk >= (1ull << 32)) return RTJGPU_E_TOOBIG;
-    int rc = ws_reserve(ctx, &ctx->ws, F, nblk);
-    if (rc) return rc;
-    SeqDev sd;
-    SelDev jd;
-    if (sel) sel_jobs(ctx, q, *sel, true);
-    if ((q.S > 1 || (sel && !ctx->sel_jobs.empty())) && (rc = seq_upload(ctx, &ctx->ws, F, q, (cudaStream_t)cuda_stream, &sd, sel ? &jd : nullptr)))
-        return rc;
-    RgbOut o;
-    o.d_rgb = d_rgb; o.row_pitch = row_pitch; o.frame_pitch = frame_pitch; o.kind = kind; o.alpha = (unsigned)alpha & 0xFFu;
-    o.d_last_yuv = q.S > 1 ? nullptr : q.last(0);
+    if (c.F == 0) { ctx->last_F = 0; return RTJGPU_OK; }
+    int nblk;
+    if ((rc = check_batch(ctx, c, true, &nblk))) return rc;
+    if ((rc = ws_reserve(ctx, &ctx->ws, c.F, nblk))) return rc;
+    CallDev dev;
+    if (c.sel) sel_jobs(ctx, c.q, *c.sel, c.rgb != nullptr);
+    if ((c.q.S > 1 || (c.sel && !ctx->sel_jobs.empty())) && (rc = seq_upload(ctx, &ctx->ws, c, &dev))) return rc;
     cudaEvent_t *ev = ctx->timing ? ctx->ev[ctx->timed_calls % TIMING_RING] : nullptr;
-    rc = run_kernels(ctx, &ctx->ws, d_stream, d_desc, F, w, h, nullptr, q.S > 1 ? nullptr : q.carry(0), (cudaStream_t)cuda_stream, ev,
-                     true, &o, q.S > 1 ? &sd : nullptr, sel ? &jd : nullptr);
+    rc = run_kernels(ctx, &ctx->ws, c, dev, ev, true);
     if (ev && rc == RTJGPU_OK) ctx->timed_calls++;
-    ctx->last_F = F;
-    ctx->last_stream = cuda_stream;
+    ctx->last_F = c.F;
+    ctx->last_stream = c.stream;
     return rc;
 }
 
 /* The encoder's workspace for F pictures of nblk blocks, shared by rtjgpu_encode_device and rtjgpu_encode_device_seq
- * (both on the stream of the call that uses it) */
+ * (both on the stream of the call that uses it), and the totals rtjgpu_get_encode_info reads back */
 int enc_reserve(rtjgpu_ctx *ctx, size_t nblk, int F)
 {
-    if (!ctx->d_enc_total) {
-        CK(ctx, cudaMalloc(&ctx->d_enc_total, 2 * sizeof(uint64_t)));
-        CK(ctx, cudaMallocHost(&ctx->h_enc_total, 2 * sizeof(uint64_t)));
-    }
     const size_t nb = nblk * (size_t)F;
-    if (nb > ctx->enc_blocks_cap) {
-        if (ctx->d_enc_slots) cudaFree(ctx->d_enc_slots);
-        if (ctx->d_enc_lens) cudaFree(ctx->d_enc_lens);
-        if (ctx->d_enc_boff) cudaFree(ctx->d_enc_boff);
-        ctx->d_enc_slots = nullptr; ctx->d_enc_lens = nullptr; ctx->d_enc_boff = nullptr; ctx->enc_blocks_cap = 0;
-        CK(ctx, cudaMalloc(&ctx->d_enc_slots, nb * 64));
-        CK(ctx, cudaMalloc(&ctx->d_enc_lens, nb));
-        CK(ctx, cudaMalloc(&ctx->d_enc_boff, nb * sizeof(uint32_t)));
-        ctx->enc_blocks_cap = nb;
-    }
-    return grow_device(ctx, &ctx->d_enc_fsize, &ctx->enc_frames_cap, (size_t)F);
+    CK(ctx, ctx->d_enc_total.reserve(2));
+    CK(ctx, ctx->h_enc_total.reserve(2));
+    CK(ctx, ctx->d_enc_slots.reserve(nb * 64));
+    CK(ctx, ctx->d_enc_lens.reserve(nb));
+    CK(ctx, ctx->d_enc_boff.reserve(nb));
+    CK(ctx, ctx->d_enc_fsize.reserve((size_t)F));
+    return RTJGPU_OK;
 }
 
 } // namespace
@@ -824,15 +755,17 @@ int rtjgpu_create(int device, rtjgpu_ctx **out)
         std::vector<rtj_dev_table> dev(RTJ_NUM_TABLES);
         for (int q = 1; q <= 255; q++) rtj_table_from_quality(q, &ctx->h_tables[q]);
         for (int t = 0; t < RTJ_NUM_TABLES; t++) rtj_table_to_device_layout(&ctx->h_tables[t], &dev[t]);
-        if ((e = cudaMalloc(&ctx->d_tables, sizeof(rtj_dev_table) * RTJ_NUM_TABLES)) != cudaSuccess) { rc = RTJGPU_E_CUDA; break; }
-        if ((e = cudaMemcpy(ctx->d_tables, dev.data(), sizeof(rtj_dev_table) * RTJ_NUM_TABLES, cudaMemcpyHostToDevice)) != cudaSuccess) { rc = RTJGPU_E_CUDA; break; }
-        if ((e = cudaMallocHost(&ctx->h_info_reset, sizeof(rtj_dev_info))) != cudaSuccess) { rc = RTJGPU_E_CUDA; break; }
-        if ((e = cudaMallocHost(&ctx->h_info, sizeof(rtj_dev_info))) != cudaSuccess) { rc = RTJGPU_E_CUDA; break; }
-        if ((e = cudaMallocHost(&ctx->h_skips_seen, 3 * sizeof(unsigned long long))) != cudaSuccess) { rc = RTJGPU_E_CUDA; break; }
-        ctx->h_skips_seen[0] = ctx->h_skips_seen[1] = ctx->h_skips_seen[2] = 0;
-        memset(ctx->h_info_reset, 0, sizeof(rtj_dev_info));
-        ctx->h_info_reset->first_bad_frame = -1;
-        *ctx->h_info = *ctx->h_info_reset;
+        if ((e = ctx->d_tables.reserve(RTJ_NUM_TABLES)) != cudaSuccess) { rc = RTJGPU_E_CUDA; break; }
+        if ((e = cudaMemcpy(ctx->d_tables.get(), dev.data(), sizeof(rtj_dev_table) * RTJ_NUM_TABLES, cudaMemcpyHostToDevice)) != cudaSuccess) { rc = RTJGPU_E_CUDA; break; }
+        if ((e = ctx->h_info_reset.reserve(1)) != cudaSuccess) { rc = RTJGPU_E_CUDA; break; }
+        if ((e = ctx->h_info.reserve(1)) != cudaSuccess) { rc = RTJGPU_E_CUDA; break; }
+        if ((e = ctx->h_skips_seen.reserve(3)) != cudaSuccess) { rc = RTJGPU_E_CUDA; break; }
+        unsigned long long *seen = ctx->h_skips_seen.get();
+        seen[0] = seen[1] = seen[2] = 0;
+        rtj_dev_info *reset = ctx->h_info_reset.get();
+        memset(reset, 0, sizeof(rtj_dev_info));
+        reset->first_bad_frame = -1;
+        *ctx->h_info.get() = *reset;
         for (int i = 0; i < TIMING_RING * 4 && rc == RTJGPU_OK; i++)
             if ((e = cudaEventCreate(&ctx->ev[i / 4][i % 4])) != cudaSuccess) rc = RTJGPU_E_CUDA;
     } while (0);
@@ -850,43 +783,14 @@ void rtjgpu_destroy(rtjgpu_ctx *ctx)
     if (!ctx) return;
     cudaSetDevice(ctx->device);
     cudaDeviceSynchronize();
-    ws_release(&ctx->ws);
     pipeline_release(&ctx->pipe);
-    for (int i = 0; i < HOST_SLOTS; i++) {
-        HostSlot &s = ctx->slot[i];
-        ws_release(&s.ws);
-        if (s.d_in) cudaFree(s.d_in);
-        if (s.d_out) cudaFree(s.d_out);
-        if (s.d_desc) cudaFree(s.d_desc);
-        if (s.h_in) cudaFreeHost(s.h_in);
-        if (s.h_out) cudaFreeHost(s.h_out);
-        if (s.h_desc) cudaFreeHost(s.h_desc);
-        if (s.h_info) cudaFreeHost(s.h_info);
+    for (HostSlot &s : ctx->slot) {
         if (s.decoded) cudaEventDestroy(s.decoded);
         if (s.stream) cudaStreamDestroy(s.stream);
     }
-    if (ctx->d_host_carry) cudaFree(ctx->d_host_carry);
-    if (ctx->h_host_skips) cudaFreeHost(ctx->h_host_skips);
-    if (ctx->d_enc_qt) cudaFree(ctx->d_enc_qt);
-    if (ctx->d_enc_old) cudaFree(ctx->d_enc_old);
-    if (ctx->d_enc_slots) cudaFree(ctx->d_enc_slots);
-    if (ctx->d_enc_lens) cudaFree(ctx->d_enc_lens);
-    if (ctx->d_enc_boff) cudaFree(ctx->d_enc_boff);
-    if (ctx->d_enc_fsize) cudaFree(ctx->d_enc_fsize);
-    if (ctx->d_enc_total) cudaFree(ctx->d_enc_total);
-    if (ctx->h_enc_total) cudaFreeHost(ctx->h_enc_total);
-    if (ctx->d_enc_qt_all) cudaFree(ctx->d_enc_qt_all);
-    if (ctx->d_enc_seq) cudaFree(ctx->d_enc_seq);
-    if (ctx->d_tables) cudaFree(ctx->d_tables);
-    if (ctx->h_info_reset) cudaFreeHost(ctx->h_info_reset);
-    if (ctx->h_info) cudaFreeHost(ctx->h_info);
-    if (ctx->h_skips_seen) cudaFreeHost(ctx->h_skips_seen);
-    for (int i = 0; i < 2; i++) {
-        if (ctx->h_seq[i]) cudaFreeHost(ctx->h_seq[i]);
-        if (ctx->seq_copied[i]) cudaEventDestroy(ctx->seq_copied[i]);
-    }
+    for (cudaEvent_t e : ctx->seq_copied) if (e) cudaEventDestroy(e);
     for (int i = 0; i < TIMING_RING * 4; i++) if (ctx->ev[i / 4][i % 4]) cudaEventDestroy(ctx->ev[i / 4][i % 4]);
-    delete ctx;
+    delete ctx;                                 /* (and with it every buffer it holds) */
 }
 
 int rtjgpu_last_cuda_error(const rtjgpu_ctx *ctx) { return ctx ? ctx->last_cuda : 0; }
@@ -935,9 +839,9 @@ int rtjgpu_encoder_set_quality(rtjgpu_ctx *ctx, int quality)
     if (quality > 255) quality = 255;
     int32_t qt[128];
     rtj_encoder_table_from_quality(quality, qt, &ctx->enc_lb8, &ctx->enc_cb8);
-    if (!ctx->d_enc_qt) CK(ctx, cudaMalloc(&ctx->d_enc_qt, sizeof(qt)));
+    CK(ctx, ctx->d_enc_qt.reserve(128));
     if (ctx->enc_stream) CK(ctx, cudaStreamSynchronize((cudaStream_t)ctx->enc_stream));   /* a batch may still read the old tables */
-    CK(ctx, cudaMemcpy(ctx->d_enc_qt, qt, sizeof(qt), cudaMemcpyHostToDevice));
+    CK(ctx, cudaMemcpy(ctx->d_enc_qt.get(), qt, sizeof(qt), cudaMemcpyHostToDevice));
     ctx->enc_quality = quality;
     return RTJGPU_OK;
 }
@@ -965,44 +869,40 @@ int rtjgpu_encode_device(rtjgpu_ctx *ctx, const uint8_t *d_frames, int F, int w,
 {
     if (!ctx || F < 0) return RTJGPU_E_ARG;
     if (ctx->format != RTJ_YUV420 && ctx->format != RTJ_YUV422) return RTJGPU_E_FORMAT;
-    if (w <= 0 || h <= 0 || (w & 15) || (h & 15) || w > 65535 || h > 65535) return RTJGPU_E_SIZE;
+    if (!valid_size(w, h)) return RTJGPU_E_SIZE;
     if (F > RTJGPU_MAX_FRAMES_PER_BATCH) return RTJGPU_E_TOOBIG;
     if (!d_offsets || (F && (!d_frames || !d_stream)) || ((uintptr_t)d_frames & 7) || ((uintptr_t)d_stream & 3)) return RTJGPU_E_ARG;
     CK(ctx, cudaSetDevice(ctx->device));
     cudaStream_t st = (cudaStream_t)cuda_stream;
     const size_t nblk = (size_t)RTJ_FMT_NBLK(ctx->format, w, h);
-    if (!ctx->d_enc_qt) {                /* never configured: the all-zero tables of a fresh RTjpeg_t (lib/RTjpeg.c:2499) */
-        CK(ctx, cudaMalloc(&ctx->d_enc_qt, 128 * sizeof(int32_t)));
-        CK(ctx, cudaMemset(ctx->d_enc_qt, 0, 128 * sizeof(int32_t)));
+    if (!ctx->d_enc_qt.get()) {          /* never configured: the all-zero tables of a fresh RTjpeg_t (lib/RTjpeg.c:2499) */
+        CK(ctx, ctx->d_enc_qt.reserve(128));
+        CK(ctx, cudaMemset(ctx->d_enc_qt.get(), 0, 128 * sizeof(int32_t)));
     }
-    if (!ctx->d_enc_total) {
-        CK(ctx, cudaMalloc(&ctx->d_enc_total, 2 * sizeof(uint64_t)));
-        CK(ctx, cudaMallocHost(&ctx->h_enc_total, 2 * sizeof(uint64_t)));
-    }
+    int rc = enc_reserve(ctx, nblk, F);             /* (F = 0: the totals alone) */
+    if (rc) return rc;
     if (ctx->enc_w != w || ctx->enc_h != h || ctx->enc_fmt != ctx->format) {
         ctx->enc_w = w; ctx->enc_h = h; ctx->enc_fmt = ctx->format;
         ctx->enc_clear_old = true;
     }
-    int rc = grow_device(ctx, &ctx->d_enc_old, &ctx->enc_old_cap, nblk * 64);
-    if (rc) return rc;
+    CK(ctx, ctx->d_enc_old.reserve(nblk * 64));
     if (ctx->enc_clear_old) {
-        CK(ctx, cudaMemsetAsync(ctx->d_enc_old, 0, nblk * 64 * sizeof(int16_t), st));
+        CK(ctx, cudaMemsetAsync(ctx->d_enc_old.get(), 0, nblk * 64 * sizeof(int16_t), st));
         ctx->enc_clear_old = false;
     }
     ctx->enc_stream = cuda_stream;
     if (F == 0) {
         CK(ctx, cudaMemsetAsync(d_offsets, 0, sizeof(uint64_t), st));
-        CK(ctx, cudaMemsetAsync(ctx->d_enc_total, 0, 2 * sizeof(uint64_t), st));
+        CK(ctx, cudaMemsetAsync(ctx->d_enc_total.get(), 0, 2 * sizeof(uint64_t), st));
         return RTJGPU_OK;
     }
-    if ((rc = enc_reserve(ctx, nblk, F))) return rc;
     rtj_encode_args a;
     a.d_frames = d_frames; a.F = F; a.w = w; a.h = h; a.fmt = ctx->format;
-    a.d_qt = ctx->d_enc_qt; a.lb8 = ctx->enc_lb8; a.cb8 = ctx->enc_cb8; a.quality = ctx->enc_quality;
+    a.d_qt = ctx->d_enc_qt.get(); a.lb8 = ctx->enc_lb8; a.cb8 = ctx->enc_cb8; a.quality = ctx->enc_quality;
     a.key_rate = ctx->enc_key_rate; a.key_count0 = ctx->enc_key_count; a.lmask = ctx->enc_lm; a.cmask = ctx->enc_cm;
-    a.d_old = ctx->d_enc_old; a.d_slots = ctx->d_enc_slots; a.d_lens = ctx->d_enc_lens; a.d_boff = ctx->d_enc_boff;
-    a.d_fsize = ctx->d_enc_fsize; a.d_stream = d_stream; a.capacity = capacity; a.d_offsets = d_offsets;
-    a.d_total = ctx->d_enc_total;
+    a.d_old = ctx->d_enc_old.get(); a.d_slots = ctx->d_enc_slots.get(); a.d_lens = ctx->d_enc_lens.get(); a.d_boff = ctx->d_enc_boff.get();
+    a.d_fsize = ctx->d_enc_fsize.get(); a.d_stream = d_stream; a.capacity = capacity; a.d_offsets = d_offsets;
+    a.d_total = ctx->d_enc_total.get();
     const int e = rtj_launch_encode(&a, cuda_stream);
     if (e < 0) { ctx->last_cuda = -e; return RTJGPU_E_CUDA; }
     ctx->launches += (uint64_t)e;
@@ -1012,13 +912,14 @@ int rtjgpu_encode_device(rtjgpu_ctx *ctx, const uint8_t *d_frames, int F, int w,
 
 int rtjgpu_get_encode_info(rtjgpu_ctx *ctx, uint64_t *bytes, int *overflow)
 {
-    if (!ctx || !ctx->d_enc_total) return RTJGPU_E_ARG;
+    if (!ctx || !ctx->d_enc_total.get()) return RTJGPU_E_ARG;
     CK(ctx, cudaSetDevice(ctx->device));
     cudaStream_t st = (cudaStream_t)ctx->enc_stream;
-    CK(ctx, cudaMemcpyAsync(ctx->h_enc_total, ctx->d_enc_total, 2 * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+    const uint64_t *total = ctx->h_enc_total.get();
+    CK(ctx, cudaMemcpyAsync(ctx->h_enc_total.get(), ctx->d_enc_total.get(), 2 * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
     CK(ctx, cudaStreamSynchronize(st));
-    if (bytes) *bytes = ctx->h_enc_total[0];
-    if (overflow) *overflow = ctx->h_enc_total[1] != 0;
+    if (bytes) *bytes = total[0];
+    if (overflow) *overflow = total[1] != 0;
     return RTJGPU_OK;
 }
 
@@ -1030,7 +931,7 @@ struct rtjgpu_seqenc {
     int         quality = 0, key_rate = 0, key_count = 0, lm = 0, cm = 0;
     bool        cleared = true;             /* the stored blocks are zeros: a run that starts here does not read them */
     int         w = 0, h = 0, fmt = -1;     /* geometry of the stored blocks */
-    int16_t    *d_old = nullptr;  size_t old_cap = 0;    /* [nblk][64], allocated at the first inter call */
+    Buf<int16_t> d_old;                     /* [nblk][64], allocated at the first inter call */
     uint64_t    call = 0;                   /* rtjgpu_ctx::enc_seq_calls of the last call that named it */
 };
 
@@ -1038,15 +939,13 @@ int rtjgpu_seqenc_create(rtjgpu_ctx *ctx, rtjgpu_seqenc **out)
 {
     if (!ctx || !out) return RTJGPU_E_ARG;
     *out = nullptr;
-    if (!ctx->d_enc_qt_all) {
+    if (!ctx->d_enc_qt_all.get()) {
         CK(ctx, cudaSetDevice(ctx->device));
         std::vector<int32_t> qt(256 * 128, 0);
         for (int q = 1; q <= 255; q++) rtj_encoder_table_from_quality(q, &qt[(size_t)q * 128], &ctx->enc_lb8_all[q], &ctx->enc_cb8_all[q]);
-        int32_t *d = nullptr;
-        CK(ctx, cudaMalloc(&d, qt.size() * sizeof(int32_t)));
-        const cudaError_t e = cudaMemcpy(d, qt.data(), qt.size() * sizeof(int32_t), cudaMemcpyHostToDevice);
-        if (e != cudaSuccess) { cudaFree(d); ctx->last_cuda = (int)e; return RTJGPU_E_CUDA; }
-        ctx->d_enc_qt_all = d;
+        CK(ctx, ctx->d_enc_qt_all.reserve(qt.size()));
+        const cudaError_t e = cudaMemcpy(ctx->d_enc_qt_all.get(), qt.data(), qt.size() * sizeof(int32_t), cudaMemcpyHostToDevice);
+        if (e != cudaSuccess) { ctx->d_enc_qt_all.release(); ctx->last_cuda = (int)e; return RTJGPU_E_CUDA; }
     }
     rtjgpu_seqenc *e = new (std::nothrow) rtjgpu_seqenc();
     if (!e) return RTJGPU_E_NOMEM;
@@ -1059,10 +958,7 @@ int rtjgpu_seqenc_create(rtjgpu_ctx *ctx, rtjgpu_seqenc **out)
 void rtjgpu_seqenc_destroy(rtjgpu_seqenc *e)
 {
     if (!e) return;
-    if (e->d_old) {
-        cudaSetDevice(e->device);
-        cudaFree(e->d_old);                 /* waits for the work that may still read or write it */
-    }
+    if (e->d_old.get()) cudaSetDevice(e->device);  /* freeing d_old waits for the work that may still read or write it */
     delete e;
 }
 
@@ -1095,9 +991,7 @@ int rtjgpu_seqenc_key_count(const rtjgpu_seqenc *e) { return e ? e->key_count : 
 
 size_t rtjgpu_encode_bound(int format, int w, int h, int F)
 {
-    if ((format != RTJ_YUV420 && format != RTJ_YUV422) || w <= 0 || h <= 0 || (w & 15) || (h & 15) || w > 65535 || h > 65535
-        || F < 0)
-        return 0;
+    if ((format != RTJ_YUV420 && format != RTJ_YUV422) || !valid_size(w, h) || F < 0) return 0;
     /* a block takes at most 64 bytes (DC byte and one byte per place, RTjpeg_b2s :109-155); header and block bytes are a
      * multiple of 4 already, so no packet needs padding */
     return (size_t)F * (RTJPEG_B200_HEADER_BYTES + 64 * (size_t)RTJ_FMT_NBLK(format, w, h));
@@ -1109,7 +1003,7 @@ int rtjgpu_encode_device_seq(rtjgpu_ctx *ctx, int F, int w, int h, int S, const 
 {
     if (!ctx) return RTJGPU_E_ARG;
     if (ctx->format != RTJ_YUV420 && ctx->format != RTJ_YUV422) return RTJGPU_E_FORMAT;
-    if (w <= 0 || h <= 0 || (w & 15) || (h & 15) || w > 65535 || h > 65535) return RTJGPU_E_SIZE;
+    if (!valid_size(w, h)) return RTJGPU_E_SIZE;
     if (F > RTJGPU_MAX_FRAMES_PER_BATCH) return RTJGPU_E_TOOBIG;
     SeqIn q;
     q.S = S; q.first = seq_first;
@@ -1129,11 +1023,8 @@ int rtjgpu_encode_device_seq(rtjgpu_ctx *ctx, int F, int w, int h, int S, const 
     for (int s = 0; s < S; s++) {
         rtjgpu_seqenc *e = encs[s];
         if (e->w != w || e->h != h || e->fmt != ctx->format) { e->w = w; e->h = h; e->fmt = ctx->format; e->cleared = true; }
-        if (e->key_rate && e->old_cap < nblk * 64) {
-            if (e->d_old) cudaFree(e->d_old);
-            e->d_old = nullptr; e->old_cap = 0;
-            CK(ctx, cudaMalloc(&e->d_old, nblk * 64 * sizeof(int16_t)));
-            e->old_cap = nblk * 64;
+        if (e->key_rate && e->d_old.cap() < nblk * 64) {
+            CK(ctx, e->d_old.reserve(nblk * 64));
             e->cleared = true;
         }
     }
@@ -1158,7 +1049,7 @@ int rtjgpu_encode_device_seq(rtjgpu_ctx *ctx, int F, int w, int h, int S, const 
         const rtjgpu_seqenc *e = encs[s];
         const int a = seq_first[s], b = seq_first[s + 1];
         rtj_enc_seq &r = hs[s];
-        r.d_frames = frames[s]; r.d_old = e->d_old; r.first = a; r.quality = e->quality;
+        r.d_frames = frames[s]; r.d_old = e->d_old.get(); r.first = a; r.quality = e->quality;
         r.lb8 = ctx->enc_lb8_all[e->quality]; r.cb8 = ctx->enc_cb8_all[e->quality]; r.lmask = e->lm; r.cmask = e->cm;
         if (!e->key_rate) {
             for (int f = a; f < b; f++) {
@@ -1182,19 +1073,20 @@ int rtjgpu_encode_device_seq(rtjgpu_ctx *ctx, int F, int w, int h, int S, const 
     const size_t runs_bytes = runs.size() * sizeof(rtj_enc_run);
     const size_t bytes = seqs_bytes + words_bytes + runs_bytes;
     memcpy(hb + seqs_bytes + words_bytes, runs.data(), runs_bytes);
-    if ((rc = grow_device(ctx, &ctx->d_enc_seq, &ctx->enc_seq_cap, bytes))) return rc;
-    if ((rc = stage_end(ctx, ctx->d_enc_seq, bytes, st))) return rc;
+    CK(ctx, ctx->d_enc_seq.reserve(bytes));
+    const uint8_t *d = ctx->d_enc_seq.get();
+    if ((rc = stage_end(ctx, ctx->d_enc_seq.get(), bytes, st))) return rc;
 
     rtj_encode_args a;
     memset(&a, 0, sizeof(a));
-    a.F = F; a.w = w; a.h = h; a.fmt = ctx->format; a.d_qt = ctx->d_enc_qt_all;
-    a.d_slots = ctx->d_enc_slots; a.d_lens = ctx->d_enc_lens; a.d_boff = ctx->d_enc_boff;
-    a.d_fsize = ctx->d_enc_fsize; a.d_stream = d_stream; a.capacity = capacity; a.d_offsets = d_offsets;
-    a.d_total = ctx->d_enc_total;
+    a.F = F; a.w = w; a.h = h; a.fmt = ctx->format; a.d_qt = ctx->d_enc_qt_all.get();
+    a.d_slots = ctx->d_enc_slots.get(); a.d_lens = ctx->d_enc_lens.get(); a.d_boff = ctx->d_enc_boff.get();
+    a.d_fsize = ctx->d_enc_fsize.get(); a.d_stream = d_stream; a.capacity = capacity; a.d_offsets = d_offsets;
+    a.d_total = ctx->d_enc_total.get();
     ctx->enc_stream = cuda_stream;
-    const int n = rtj_launch_encode_seq(&a, reinterpret_cast<const rtj_enc_run *>(ctx->d_enc_seq + seqs_bytes + words_bytes),
-                                        n_intra, (int)runs.size() - n_intra, reinterpret_cast<const rtj_enc_seq *>(ctx->d_enc_seq),
-                                        reinterpret_cast<const uint32_t *>(ctx->d_enc_seq + seqs_bytes), cuda_stream);
+    const int n = rtj_launch_encode_seq(&a, reinterpret_cast<const rtj_enc_run *>(d + seqs_bytes + words_bytes),
+                                        n_intra, (int)runs.size() - n_intra, reinterpret_cast<const rtj_enc_seq *>(d),
+                                        reinterpret_cast<const uint32_t *>(d + seqs_bytes), cuda_stream);
     if (n < 0) { ctx->last_cuda = -n; return RTJGPU_E_CUDA; }
     ctx->launches += (uint64_t)n;
     /* the handles move on as RTjpeg_compress would have, whether the packets fit or not */
@@ -1220,7 +1112,7 @@ int rtjgpu_convert_device(rtjgpu_ctx *ctx, int kind, const uint8_t *d_frames, si
     if (!bpp) return RTJGPU_E_FORMAT;
     if (F == 0) return RTJGPU_OK;
     if (!d_frames || !d_out) return RTJGPU_E_ARG;
-    if (w <= 0 || h <= 0 || (w & 15) || (h & 15) || w > 65535 || h > 65535) return RTJGPU_E_SIZE;
+    if (!valid_size(w, h)) return RTJGPU_E_SIZE;
     if (F > 65535) return RTJGPU_E_TOOBIG;                                   /* frames are the grid's second dimension */
     if ((row_pitch & 15) || row_pitch < (size_t)w * bpp || frame_pitch < row_pitch * (size_t)h
         || ((uintptr_t)d_out & 15) || ((uintptr_t)d_frames & 7) || (src_frame_bytes & 7) || (frame_pitch & 15))
@@ -1251,7 +1143,7 @@ int rtjgpu_set_custom_tables(rtjgpu_ctx *ctx, const uint32_t raw[128])
     }
     if (ctx->pipe.ready) { CK(ctx, cudaStreamSynchronize(ctx->pipe.scan)); CK(ctx, cudaStreamSynchronize(ctx->pipe.idct)); }
     if (ctx->slots_ready) for (int i = 0; i < HOST_SLOTS; i++) CK(ctx, cudaStreamSynchronize(ctx->slot[i].stream));
-    CK(ctx, cudaMemcpy(ctx->d_tables + RTJGPU_TABLE_CUSTOM, &dev, sizeof(dev), cudaMemcpyHostToDevice));
+    CK(ctx, cudaMemcpy(ctx->d_tables.get() + RTJGPU_TABLE_CUSTOM, &dev, sizeof(dev), cudaMemcpyHostToDevice));
     return RTJGPU_OK;
 }
 
@@ -1294,7 +1186,7 @@ int rtjgpu_plan_n(const uint8_t *stream, const uint64_t *offsets, const uint32_t
         if (!lengths && framesize >= RTJPEG_B200_HEADER_BYTES && framesize < len) len = framesize;
         if (len - RTJPEG_B200_HEADER_BYTES > RTJGPU_MAX_PAYLOAD_BYTES) return RTJGPU_E_TOOBIG;
         if (w != st.width || h != st.height) { st.width = w; st.height = h; }   /* :3568-3574 */
-        if (w == 0 || h == 0 || (w & 15) || (h & 15)) return RTJGPU_E_SIZE;     /* the row loop of :2701 needs /16 */
+        if (!valid_size(w, h)) return RTJGPU_E_SIZE;                             /* the row loop of :2701 needs /16 */
         if (f == 0) { bw = w; bh = h; }
         else if (w != bw || h != bh) return RTJGPU_E_SIZE;
         if (q != st.quality) {                                                   /* :3575-3579 */
@@ -1314,49 +1206,56 @@ int rtjgpu_plan_n(const uint8_t *stream, const uint64_t *offsets, const uint32_t
 int rtjgpu_decode_device(rtjgpu_ctx *ctx, const uint8_t *d_stream, const rtjgpu_frame_desc *d_desc, int F,
                          int w, int h, uint8_t *d_out, const uint8_t *d_carry, void *cuda_stream)
 {
-    SeqIn q;
-    q.carries = &d_carry;
-    return decode_device(ctx, d_stream, d_desc, F, w, h, q, d_out, cuda_stream);
+    DecodeCall c(d_stream, d_desc, F, w, h, cuda_stream);
+    c.q.carries = &d_carry;
+    c.d_out = d_out;
+    return decode(ctx, c);
 }
 
 int rtjgpu_decode_device_seq(rtjgpu_ctx *ctx, const uint8_t *d_stream, const rtjgpu_frame_desc *d_desc, int F, int w, int h,
                              int S, const int *seq_first, uint8_t *d_out, const uint8_t *const *carries, void *cuda_stream)
 {
-    SeqIn q;
-    q.S = S; q.first = seq_first; q.carries = carries;
     if (!seq_first) return RTJGPU_E_ARG;
-    return decode_device(ctx, d_stream, d_desc, F, w, h, q, d_out, cuda_stream);
+    DecodeCall c(d_stream, d_desc, F, w, h, cuda_stream);
+    c.q.S = S; c.q.first = seq_first; c.q.carries = carries;
+    c.d_out = d_out;
+    return decode(ctx, c);
 }
 
 int rtjgpu_decode_device_rgb(rtjgpu_ctx *ctx, const uint8_t *d_stream, const rtjgpu_frame_desc *d_desc, int F,
                              int w, int h, int kind, uint8_t *d_rgb, size_t row_pitch, size_t frame_pitch, int alpha,
                              const uint8_t *d_carry, uint8_t *d_last_yuv, void *cuda_stream)
 {
-    SeqIn q;
-    q.carries = &d_carry; q.last_yuv = &d_last_yuv;
-    return decode_device_rgb(ctx, d_stream, d_desc, F, w, h, q, kind, d_rgb, row_pitch, frame_pitch, alpha, cuda_stream);
+    const RgbOut o{d_rgb, row_pitch, frame_pitch, kind, alpha};
+    DecodeCall c(d_stream, d_desc, F, w, h, cuda_stream);
+    c.q.carries = &d_carry; c.q.last_yuv = &d_last_yuv;
+    c.rgb = &o;
+    return decode(ctx, c);
 }
 
 int rtjgpu_decode_device_rgb_seq(rtjgpu_ctx *ctx, const uint8_t *d_stream, const rtjgpu_frame_desc *d_desc, int F, int w, int h,
                                  int S, const int *seq_first, int kind, uint8_t *d_rgb, size_t row_pitch, size_t frame_pitch,
                                  int alpha, const uint8_t *const *carries, uint8_t *const *last_yuv, void *cuda_stream)
 {
-    SeqIn q;
-    q.S = S; q.first = seq_first; q.carries = carries; q.last_yuv = last_yuv;
     if (!seq_first) return RTJGPU_E_ARG;
-    return decode_device_rgb(ctx, d_stream, d_desc, F, w, h, q, kind, d_rgb, row_pitch, frame_pitch, alpha, cuda_stream);
+    const RgbOut o{d_rgb, row_pitch, frame_pitch, kind, alpha};
+    DecodeCall c(d_stream, d_desc, F, w, h, cuda_stream);
+    c.q.S = S; c.q.first = seq_first; c.q.carries = carries; c.q.last_yuv = last_yuv;
+    c.rgb = &o;
+    return decode(ctx, c);
 }
 
 int rtjgpu_decode_device_select(rtjgpu_ctx *ctx, const uint8_t *d_stream, const rtjgpu_frame_desc *d_desc, int F, int w, int h,
                                 int S, const int *seq_first, const uint8_t *const *carries,
                                 int n, const int *sel, uint8_t *d_out, void *cuda_stream)
 {
-    SeqIn q;
-    q.S = S; q.first = seq_first; q.carries = carries;
-    SelIn s;
-    s.n = n; s.idx = sel;
     if (!seq_first) return RTJGPU_E_ARG;
-    return decode_device(ctx, d_stream, d_desc, F, w, h, q, d_out, cuda_stream, &s);
+    const SelIn s{n, sel};
+    DecodeCall c(d_stream, d_desc, F, w, h, cuda_stream);
+    c.q.S = S; c.q.first = seq_first; c.q.carries = carries;
+    c.sel = &s;
+    c.d_out = d_out;
+    return decode(ctx, c);
 }
 
 int rtjgpu_decode_device_rgb_select(rtjgpu_ctx *ctx, const uint8_t *d_stream, const rtjgpu_frame_desc *d_desc, int F, int w, int h,
@@ -1364,12 +1263,14 @@ int rtjgpu_decode_device_rgb_select(rtjgpu_ctx *ctx, const uint8_t *d_stream, co
                                     int n, const int *sel, int kind, uint8_t *d_rgb, size_t row_pitch, size_t frame_pitch,
                                     int alpha, uint8_t *const *last_yuv, void *cuda_stream)
 {
-    SeqIn q;
-    q.S = S; q.first = seq_first; q.carries = carries; q.last_yuv = last_yuv;
-    SelIn s;
-    s.n = n; s.idx = sel;
     if (!seq_first) return RTJGPU_E_ARG;
-    return decode_device_rgb(ctx, d_stream, d_desc, F, w, h, q, kind, d_rgb, row_pitch, frame_pitch, alpha, cuda_stream, &s);
+    const SelIn s{n, sel};
+    const RgbOut o{d_rgb, row_pitch, frame_pitch, kind, alpha};
+    DecodeCall c(d_stream, d_desc, F, w, h, cuda_stream);
+    c.q.S = S; c.q.first = seq_first; c.q.carries = carries; c.q.last_yuv = last_yuv;
+    c.sel = &s;
+    c.rgb = &o;
+    return decode(ctx, c);
 }
 
 int rtjgpu_sync(rtjgpu_ctx *ctx)
@@ -1407,14 +1308,15 @@ int rtjgpu_get_batch_info(rtjgpu_ctx *ctx, rtjgpu_batch_info *out)
     if (!ctx || !out) return RTJGPU_E_ARG;
     memset(out, 0, sizeof(*out));
     out->first_bad_frame = -1;
-    if (ctx->last_F == 0 || !ctx->ws.d_info) return RTJGPU_OK;
+    if (ctx->last_F == 0 || !ctx->ws.d_info.get()) return RTJGPU_OK;
     CK(ctx, cudaSetDevice(ctx->device));
     CK(ctx, cudaDeviceSynchronize());
-    CK(ctx, cudaMemcpy(ctx->h_info, ctx->ws.d_info, sizeof(rtj_dev_info), cudaMemcpyDeviceToHost));
-    out->skipped_blocks = ctx->h_info->skipped_blocks;
-    out->payload_bytes = ctx->h_info->payload_bytes;
-    out->bad_frames = ctx->h_info->bad_frames;
-    out->first_bad_frame = ctx->h_info->first_bad_frame;
+    const rtj_dev_info *info = ctx->h_info.get();
+    CK(ctx, cudaMemcpy(ctx->h_info.get(), ctx->ws.d_info.get(), sizeof(rtj_dev_info), cudaMemcpyDeviceToHost));
+    out->skipped_blocks = info->skipped_blocks;
+    out->payload_bytes = info->payload_bytes;
+    out->bad_frames = info->bad_frames;
+    out->first_bad_frame = info->first_bad_frame;
     return RTJGPU_OK;
 }
 
@@ -1424,16 +1326,16 @@ int rtjgpu_get_skip_counts(rtjgpu_ctx *ctx, uint32_t *counts, int F)
     if (F == 0) return RTJGPU_OK;
     CK(ctx, cudaSetDevice(ctx->device));
     CK(ctx, cudaDeviceSynchronize());
-    CK(ctx, cudaMemcpy(counts, ctx->ws.d_frame_skips, (size_t)F * sizeof(uint32_t), cudaMemcpyDeviceToHost));
+    CK(ctx, cudaMemcpy(counts, ctx->ws.frame_skips(), (size_t)F * sizeof(uint32_t), cudaMemcpyDeviceToHost));
     return RTJGPU_OK;
 }
 
 int rtjgpu_get_entries(rtjgpu_ctx *ctx, uint32_t *entries, size_t n)
 {
-    if (!ctx || !entries || n > ctx->ws.cap_entries) return RTJGPU_E_ARG;
+    if (!ctx || !entries || n > ctx->ws.d_ent.cap()) return RTJGPU_E_ARG;
     CK(ctx, cudaSetDevice(ctx->device));
     CK(ctx, cudaDeviceSynchronize());
-    CK(ctx, cudaMemcpy(entries, ctx->ws.d_ent, n * sizeof(uint32_t), cudaMemcpyDeviceToHost));
+    CK(ctx, cudaMemcpy(entries, ctx->ws.d_ent.get(), n * sizeof(uint32_t), cudaMemcpyDeviceToHost));
     return RTJGPU_OK;
 }
 
@@ -1496,29 +1398,14 @@ int rtjgpu_scan_device(rtjgpu_ctx *ctx, const uint8_t *d_stream, const rtjgpu_fr
 {
     if (!ctx || F < 0) return RTJGPU_E_ARG;
     if (F == 0) { ctx->last_F = 0; return RTJGPU_OK; }
-    if (!d_stream || !d_desc || ((uintptr_t)d_stream & 3)) return RTJGPU_E_ARG;
-    if (w <= 0 || h <= 0 || (w & 15) || (h & 15) || w > 65535 || h > 65535) return RTJGPU_E_SIZE;
-    if (F > RTJGPU_MAX_FRAMES_PER_BATCH) return RTJGPU_E_TOOBIG;
-    CK(ctx, cudaSetDevice(ctx->device));
-    const int nblk = RTJ_FMT_NBLK(ctx->format, w, h);
-    if ((uint64_t)F * (uint64_t)nblk >= (1ull << 32)) return RTJGPU_E_TOOBIG;
-    int rc = ws_reserve(ctx, &ctx->ws, F, nblk);
-    if (rc) return rc;
-    cudaStream_t st = (cudaStream_t)cuda_stream;
-    rtj_launch_args a;
-    memset(&a, 0, sizeof(a));
-    a.d_stream = d_stream; a.d_desc = d_desc; a.d_tables = ctx->d_tables;
-    a.F = F; a.w = w; a.h = h; a.f0 = 0; a.f1 = F; a.slice = 0;
-    a.fmt = ctx->format;
-    a.d_ent = ctx->ws.d_ent; a.d_frame_skips = ctx->ws.d_frame_skips; a.d_info = ctx->ws.d_info;
-    a.d_walk = ctx->ws.d_walk;
-    a.d_redo = ctx->ws.d_frame_skips + ctx->ws.cap_frames;
-    a.raw_expected = ((volatile unsigned long long *)ctx->h_skips_seen)[1] != 0;
-    a.row1 = RTJ_FMT_UNITS_Y(ctx->format, h);
-    a.scan_mode = ctx->scan_mode;
+    const DecodeCall c(d_stream, d_desc, F, w, h, cuda_stream);
+    int nblk, rc;
+    if ((rc = check_batch(ctx, c, false, &nblk))) return rc;
+    if ((rc = ws_reserve(ctx, &ctx->ws, F, nblk))) return rc;
+    rtj_launch_args a = k1_args(ctx, ctx->ws, c);
     if ((rc = seg_reserve(ctx, &ctx->ws, F, nblk, ctx->scan_mode, &a.seg))) return rc;
-    CK(ctx, cudaMemcpyAsync(ctx->ws.d_info, ctx->h_info_reset, sizeof(rtj_dev_info), cudaMemcpyHostToDevice, st));
-    const int e = rtj_launch_scan(&a, st);
+    CK(ctx, cudaMemcpyAsync(ctx->ws.d_info.get(), ctx->h_info_reset.get(), sizeof(rtj_dev_info), cudaMemcpyHostToDevice, c.stream));
+    const int e = rtj_launch_scan(&a, c.stream);
     if (e < 0) { ctx->last_cuda = -e; return RTJGPU_E_CUDA; }
     ctx->launches += (uint64_t)e;
     ctx->last_F = F;
@@ -1569,7 +1456,7 @@ static int slots_init(rtjgpu_ctx *ctx)
     for (int i = 0; i < HOST_SLOTS; i++) {
         CK(ctx, cudaStreamCreateWithFlags(&ctx->slot[i].stream, cudaStreamNonBlocking));
         CK(ctx, cudaEventCreateWithFlags(&ctx->slot[i].decoded, cudaEventDisableTiming));
-        CK(ctx, cudaMallocHost(&ctx->slot[i].h_info, sizeof(rtj_dev_info)));
+        CK(ctx, ctx->slot[i].h_info.reserve(1));
     }
     ctx->slots_ready = true;
     return RTJGPU_OK;
@@ -1580,8 +1467,8 @@ static int slot_drain(rtjgpu_ctx *ctx, HostSlot &s)
     if (!s.busy) return RTJGPU_OK;
     const cudaError_t e = cudaStreamSynchronize(s.stream);
     if (e == cudaSuccess) {
-        ctx->host_bad += s.h_info->bad_frames;
-        if (s.pending_dst) memcpy(s.pending_dst, s.h_out, s.pending_bytes);
+        ctx->host_bad += s.h_info.get()->bad_frames;
+        if (s.pending_dst) memcpy(s.pending_dst, s.h_out.get(), s.pending_bytes);
     }
     s.pending_dst = nullptr;              /* whatever happened: never again touch the memory of the call that queued this */
     s.pending_bytes = 0;
@@ -1609,7 +1496,7 @@ int rtjgpu_decode_host_n(rtjgpu_ctx *ctx, const uint8_t *h_stream, const uint64_
     /* geometry from the first header; rtjgpu_plan re-checks every frame */
     if ((lengths ? (uint64_t)lengths[0] : offsets[1] - offsets[0]) < RTJPEG_B200_HEADER_BYTES) return RTJGPU_E_HEADER;
     const int w = rd_u16le(h_stream + offsets[0] + 6), h = rd_u16le(h_stream + offsets[0] + 8);
-    if (w == 0 || h == 0 || (w & 15) || (h & 15)) return RTJGPU_E_SIZE;
+    if (!valid_size(w, h)) return RTJGPU_E_SIZE;
     const size_t fsz = RTJ_FMT_FRAME_BYTES(ctx->format, w, h);
     const int nblk = RTJ_FMT_NBLK(ctx->format, w, h);
 
@@ -1619,15 +1506,14 @@ int rtjgpu_decode_host_n(rtjgpu_ctx *ctx, const uint8_t *h_stream, const uint64_
     chunk = std::min(chunk, RTJGPU_MAX_FRAMES_PER_BATCH);
     chunk = std::min(chunk, F);
 
-    rc = grow_device(ctx, &ctx->d_host_carry, &ctx->d_host_carry_cap, fsz);
-    if (rc) return rc;
-    if ((rc = grow_pinned(ctx, &ctx->h_host_skips, &ctx->host_skips_cap, (size_t)F))) return rc;
+    CK(ctx, ctx->d_host_carry.reserve(fsz));
+    CK(ctx, ctx->h_host_skips.reserve((size_t)F));
     ctx->host_F = 0;
     const bool have_carry = h_carry_inout != nullptr;
     if (have_carry)
-        CK(ctx, cudaMemcpy(ctx->d_host_carry, h_carry_inout, fsz, cudaMemcpyHostToDevice));
+        CK(ctx, cudaMemcpy(ctx->d_host_carry.get(), h_carry_inout, fsz, cudaMemcpyHostToDevice));
 
-    const uint8_t *d_prev = have_carry ? ctx->d_host_carry : nullptr;
+    const uint8_t *d_prev = have_carry ? ctx->d_host_carry.get() : nullptr;
     cudaEvent_t prev_decoded = nullptr;
     rtjgpu_state st = *state;
     int result = RTJGPU_OK;
@@ -1645,46 +1531,45 @@ int rtjgpu_decode_host_n(rtjgpu_ctx *ctx, const uint8_t *h_stream, const uint64_
 
         const uint64_t b0 = offsets[c0], b1 = offsets[c0 + n];
         const size_t in_bytes = (size_t)(b1 - b0);
-        if ((rc = grow_device(ctx, &s.d_in, &s.d_in_cap, in_bytes + RTJGPU_STREAM_SLACK_BYTES))) { result = rc; break; }
-        if ((rc = grow_device(ctx, &s.d_out, &s.d_out_cap, fsz * (size_t)n))) { result = rc; break; }
-        size_t dcap = (size_t)s.desc_cap;
-        if ((rc = grow_device(ctx, &s.d_desc, &dcap, (size_t)n))) { result = rc; break; }
-        s.desc_cap = (int)dcap;
-        size_t hcap = (size_t)s.h_desc_cap;
-        if ((rc = grow_pinned(ctx, &s.h_desc, &hcap, (size_t)n))) { result = rc; break; }
-        s.h_desc_cap = (int)hcap;
+        CKB(s.d_in.reserve(in_bytes + RTJGPU_STREAM_SLACK_BYTES));
+        CKB(s.d_out.reserve(fsz * (size_t)n));
+        CKB(s.d_desc.reserve((size_t)n));
+        CKB(s.h_desc.reserve((size_t)n));
         if ((rc = ws_reserve(ctx, &s.ws, n, nblk))) { result = rc; break; }
 
         /* descriptors relative to the chunk's own device buffer */
         rel.resize((size_t)n + 1);
         for (int i = 0; i <= n; i++) rel[(size_t)i] = offsets[c0 + i] - b0;
-        if ((rc = rtjgpu_plan_n(h_stream + b0, rel.data(), lengths ? lengths + c0 : nullptr, n, &st, s.h_desc))) { result = rc; break; }
+        if ((rc = rtjgpu_plan_n(h_stream + b0, rel.data(), lengths ? lengths + c0 : nullptr, n, &st, s.h_desc.get()))) { result = rc; break; }
         if (st.width != w || st.height != h) { result = RTJGPU_E_SIZE; break; }
 
         const uint8_t *src = h_stream + b0;
         if (!(flags & RTJGPU_HOST_IN_PINNED)) {
-            if ((rc = grow_pinned(ctx, &s.h_in, &s.h_in_cap, in_bytes))) { result = rc; break; }
-            memcpy(s.h_in, src, in_bytes);
-            src = s.h_in;
+            CKB(s.h_in.reserve(in_bytes));
+            memcpy(s.h_in.get(), src, in_bytes);
+            src = s.h_in.get();
         }
-        CKB(cudaMemcpyAsync(s.d_in, src, in_bytes, cudaMemcpyHostToDevice, s.stream));
-        CKB(cudaMemsetAsync(s.d_in + in_bytes, 0x7F, RTJGPU_STREAM_SLACK_BYTES, s.stream));
-        CKB(cudaMemcpyAsync(s.d_desc, s.h_desc, sizeof(rtjgpu_frame_desc) * (size_t)n, cudaMemcpyHostToDevice, s.stream));
+        CKB(cudaMemcpyAsync(s.d_in.get(), src, in_bytes, cudaMemcpyHostToDevice, s.stream));
+        CKB(cudaMemsetAsync(s.d_in.get() + in_bytes, 0x7F, RTJGPU_STREAM_SLACK_BYTES, s.stream));
+        CKB(cudaMemcpyAsync(s.d_desc.get(), s.h_desc.get(), sizeof(rtjgpu_frame_desc) * (size_t)n, cudaMemcpyHostToDevice, s.stream));
         if (prev_decoded) CKB(cudaStreamWaitEvent(s.stream, prev_decoded, 0));   /* carry comes from the previous chunk */
-        if ((rc = run_kernels(ctx, &s.ws, s.d_in, s.d_desc, n, w, h, s.d_out, d_prev, s.stream, nullptr, false))) { result = rc; break; }
+        DecodeCall c(s.d_in.get(), s.d_desc.get(), n, w, h, s.stream);
+        c.q.carries = &d_prev;
+        c.d_out = s.d_out.get();
+        if ((rc = run_kernels(ctx, &s.ws, c, CallDev(), nullptr, false))) { result = rc; break; }
         CKB(cudaEventRecord(s.decoded, s.stream));
-        CKB(cudaMemcpyAsync(s.h_info, s.ws.d_info, sizeof(rtj_dev_info), cudaMemcpyDeviceToHost, s.stream));
-        CKB(cudaMemcpyAsync(ctx->h_host_skips + c0, s.ws.d_frame_skips, sizeof(uint32_t) * (size_t)n, cudaMemcpyDeviceToHost, s.stream));
+        CKB(cudaMemcpyAsync(s.h_info.get(), s.ws.d_info.get(), sizeof(rtj_dev_info), cudaMemcpyDeviceToHost, s.stream));
+        CKB(cudaMemcpyAsync(ctx->h_host_skips.get() + c0, s.ws.frame_skips(), sizeof(uint32_t) * (size_t)n, cudaMemcpyDeviceToHost, s.stream));
         prev_decoded = s.decoded;
-        d_prev = s.d_out + fsz * (size_t)(n - 1);
+        d_prev = s.d_out.get() + fsz * (size_t)(n - 1);
 
         uint8_t *dst = h_out + fsz * (size_t)c0;
         if (flags & RTJGPU_HOST_OUT_PINNED) {
-            CKB(cudaMemcpyAsync(dst, s.d_out, fsz * (size_t)n, cudaMemcpyDeviceToHost, s.stream));
+            CKB(cudaMemcpyAsync(dst, s.d_out.get(), fsz * (size_t)n, cudaMemcpyDeviceToHost, s.stream));
             s.pending_dst = nullptr;
         } else {
-            if ((rc = grow_pinned(ctx, &s.h_out, &s.h_out_cap, fsz * (size_t)n))) { result = rc; break; }
-            CKB(cudaMemcpyAsync(s.h_out, s.d_out, fsz * (size_t)n, cudaMemcpyDeviceToHost, s.stream));
+            CKB(s.h_out.reserve(fsz * (size_t)n));
+            CKB(cudaMemcpyAsync(s.h_out.get(), s.d_out.get(), fsz * (size_t)n, cudaMemcpyDeviceToHost, s.stream));
             s.pending_dst = dst;
             s.pending_bytes = fsz * (size_t)n;
         }
@@ -1708,7 +1593,7 @@ int rtjgpu_decode_host_n(rtjgpu_ctx *ctx, const uint8_t *h_stream, const uint64_
 int rtjgpu_get_host_skip_counts(rtjgpu_ctx *ctx, uint32_t *counts, int F)
 {
     if (!ctx || !counts || F < 0 || F > ctx->host_F) return RTJGPU_E_ARG;
-    if (F) memcpy(counts, ctx->h_host_skips, sizeof(uint32_t) * (size_t)F);
+    if (F) memcpy(counts, ctx->h_host_skips.get(), sizeof(uint32_t) * (size_t)F);
     return RTJGPU_OK;
 }
 

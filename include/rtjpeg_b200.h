@@ -331,7 +331,8 @@ int  rtjgpu_plan_n(const uint8_t *stream, const uint64_t *offsets, const uint32_
  * one persistent frame).  cuda_stream is a cudaStream_t passed as void*
  * (NULL = the legacy default stream).  Asynchronous: returns after the launches.
  * Alignment (RTJGPU_E_ARG otherwise): d_stream 4 bytes -- and every packet offset a multiple of 4, which rtjgpu_plan
- * checks --, d_desc 8, d_out 16 (frames are w*h*3/2 bytes, a multiple of 16, apart), d_carry 8. */
+ * checks --, d_desc 8, d_out 16 (frames are w*h*3/2 bytes, a multiple of 16, apart), d_carry 8.  Every
+ * rtjgpu_decode_device* call, the _rgb ones included, and rtjgpu_scan_device (d_stream and d_desc) check the same. */
 int  rtjgpu_decode_device(rtjgpu_ctx *ctx, const uint8_t *d_stream,
                           const rtjgpu_frame_desc *d_desc, int F, int w, int h,
                           uint8_t *d_out, const uint8_t *d_carry, void *cuda_stream);
