@@ -156,6 +156,13 @@ def load_library() -> C.CDLL:
     L.rtjgpu_decode_device_rgb_select.argtypes = [vp, vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_int),
                                                   C.POINTER(vp), C.c_int, C.POINTER(C.c_int), C.c_int, vp, C.c_size_t,
                                                   C.c_size_t, C.c_int, C.POINTER(vp), vp]
+    L.rtjgpu_decode_device_window.argtypes = [vp, vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_int), C.POINTER(vp),
+                                              C.c_int, C.POINTER(C.c_int), C.c_int, C.c_int, C.POINTER(C.c_int), vp,
+                                              C.POINTER(vp), vp]
+    L.rtjgpu_decode_device_rgb_window.argtypes = [vp, vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_int),
+                                                  C.POINTER(vp), C.c_int, C.POINTER(C.c_int), C.c_int, C.c_int,
+                                                  C.POINTER(C.c_int), C.c_int, vp, C.c_size_t, C.c_size_t, C.c_int,
+                                                  C.POINTER(vp), vp]
     L.rtjgpu_decode_host.argtypes = [vp, _u8p, _u64p, C.c_int, C.POINTER(State), _u8p, _u8p, C.c_int]
     L.rtjgpu_sync.argtypes = [vp]
     L.rtjgpu_enable_timing.argtypes = [vp, C.c_int]
@@ -213,6 +220,13 @@ def _ptr_array(v):
     if v is None:
         return None
     return (C.c_void_p * max(len(v), 1))(*[int(x) if x else None for x in v])
+
+
+def _origins_array(origins):
+    """[(x, y), ...] -> the host array of 2 S ints the window calls take, or NULL for None."""
+    if origins is None:
+        return None
+    return _int_array([int(v) for xy in origins for v in xy])
 
 
 def _check(rc: int, what: str) -> None:
@@ -530,6 +544,33 @@ class BatchContext:
                                                        kind, C.c_void_p(d_rgb or 0), row_pitch, frame_pitch, alpha,
                                                        _ptr_array(last_yuv), C.c_void_p(cuda_stream or 0)),
                "rtjgpu_decode_device_rgb_select")
+
+    def decode_device_window(self, d_stream: int, d_desc: int, F: int, w: int, h: int, seq_first, sel, size, origins,
+                             d_out: int, carries=None, last_yuv=None, cuda_stream: int | None = None) -> None:
+        """rtjgpu_decode_device_window: the selection of decode_device_select, only a window of size (cw, ch) of each frame,
+        at origins[s] = (x, y) of its sequence, frame sel[k] to d_out + k * window_bytes as tight planes.  last_yuv: a list
+        of S device addresses (None = not wanted) or None, receiving each sequence's last frame whole."""
+        S = len(seq_first) - 1
+        cw, ch = size
+        _check(self._L.rtjgpu_decode_device_window(self._h, C.c_void_p(d_stream), C.c_void_p(d_desc), F, w, h, S,
+                                                   _int_array(seq_first), _ptr_array(carries), len(sel), _int_array(sel),
+                                                   cw, ch, _origins_array(origins), C.c_void_p(d_out or 0),
+                                                   _ptr_array(last_yuv), C.c_void_p(cuda_stream or 0)),
+               "rtjgpu_decode_device_window")
+
+    def decode_device_rgb_window(self, d_stream: int, d_desc: int, F: int, w: int, h: int, seq_first, sel, size, origins,
+                                 kind: int, d_rgb: int, row_pitch: int, frame_pitch: int, alpha: int = 0, carries=None,
+                                 last_yuv=None, cuda_stream: int | None = None) -> None:
+        """rtjgpu_decode_device_rgb_window: window row r of frame sel[k] to d_rgb + k * frame_pitch + r * row_pitch;
+        last_yuv as for decode_device_window."""
+        S = len(seq_first) - 1
+        cw, ch = size
+        _check(self._L.rtjgpu_decode_device_rgb_window(self._h, C.c_void_p(d_stream), C.c_void_p(d_desc), F, w, h, S,
+                                                       _int_array(seq_first), _ptr_array(carries), len(sel), _int_array(sel),
+                                                       cw, ch, _origins_array(origins), kind, C.c_void_p(d_rgb or 0),
+                                                       row_pitch, frame_pitch, alpha, _ptr_array(last_yuv),
+                                                       C.c_void_p(cuda_stream or 0)),
+               "rtjgpu_decode_device_rgb_window")
 
     def decode_host(self, stream: np.ndarray, offsets: np.ndarray, out: np.ndarray, state: State | None = None,
                     carry: np.ndarray | None = None, flags: int = 0) -> State:

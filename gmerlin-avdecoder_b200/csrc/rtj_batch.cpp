@@ -192,6 +192,8 @@ struct rtjgpu_ctx {
     bool           seq_pending[2] = {};
     int            seq_turn = 0;
     std::vector<uint32_t> sel_jobs;           /* host scratch of rtjgpu_decode_device[_rgb]_select: K2's job list (RTJ_JOB) */
+    std::vector<uint32_t> win_words;          /* host scratch of rtjgpu_decode_device[_rgb]_window: [S] RTJ_WIN origins, then
+                                               * the jobs of the sequences' last frames (RTJ_JOB(frame, sequence)) */
 };
 
 namespace {
@@ -356,8 +358,16 @@ struct RgbOut {
     int      alpha;              /* its low byte */
 };
 
+/* A window of the selected frames as the caller gave it: cw x ch pixels at origins[2 s], origins[2 s + 1] of sequence s
+ * (host array).  The sequences' last frames leave whole, as planes, to their last_yuv. */
+struct WinIn {
+    int        cw, ch;
+    const int *origins;
+};
+
 /* What a device decode is given: the batch, its sequences, which frames it wants and where they go -- planes to d_out, or
- * packed pixels (rgb != NULL).  rtjgpu_scan_device gives the batch alone. */
+ * packed pixels (rgb != NULL), of the whole picture or of a window (win != NULL, with a selection).  rtjgpu_scan_device
+ * gives the batch alone. */
 struct DecodeCall {
     const uint8_t           *d_stream;
     const rtjgpu_frame_desc *d_desc;
@@ -365,6 +375,7 @@ struct DecodeCall {
     cudaStream_t             stream;
     SeqIn                    q;
     const SelIn             *sel = nullptr;      /* NULL: every frame, at its own index */
+    const WinIn             *win = nullptr;
     uint8_t                 *d_out = nullptr;
     const RgbOut            *rgb = nullptr;
 
@@ -381,6 +392,9 @@ struct CallDev {
     uint8_t *const       *last_yuvs = nullptr;   /* [S] */
     const uint32_t       *d_jobs = nullptr, *h_jobs = nullptr;
     int                   njobs = 0;
+    /* a window (the layout goes up for S = 1 too): [S] RTJ_WIN origins, and the jobs of the last-frame launch */
+    const uint32_t       *win = nullptr, *d_last_jobs = nullptr;
+    int                   nlast = 0;
 };
 
 /* What K1 reads of rtj_launch_args, for all frames of c on ws; every other field zero */
@@ -443,6 +457,23 @@ int run_kernels(rtjgpu_ctx *ctx, Workspace *ws, const DecodeCall &c, const CallD
         a.rgb_kind = rgb->kind; a.rgb_alpha = (unsigned)rgb->alpha & 0xFFu; a.d_last_yuv = c.q.S > 1 ? nullptr : c.q.last(0);
     }
     a.d_seq = dev.seq; a.d_carries = dev.carries; a.d_last_yuvs = dev.last_yuvs;
+    /* a window: K2 of the selected frames over the rows of units the windows span; then one launch over the sequences' last
+     * frames, whole, to their last_yuv (a window is no carry).  No K2b: the window kernels decode HARD blocks themselves. */
+    const WinIn *win = c.win;
+    if (win) {
+        const int lr = ctx->format == RTJ_YUV420 ? 16 : 8;
+        a.d_win = dev.win; a.win_w = win->cw; a.win_h = win->ch; a.win_rows = 0;
+        for (int s = 0; s < c.q.S; s++) {
+            const int y = win->origins[2 * s + 1];
+            a.win_rows = std::max(a.win_rows, (y + win->ch - 1) / lr - y / lr + 1);
+        }
+    }
+    auto last_frames_launch = [&](cudaStream_t s) {
+        rtj_launch_args l = a;
+        l.d_jobs = dev.d_last_jobs; l.j0 = 0; l.j1 = l.njobs = dev.nlast;
+        l.win_w = c.w; l.win_h = c.h; l.win_rows = RTJ_FMT_UNITS_Y(ctx->format, c.h); l.win_last = 1;
+        return rtj_launch_idct(&l, s);
+    };
     {
         const int rc = seg_reserve(ctx, ws, F, nblk, ctx->scan_mode, &a.seg);
         if (rc) return rc;
@@ -488,8 +519,9 @@ int run_kernels(rtjgpu_ctx *ctx, Workspace *ws, const DecodeCall &c, const CallD
         if (sel) job_range(0, F);
         if (!sel || a.j1 > a.j0) {                              /* (an empty selection: K1 and K3 only) */
             LAUNCHED(rtj_launch_idct(&a, st), 1);
-            if (!rgb) LAUNCHED(rtj_launch_idct_hard(&a, st), 2);
+            if (!rgb && !win) LAUNCHED(rtj_launch_idct_hard(&a, st), 2);
         }
+        if (win && dev.nlast) LAUNCHED(last_frames_launch(st), 1);
         if (ev) CK(ctx, cudaEventRecord(ev[3], st));
         return RTJGPU_OK;
     }
@@ -516,7 +548,8 @@ int run_kernels(rtjgpu_ctx *ctx, Workspace *ws, const DecodeCall &c, const CallD
         CK(ctx, cudaEventRecord(ev[2], p.scan));
     }
     a.f0 = 0; a.f1 = F;
-    if (!rgb && (!sel || dev.njobs > 0)) LAUNCHED(rtj_launch_idct_hard(&a, p.idct), 2);
+    if (!rgb && !win && (!sel || dev.njobs > 0)) LAUNCHED(rtj_launch_idct_hard(&a, p.idct), 2);
+    if (win && dev.nlast) LAUNCHED(last_frames_launch(p.idct), 1);
     CK(ctx, cudaEventRecord(p.join, p.idct));
     CK(ctx, cudaStreamWaitEvent(st, p.join, 0));
     if (ev) CK(ctx, cudaEventRecord(ev[3], st));
@@ -568,15 +601,17 @@ int stage_end(rtjgpu_ctx *ctx, void *d_dst, size_t bytes, cudaStream_t st)
 }
 
 /* The device copy of c's layout of S > 1 sequences, in the workspace: [F] RTJ_SEQ words, then [S] carry pointers, then
- * [S] last_yuv pointers -- and behind them, for a selection, its ctx->sel_jobs: one copy either way.  S = 1 uploads the
- * jobs alone. */
+ * [S] last_yuv pointers -- and behind them, for a selection, its ctx->sel_jobs, and for a window its ctx->win_words: one
+ * copy either way.  S = 1 uploads the jobs alone, unless there is a window: the window kernels take every sequence's
+ * origin, carry and last_yuv from the layout. */
 int seq_upload(rtjgpu_ctx *ctx, Workspace *ws, const DecodeCall &c, CallDev *out)
 {
     const SeqIn &q = c.q;
-    const bool layout = q.S > 1;
+    const bool layout = q.S > 1 || c.win;
     const size_t words = layout ? ((size_t)c.F * sizeof(uint32_t) + 7) & ~(size_t)7 : 0, ptrs = layout ? (size_t)q.S * sizeof(void *) : 0;
     const size_t jbytes = c.sel ? ctx->sel_jobs.size() * sizeof(uint32_t) : 0;
-    const size_t bytes = words + 2 * ptrs + jbytes;
+    const size_t wbytes = c.win ? ctx->win_words.size() * sizeof(uint32_t) : 0;
+    const size_t bytes = words + 2 * ptrs + jbytes + wbytes;
     uint8_t *h;
     int rc = stage_begin(ctx, bytes, &h);
     if (rc) return rc;
@@ -590,6 +625,7 @@ int seq_upload(rtjgpu_ctx *ctx, Workspace *ws, const DecodeCall &c, CallDev *out
         for (int s = 0; s < q.S; s++) { hc[s] = q.carry(s); hl[s] = q.last(s); }
     }
     if (jbytes) memcpy(h + words + 2 * ptrs, ctx->sel_jobs.data(), jbytes);
+    if (wbytes) memcpy(h + words + 2 * ptrs + jbytes, ctx->win_words.data(), wbytes);
     const uint8_t *d = ws->d_seq.get();
     if ((rc = stage_end(ctx, ws->d_seq.get(), bytes, c.stream))) return rc;
     if (layout) {
@@ -601,6 +637,12 @@ int seq_upload(rtjgpu_ctx *ctx, Workspace *ws, const DecodeCall &c, CallDev *out
         out->d_jobs = reinterpret_cast<const uint32_t *>(d + words + 2 * ptrs);
         out->h_jobs = ctx->sel_jobs.data();
         out->njobs = (int)ctx->sel_jobs.size();
+    }
+    if (c.win) {
+        const uint32_t *wd = reinterpret_cast<const uint32_t *>(d + words + 2 * ptrs + jbytes);
+        out->win = wd;
+        out->d_last_jobs = wd + q.S;
+        out->nlast = (int)ctx->win_words.size() - q.S;
     }
     return RTJGPU_OK;
 }
@@ -641,10 +683,21 @@ int check_batch(rtjgpu_ctx *ctx, const DecodeCall &c, bool output, int *nblk)
     /* K1 reads the stream as 32-bit words, K2 leaves its strips as 16-byte bulk stores and reads the carry as 8-byte rows */
     if (((uintptr_t)c.d_stream & 3) || ((uintptr_t)c.d_desc & 7)) return RTJGPU_E_ARG;
     if (output && (((uintptr_t)dst & 15) || ((uintptr_t)c.q.carry(0) & 7) || ((uintptr_t)c.q.last(0) & 15))) return RTJGPU_E_ARG;
+    /* a window: x and cw multiples of 16, y and ch even, inside the picture -- every output row starts 8- or 16-byte aligned
+     * and the two luma rows of a chroma row stay together */
+    if (output && c.win) {
+        const WinIn &v = *c.win;
+        if (v.cw <= 0 || v.ch <= 0 || (v.cw & 15) || (v.ch & 1) || !v.origins) return RTJGPU_E_ARG;
+        for (int s = 0; s < c.q.S; s++) {
+            const int x = v.origins[2 * s], y = v.origins[2 * s + 1];
+            if (x < 0 || y < 0 || (x & 15) || (y & 1) || x > c.w - v.cw || y > c.h - v.ch) return RTJGPU_E_ARG;
+        }
+    }
     if (output && c.rgb) {
         const RgbOut &o = *c.rgb;
-        if ((o.row_pitch & 15) || (o.frame_pitch & 15) || o.row_pitch < (size_t)c.w * rtj_convert_bpp(o.kind)
-            || o.frame_pitch < o.row_pitch * (size_t)c.h)
+        const int ow = c.win ? c.win->cw : c.w, oh = c.win ? c.win->ch : c.h;     /* the picture that leaves */
+        if ((o.row_pitch & 15) || (o.frame_pitch & 15) || o.row_pitch < (size_t)ow * rtj_convert_bpp(o.kind)
+            || o.frame_pitch < o.row_pitch * (size_t)oh)
             return RTJGPU_E_ARG;
     }
     if (!valid_size(c.w, c.h)) return RTJGPU_E_SIZE;
@@ -671,15 +724,24 @@ int decode(rtjgpu_ctx *ctx, DecodeCall c)
     if (c.q.first && (rc = seq_check(c.F, c.q))) return rc;
     if (c.sel) {
         if ((rc = sel_check(c.F, *c.sel))) return rc;
-        if (c.sel->n == c.F) c.sel = nullptr;         /* every frame: the full call, runs of frames and last frames as planes included */
+        /* every frame: the full call, runs of frames and last frames as planes included (a window stays a selection) */
+        if (c.sel->n == c.F && !c.win) c.sel = nullptr;
     }
     if (c.F == 0) { ctx->last_F = 0; return RTJGPU_OK; }
     int nblk;
     if ((rc = check_batch(ctx, c, true, &nblk))) return rc;
     if ((rc = ws_reserve(ctx, &ctx->ws, c.F, nblk))) return rc;
     CallDev dev;
-    if (c.sel) sel_jobs(ctx, c.q, *c.sel, c.rgb != nullptr);
-    if ((c.q.S > 1 || (c.sel && !ctx->sel_jobs.empty())) && (rc = seq_upload(ctx, &ctx->ws, c, &dev))) return rc;
+    if (c.sel) sel_jobs(ctx, c.q, *c.sel, c.rgb != nullptr && !c.win);
+    if (c.win) {
+        /* the sequences' origins, then the jobs of the last-frame launch: each sequence's last frame that has a last_yuv */
+        std::vector<uint32_t> &ww = ctx->win_words;
+        ww.clear();
+        for (int s = 0; s < c.q.S; s++) ww.push_back(RTJ_WIN(c.win->origins[2 * s], c.win->origins[2 * s + 1]));
+        for (int s = 0; s < c.q.S; s++)
+            if (c.q.last(s)) ww.push_back(RTJ_JOB(c.q.first[s + 1] - 1, s));
+    }
+    if ((c.q.S > 1 || c.win || (c.sel && !ctx->sel_jobs.empty())) && (rc = seq_upload(ctx, &ctx->ws, c, &dev))) return rc;
     cudaEvent_t *ev = ctx->timing ? ctx->ev[ctx->timed_calls % TIMING_RING] : nullptr;
     rc = run_kernels(ctx, &ctx->ws, c, dev, ev, true);
     if (ev && rc == RTJGPU_OK) ctx->timed_calls++;
@@ -1269,6 +1331,40 @@ int rtjgpu_decode_device_rgb_select(rtjgpu_ctx *ctx, const uint8_t *d_stream, co
     DecodeCall c(d_stream, d_desc, F, w, h, cuda_stream);
     c.q.S = S; c.q.first = seq_first; c.q.carries = carries; c.q.last_yuv = last_yuv;
     c.sel = &s;
+    c.rgb = &o;
+    return decode(ctx, c);
+}
+
+int rtjgpu_decode_device_window(rtjgpu_ctx *ctx, const uint8_t *d_stream, const rtjgpu_frame_desc *d_desc, int F, int w, int h,
+                                int S, const int *seq_first, const uint8_t *const *carries,
+                                int n, const int *sel, int cw, int ch, const int *origins,
+                                uint8_t *d_out, uint8_t *const *last_yuv, void *cuda_stream)
+{
+    if (!seq_first) return RTJGPU_E_ARG;
+    const SelIn s{n, sel};
+    const WinIn v{cw, ch, origins};
+    DecodeCall c(d_stream, d_desc, F, w, h, cuda_stream);
+    c.q.S = S; c.q.first = seq_first; c.q.carries = carries; c.q.last_yuv = last_yuv;
+    c.sel = &s;
+    c.win = &v;
+    c.d_out = d_out;
+    return decode(ctx, c);
+}
+
+int rtjgpu_decode_device_rgb_window(rtjgpu_ctx *ctx, const uint8_t *d_stream, const rtjgpu_frame_desc *d_desc, int F, int w, int h,
+                                    int S, const int *seq_first, const uint8_t *const *carries,
+                                    int n, const int *sel, int cw, int ch, const int *origins,
+                                    int kind, uint8_t *d_rgb, size_t row_pitch, size_t frame_pitch, int alpha,
+                                    uint8_t *const *last_yuv, void *cuda_stream)
+{
+    if (!seq_first) return RTJGPU_E_ARG;
+    const SelIn s{n, sel};
+    const WinIn v{cw, ch, origins};
+    const RgbOut o{d_rgb, row_pitch, frame_pitch, kind, alpha};
+    DecodeCall c(d_stream, d_desc, F, w, h, cuda_stream);
+    c.q.S = S; c.q.first = seq_first; c.q.carries = carries; c.q.last_yuv = last_yuv;
+    c.sel = &s;
+    c.win = &v;
     c.rgb = &o;
     return decode(ctx, c);
 }

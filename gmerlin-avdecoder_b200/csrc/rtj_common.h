@@ -66,6 +66,12 @@ extern "C" {
 #define RTJ_JOB_SLOT(v) ((v) >> 16)
 #define RTJ_JOB_NO_SLOT 0xFFFFu
 
+/* Per-sequence word of a call that decodes a window of its frames (rtjgpu_decode_device[_rgb]_window): the window's origin
+ * in pixels, x a multiple of 16 and y even, both below 2^16 (they lie inside a picture of at most 65535 x 65535). */
+#define RTJ_WIN(x, y) ((uint32_t)(x) | (uint32_t)(y) << 16)
+#define RTJ_WIN_X(v) ((v) & 0xFFFFu)
+#define RTJ_WIN_Y(v) ((v) >> 16)
+
 #define RTJ_NUM_TABLES 257
 
 /* Dequantisation tables as the kernels read them: zig-zag order (entry k is
@@ -184,6 +190,11 @@ typedef struct rtj_launch_args {
      * frame per CTA over jobs [j0, j1) of the batch's njobs RTJ_JOB words, sorted by frame */
     const uint32_t          *d_jobs;
     int                      j0, j1, njobs;
+    /* a window of the selected frames (rtjgpu_decode_device[_rgb]_window; win_w == 0: none): win_w x win_h pixels at each
+     * sequence's RTJ_WIN origin in d_win, over the most rows of units any sequence's window spans (win_rows).  win_last: the
+     * launch of the sequences' last frames, a whole-picture window that leaves as planes to d_last_yuvs */
+    const uint32_t          *d_win;
+    int                      win_w, win_h, win_rows, win_last;
 } rtj_launch_args;
 
 int rtj_launch_scan(const rtj_launch_args *a, void *stream);          /* returns the number of launches (>0) or -cudaError */

@@ -525,6 +525,11 @@ struct K2Params {
      * `ahead` then counts jobs */
     const uint32_t *jobs;
     int j0, njobs;
+    /* WIN: a window of win_w x win_h pixels of every job's frame, at the origin of the frame's sequence (RTJ_WIN words,
+     * per sequence; seq is never NULL).  win_last = 0: the window leaves to out + slot * frame_bytes(win_w, win_h) as tight
+     * planes, or as packed pixels; 1: the window is the whole picture and leaves as planes to last_yuvs[sequence] */
+    const uint32_t *win;
+    int win_w, win_h, win_last;
 };
 
 /* The general decoder for one block that K2's sparse classes do not take (long blocks; blocks whose last writer used
@@ -602,13 +607,19 @@ constexpr int RGB_NONE = -1, RGB_ANY = 99;
  * frame needs only its own entries and its last writers' (K3), never the pixels of the frames before it.  Its pixels go to
  * the job's output slot -- K2b's queue names the slot as the place they go to --; a fused-RGB job without a slot (an
  * unselected last frame of a sequence) leaves as planes for last_yuv only. */
-template <bool SINGLE, int FMT, int WARPS, int RGBK, bool RUN, bool RES = false, bool SEL = false>
+/* WIN: a window of every selected frame (rtjgpu_decode_device[_rgb]_window), strips only.  blockIdx.x walks the strips and
+ * rows of units of the window of the frame's sequence, from its origin; a CTA below its own window returns at once.  HARD
+ * blocks are decoded here by the general path, as in the fused-RGB kernels: no K2b, so no block of K2b's would have to be
+ * clipped.  The strip is complete in shared memory before it leaves, clipped to the window's rows. */
+template <bool SINGLE, int FMT, int WARPS, int RGBK, bool RUN, bool RES = false, bool SEL = false, bool WIN = false>
 __global__ void __launch_bounds__(WARPS * 32, WARPS == 4 ? 8 : 10)
 rtj_idct_kernel(const K2Params P)
 {
     constexpr bool RGB = RGBK != RGB_NONE;
     static_assert(!RGB || FMT == 0, "the fused converters are the reference's yuv420 ones");
     static_assert(!SEL || (!RUN && !RES), "a selection is decoded one frame per CTA, without K2b's reservations");
+    static_assert(!WIN || (SEL && !SINGLE), "a window is a selection, decoded in strips");
+    constexpr bool GENERAL = RGB || WIN;                     /* HARD blocks decoded in this kernel, not queued for K2b */
     constexpr int THREADS = WARPS * 32;
     typedef Geo<FMT> G;
     extern __shared__ __align__(128) uint8_t smem[];
@@ -623,10 +634,14 @@ rtj_idct_kernel(const K2Params P)
     const unsigned f_last = RUN ? min(f_first + (unsigned)P.run, (unsigned)P.f_end) : f_first + 1u;       /* one behind */
     constexpr bool runs = RUN;
     const int w = P.w, h = P.h, mbw = w / G::UNIT_W;           /* units per picture row */
+    /* WIN: the window's origin -- wx in units, wy in pixels -- and the unit it starts in */
+    const uint32_t worg = WIN && !P.win_last ? __ldg(P.win + RTJ_SEQ_INDEX(P.seq[f_first])) : 0u;
+    const int wx = WIN ? (int)RTJ_WIN_X(worg) / G::UNIT_W : 0, wy = WIN ? (int)RTJ_WIN_Y(worg) : 0;
     const int strip = SINGLE ? 0 : (int)(blockIdx.x % (unsigned)P.nstrips);
-    const int my = P.row0 + (SINGLE ? (int)blockIdx.x : (int)(blockIdx.x / (unsigned)P.nstrips));
-    const int mx0 = strip * P.seg_mb;
-    const int mbs = SINGLE ? mbw : min(P.seg_mb, mbw - mx0);
+    const int my = (WIN ? wy / G::LUMA_ROWS : P.row0) + (SINGLE ? (int)blockIdx.x : (int)(blockIdx.x / (unsigned)P.nstrips));
+    if (WIN && my > (wy + P.win_h - 1) / G::LUMA_ROWS) return;  /* below this sequence's window (before any barrier) */
+    const int mx0 = (WIN ? wx : 0) + strip * P.seg_mb;
+    const int mbs = SINGLE ? mbw : min(P.seg_mb, (WIN ? wx + P.win_w / G::UNIT_W : mbw) - mx0);
     const int nb = mbs * G::BLK;
     const unsigned strip_blk0 = (unsigned)(my * mbw + mx0) * (unsigned)G::BLK;
 
@@ -842,8 +857,9 @@ rtj_idct_kernel(const K2Params P)
             const bool hard = live && !(ie >> 31);
             const bool full = hard && ((ie >> 30) & 1u);
             const int bi = (int)(ie & 0x3FFFFFFFu);              /* stream-order index inside the strip */
-            if (RGB) {
-                /* no planes for rtj_idct_hard_kernel to patch: the general decoder runs here, out of line */
+            if (GENERAL) {
+                /* no planes for rtj_idct_hard_kernel to patch (packed pixels, or a window's): the general decoder runs here,
+                 * out of line */
                 if (hard) {
                     uint32_t px[16];
                     decode_general_call(P.stream, P.desc, P.tables, P.ent, P.srcf, P.nblk, frame_blk0 + (unsigned)bi,
@@ -851,7 +867,7 @@ rtj_idct_kernel(const K2Params P)
                     store_block<FMT>(tile_s, off, mbs, px);
                 }
             }
-            const unsigned mH = RGB ? 0u : __ballot_sync(FULL, hard && !full), mF = RGB ? 0u : __ballot_sync(FULL, full);
+            const unsigned mH = GENERAL ? 0u : __ballot_sync(FULL, hard && !full), mF = GENERAL ? 0u : __ballot_sync(FULL, full);
             if (mH | mF) {
                 /* the device queue is filled from both ends: mid-size blocks from the front, long ones from the back */
                 unsigned base = qbase16, baseF = qbaseF;
@@ -914,11 +930,15 @@ rtj_idct_kernel(const K2Params P)
         const uint8_t *tU = tile + G::CHROMA_AT * mbs, *tV = tU + 64 * mbs;
         const int kind = RGBK == RGB_ANY ? P.rgb_kind : RGBK;
         const int bpp = (kind == RTJ_CONV_RGB32 || kind == RTJ_CONV_BGR32) ? 4 : kind == RTJ_CONV_RGB16 ? 2 : 3;
-        uint8_t *base = P.rgb + (size_t)(SEL ? RTJ_JOB_SLOT(job) : f) * P.rgb_frame_pitch + (size_t)(my * 16) * P.rgb_row_pitch
-                        + (size_t)(mx0 * 16) * bpp;
-        const int items = SEL && RTJ_JOB_SLOT(job) == RTJ_JOB_NO_SLOT ? 0 : 8 * chunks;    /* SEL: planes for last_yuv only */
+        /* WIN: strip row r is window row top + r; the row pairs inside the window are [rp0, rp1) (top, wy and win_h are even) */
+        const int top = my * 16 - wy;
+        const int rp0 = WIN ? max(0, -top) >> 1 : 0, rp1 = WIN ? min(16, P.win_h - top) >> 1 : 8;
+        uint8_t *base = WIN ? P.rgb + (size_t)RTJ_JOB_SLOT(job) * P.rgb_frame_pitch + (size_t)((mx0 - wx) * 16) * bpp
+                            : P.rgb + (size_t)(SEL ? RTJ_JOB_SLOT(job) : f) * P.rgb_frame_pitch + (size_t)(my * 16) * P.rgb_row_pitch
+                              + (size_t)(mx0 * 16) * bpp;
+        const int items = SEL && RTJ_JOB_SLOT(job) == RTJ_JOB_NO_SLOT ? 0 : (rp1 - rp0) * chunks;    /* SEL: planes for last_yuv only */
         for (int item = tid; item < items; item += THREADS) {
-            const int rp = item / chunks, c = item - rp * chunks;
+            const int rp = rp0 + item / chunks, c = item - (rp - rp0) * chunks;
             const uint2 y0 = *reinterpret_cast<const uint2 *>(tile + (2 * rp) * lw + c * 8);
             const uint2 y1 = *reinterpret_cast<const uint2 *>(tile + (2 * rp + 1) * lw + c * 8);
             const uint32_t ub = *reinterpret_cast<const uint32_t *>(tU + rp * (lw >> 1) + c * 4);
@@ -926,7 +946,7 @@ rtj_idct_kernel(const K2Params P)
             Chroma ct[4];
 #pragma unroll
             for (int k = 0; k < 4; k++) ct[k] = chroma_terms((ub >> (8 * k)) & 0xFFu, (vb >> (8 * k)) & 0xFFu);
-            uint8_t *o = base + (size_t)(2 * rp) * P.rgb_row_pitch + (size_t)c * (8 * bpp);
+            uint8_t *o = base + (size_t)((WIN ? top : 0) + 2 * rp) * P.rgb_row_pitch + (size_t)c * (8 * bpp);
             switch (kind) {
             case RTJ_CONV_RGB32: row8<RTJ_CONV_RGB32>(y0, ct, P.rgb_alpha, o); row8<RTJ_CONV_RGB32>(y1, ct, P.rgb_alpha, o + P.rgb_row_pitch); break;
             case RTJ_CONV_BGR32: row8<RTJ_CONV_BGR32>(y0, ct, P.rgb_alpha, o); row8<RTJ_CONV_BGR32>(y1, ct, P.rgb_alpha, o + P.rgb_row_pitch); break;
@@ -935,12 +955,48 @@ rtj_idct_kernel(const K2Params P)
             default:             row8<RTJ_CONV_RGB16>(y0, ct, P.rgb_alpha, o); row8<RTJ_CONV_RGB16>(y1, ct, P.rgb_alpha, o + P.rgb_row_pitch); break;
             }
         }
-        /* the last frame also leaves as planes: the next batch's carry -- with several sequences, the last frame of each */
-        if (P.seq) {
+        /* the last frame also leaves as planes: the next batch's carry -- with several sequences, the last frame of each
+         * (WIN: the strips cover the window only; the last frames have a launch of their own) */
+        if (WIN) last_planes = nullptr;
+        else if (P.seq) {
             const unsigned nx = f + 1u;
             last_planes = nx == (unsigned)P.F || RTJ_SEQ_FIRST(P.seq[nx]) == nx ? P.last_yuvs[RTJ_SEQ_INDEX(P.seq[f])] : nullptr;
         } else if (f + 1u != (unsigned)P.F) last_planes = nullptr;
         if (!last_planes) planes_leave = false;
+    } else if (WIN) {
+        /* The window's planes, tight at the window's pitch: the strip's rows inside the window, in the strip path's vector
+         * widths.  Strip luma row r is window row top + r, strip chroma row r window chroma row ctop + r. */
+        const int ww = P.win_w, wh = P.win_h, wcw = ww >> 1;
+        constexpr int VS = FMT == 0 ? 2 : 1;                     /* vertical chroma subsampling */
+        uint8_t *const planes = P.win_last ? P.last_yuvs[RTJ_SEQ_INDEX(P.seq[f])]
+                                           : P.out + (size_t)RTJ_JOB_SLOT(job) * RTJ_FMT_FRAME_BYTES(FMT, ww, wh);
+        const int top = my * G::LUMA_ROWS - wy, ctop = my * 8 - wy / VS;
+        const int r0 = max(0, -top), r1 = min(G::LUMA_ROWS, wh - top);
+        const int c0 = max(0, -ctop), c1 = min(8, wh / VS - ctop);
+        uint8_t *oy = planes + (mx0 - wx) * G::UNIT_W;
+        uint8_t *ou = planes + (size_t)ww * wh + (mx0 - wx) * 8;
+        uint8_t *ov = ou + (size_t)wcw * (wh / VS);
+        const uint8_t *tileU = tile + G::CHROMA_AT * mbs, *tileV = tileU + 64 * mbs;
+        for (int r = r0 + warp; r < r1; r += WARPS) {
+            if (G::UNIT_W == 16) {
+                for (int c = lane; c < mbs; c += 32)
+                    *reinterpret_cast<uint4 *>(oy + (size_t)(top + r) * ww + c * 16) = *reinterpret_cast<const uint4 *>(tile + r * lw + c * 16);
+            } else {
+                for (int c = lane; c < mbs; c += 32)
+                    *reinterpret_cast<uint2 *>(oy + (size_t)(top + r) * ww + c * 8) = *reinterpret_cast<const uint2 *>(tile + r * lw + c * 8);
+            }
+        }
+        if (G::PLANES == 3) {
+            const int segC = lw >> 1;
+            for (int r = warp; r < 16; r += WARPS) {
+                const int pl = r >> 3, rr = r & 7;
+                if (rr < c0 || rr >= c1) continue;
+                for (int c = lane; c < (segC >> 3); c += 32)
+                    *reinterpret_cast<uint2 *>((pl ? ov : ou) + (size_t)(ctop + rr) * wcw + c * 8) =
+                        *reinterpret_cast<const uint2 *>((pl ? tileV : tileU) + rr * segC + c * 8);
+            }
+        }
+        planes_leave = false;
     } else {
         /* What rtj_idct_hard*_kernel patch need not be written here first.  All blocks HARD: nothing leaves; all luma blocks
          * (a quality above 170, where every luma block carries ten coefficients or more): the chroma rows only. */
@@ -1303,6 +1359,11 @@ cudaError_t k2_attr()
     if (e == cudaSuccess)
         e = cudaFuncSetAttribute(rtj_idct_kernel<SINGLE, FMT, WARPS, RGBK, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                  (int)idct_smem_bytes(IDCT_MAX_MB, FMT, 3));
+    if constexpr (!SINGLE) {
+        if (e == cudaSuccess)
+            e = cudaFuncSetAttribute(rtj_idct_kernel<false, FMT, WARPS, RGBK, false, false, true, true>,
+                                     cudaFuncAttributeMaxDynamicSharedMemorySize, (int)idct_smem_bytes(IDCT_MAX_MB, FMT, 3));
+    }
     return e;
 }
 
@@ -1369,6 +1430,23 @@ cudaError_t k2_launch(K2Params &P, int grid_x, int F, cudaStream_t st)
         if (warps == 4) e = launch_pdl(rtj_idct_kernel<false, FMT, 4, RGBS, false>, grid, dim3(128), smem, st, P);
         else e = launch_pdl(rtj_idct_kernel<false, FMT, 3, RGBS, false>, grid, dim3(96), smem, st, P);
     }
+    return e != cudaSuccess ? e : cudaGetLastError();
+}
+
+/* a window of a selection (P.win_w != 0): the strip kernels, one frame per CTA; RGBK is RGB_NONE or RGB_ANY */
+template <int FMT, int RGBK>
+cudaError_t k2_launch_win(K2Params &P, int grid_x, int njobs, cudaStream_t st)
+{
+    const int blk = FMT == 0 ? 6 : FMT == 1 ? 4 : 1;
+    const int warps = idct_warps(P.seg_mb * blk);
+    P.wq = idct_wq(P.seg_mb * blk, warps);
+    const int resident = (g_sm_count > 0 ? g_sm_count : 148) * (warps == 4 ? 8 : 10);
+    P.ahead = (resident + grid_x - 1) / grid_x;
+    P.run = 1;
+    const size_t smem = idct_smem_bytes(P.seg_mb, FMT, warps);
+    const dim3 grid((unsigned)grid_x, (unsigned)njobs);
+    const cudaError_t e = warps == 4 ? launch_pdl(rtj_idct_kernel<false, FMT, 4, RGBK, false, false, true, true>, grid, dim3(128), smem, st, P)
+                                     : launch_pdl(rtj_idct_kernel<false, FMT, 3, RGBK, false, false, true, true>, grid, dim3(96), smem, st, P);
     return e != cudaSuccess ? e : cudaGetLastError();
 }
 
@@ -1448,6 +1526,16 @@ extern "C" int rtj_launch_idct(const rtj_launch_args *a, void *stream)
     P.rgb = a->d_rgb; P.rgb_row_pitch = a->rgb_row_pitch; P.rgb_frame_pitch = a->rgb_frame_pitch;
     P.rgb_kind = a->rgb_kind; P.rgb_alpha = a->rgb_alpha & 0xFFu; P.last_yuv = a->d_last_yuv;
     P.seq = a->d_seq; P.carries = a->d_carries; P.last_yuvs = a->d_last_yuvs;
+    P.win = a->d_win; P.win_w = a->win_w; P.win_h = a->win_h; P.win_last = a->win_last;
+    if (a->win_w) {
+        /* a window: strips cut from the window's width, over the most rows of units any sequence's window spans */
+        if (!a->d_jobs || !a->d_seq || a->win_rows <= 0) return (int)cudaErrorInvalidValue;
+        P.seg_mb = idct_seg_mb(RTJ_FMT_UNITS_X(fmt, a->win_w), &P.nstrips);
+        const int gx = P.nstrips * a->win_rows;
+        if (a->fused_rgb && !a->win_last) return fmt == 0 ? (int)k2_launch_win<0, RGB_ANY>(P, gx, nf, st) : (int)cudaErrorInvalidValue;
+        return (int)(fmt == 0 ? k2_launch_win<0, RGB_NONE>(P, gx, nf, st) : fmt == 1 ? k2_launch_win<1, RGB_NONE>(P, gx, nf, st)
+                                                                       : k2_launch_win<2, RGB_NONE>(P, gx, nf, st));
+    }
     if (a->fused_rgb) {
         if (fmt != 0) return (int)cudaErrorInvalidValue;
         switch (a->rgb_kind) {

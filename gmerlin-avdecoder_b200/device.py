@@ -90,6 +90,54 @@ def decode_select(ctx: capi.BatchContext, b: DeviceBatch, seq_first, sel, carrie
     return out
 
 
+def _window_args(seq_first, sel, size, origins, last):
+    S = len(seq_first) - 1
+    sel = [int(x) for x in np.asarray(sel, dtype=np.int64).reshape(-1)]
+    cw, ch = int(size[0]), int(size[1])
+    origins = [tuple(origins)] * S if np.ndim(origins) == 1 else [tuple(o) for o in origins]
+    last_ptrs = None if last is None else [None if t is None else t.data_ptr() for t in last]
+    return sel, cw, ch, origins, last_ptrs
+
+
+def decode_window(ctx: capi.BatchContext, b: DeviceBatch, seq_first, sel, size, origins, carries=None, last=None,
+                  out: torch.Tensor | None = None, stream: torch.cuda.Stream | None = None) -> torch.Tensor:
+    """rtjgpu_decode_device_window over a batch of upload_sequences: the batch frames sel (as for decode_select), only a
+    window of size = (cw, ch) pixels of each, at origins -- one (x, y) for every sequence, or S pairs.  Frame sel[k] goes
+    to row k of the result as the tight planes of a cw x ch picture.  last: a list of S tensors (or None entries) that
+    receive each sequence's last frame whole, as planes (the next call's carries), or None.  out: a [n, window_bytes]
+    uint8 tensor to fill (default: a new one).  Returns out."""
+    st = stream if stream is not None else torch.cuda.current_stream(b.stream.device)
+    sel, cw, ch, origins, last_ptrs = _window_args(seq_first, sel, size, origins, last)
+    if out is None:
+        out = torch.empty((len(sel), capi.frame_bytes(b.fmt, cw, ch)), dtype=torch.uint8, device=b.stream.device)
+    assert out.dtype == torch.uint8 and out.is_contiguous() and out.numel() >= len(sel) * capi.frame_bytes(b.fmt, cw, ch)
+    ctx.set_format(b.fmt)
+    ptrs = None if carries is None else [None if c is None else c.data_ptr() for c in carries]
+    ctx.decode_device_window(b.stream.data_ptr(), b.desc.data_ptr(), b.F, b.w, b.h, list(seq_first), sel, (cw, ch), origins,
+                             out.data_ptr() if len(sel) else None, ptrs, last_ptrs, st.cuda_stream)
+    return out
+
+
+def decode_rgb_window(ctx: capi.BatchContext, b: DeviceBatch, seq_first, sel, size, origins, kind: int, alpha: int = 255,
+                      carries=None, last=None, out: torch.Tensor | None = None,
+                      stream: torch.cuda.Stream | None = None) -> torch.Tensor:
+    """rtjgpu_decode_device_rgb_window: decode_window with one of the reference's yuv420 converters (capi.CONV_RGB32 ...
+    RGB16) fused in.  Returns a tight [n, ch, cw, bpp] uint8 tensor (out, if given, must be one), alpha in the fourth byte
+    of 32-bit pixels.  YUV420 batches only."""
+    st = stream if stream is not None else torch.cuda.current_stream(b.stream.device)
+    sel, cw, ch, origins, last_ptrs = _window_args(seq_first, sel, size, origins, last)
+    bpp = capi.CONV_BPP[kind]
+    if out is None:
+        out = torch.empty((len(sel), ch, cw, bpp), dtype=torch.uint8, device=b.stream.device)
+    assert out.dtype == torch.uint8 and out.is_contiguous() and tuple(out.shape) == (len(sel), ch, cw, bpp)
+    ctx.set_format(b.fmt)
+    ptrs = None if carries is None else [None if c is None else c.data_ptr() for c in carries]
+    ctx.decode_device_rgb_window(b.stream.data_ptr(), b.desc.data_ptr(), b.F, b.w, b.h, list(seq_first), sel, (cw, ch),
+                                 origins, kind, out.data_ptr() if len(sel) else None, cw * bpp, ch * cw * bpp, alpha, ptrs,
+                                 last_ptrs, st.cuda_stream)
+    return out
+
+
 def encode_sequences(ctx: capi.BatchContext, pictures, encoders, w: int, h: int, fmt: int = 0,
                      stream: torch.cuda.Stream | None = None):
     """rtjgpu_encode_device_seq: pictures a list of S uint8 device tensors (or views), each one sequence's consecutive

@@ -393,6 +393,33 @@ int  rtjgpu_decode_device_rgb_select(rtjgpu_ctx *ctx, const uint8_t *d_stream, c
                                      int n, const int *sel, int kind, uint8_t *d_rgb, size_t row_pitch, size_t frame_pitch,
                                      int alpha, uint8_t *const *last_yuv, void *cuda_stream);
 
+/* ONLY THE PART OF THE PICTURE A CALLER ASKS FOR.  The batch (F, S, seq_first, carries) and the selection (n, sel) are exactly
+ * those of rtjgpu_decode_device_select.  origins is a HOST array of 2 S ints, (x, y) of sequence s's window, read before the
+ * call returns; the window is cw x ch pixels for every sequence.  Selected frame sel[k] goes to d_out + k * window_bytes,
+ * window_bytes = the tight planes of a cw x ch picture of the context's format (Y cw x ch, then U and V: (cw/2) x (ch/2) in
+ * YUV420, (cw/2) x ch in YUV422; grey Y only), each plane byte for byte the crop of what rtjgpu_decode_device_select writes
+ * for that frame.  A window is no carry: last_yuv (host array of S device pointers, or NULL; entries may be NULL, 16-byte
+ * aligned) receives each sequence's last frame of the batch as FULL planes, selected or not -- that sequence's next carry.
+ * n = 0 writes those planes only (d_out may then be NULL).  Nothing else is written; afterwards rtjgpu_get_batch_info and
+ * rtjgpu_get_skip_counts describe all F frames, and K2 decodes one frame per CTA whatever rtjgpu_set_frame_runs says.  Only
+ * the units that cover a window are decoded; a sequence's last frame that is selected is decoded twice (window and planes).
+ * Every argument is checked before anything is launched: rtjgpu_decode_device_select's rules, and RTJGPU_E_ARG for cw or ch
+ * <= 0, cw or any x not a multiple of 16, ch or any y odd, origins == NULL, a window that does not lie inside the picture, or
+ * a misaligned last_yuv entry.  Asynchronous on cuda_stream. */
+int  rtjgpu_decode_device_window(rtjgpu_ctx *ctx, const uint8_t *d_stream, const rtjgpu_frame_desc *d_desc, int F, int w, int h,
+                                 int S, const int *seq_first, const uint8_t *const *carries,
+                                 int n, const int *sel, int cw, int ch, const int *origins,
+                                 uint8_t *d_out, uint8_t *const *last_yuv, void *cuda_stream);
+/* The same with rtjgpu_decode_device_rgb_select's fused converter: window row r of frame sel[k] goes to d_rgb + k * frame_pitch
+ * + r * row_pitch, cw * bytes-per-pixel bytes, byte for byte the crop of rtjgpu_decode_device_rgb_select's picture (alpha in
+ * the fourth byte).  last_yuv as above.  RTJGPU_E_ARG also for a pitch that is not a multiple of 16, row_pitch < cw * bpp or
+ * frame_pitch < ch * row_pitch; RTJGPU_E_FORMAT on a context that is not RTJ_YUV420. */
+int  rtjgpu_decode_device_rgb_window(rtjgpu_ctx *ctx, const uint8_t *d_stream, const rtjgpu_frame_desc *d_desc, int F, int w, int h,
+                                     int S, const int *seq_first, const uint8_t *const *carries,
+                                     int n, const int *sel, int cw, int ch, const int *origins,
+                                     int kind, uint8_t *d_rgb, size_t row_pitch, size_t frame_pitch, int alpha,
+                                     uint8_t *const *last_yuv, void *cuda_stream);
+
 /* Host-buffer decode: packets in host memory in, frames in host memory out.
  * The batch is cut into chunks that move through pinned staging buffers with
  * cudaMemcpyAsync on several streams so that copies overlap the kernels.
