@@ -163,6 +163,10 @@ def load_library() -> C.CDLL:
                                                   C.POINTER(vp), C.c_int, C.POINTER(C.c_int), C.c_int, C.c_int,
                                                   C.POINTER(C.c_int), C.c_int, vp, C.c_size_t, C.c_size_t, C.c_int,
                                                   C.POINTER(vp), vp]
+    L.rtjgpu_decode_device_chw_window.argtypes = [vp, vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_int),
+                                                  C.POINTER(vp), C.c_int, C.POINTER(C.c_int), C.c_int, C.c_int,
+                                                  C.POINTER(C.c_int), C.POINTER(C.c_int), C.c_int, C.c_int,
+                                                  C.POINTER(C.c_float), C.POINTER(C.c_float), vp, C.POINTER(vp), vp]
     L.rtjgpu_decode_host.argtypes = [vp, _u8p, _u64p, C.c_int, C.POINTER(State), _u8p, _u8p, C.c_int]
     L.rtjgpu_sync.argtypes = [vp]
     L.rtjgpu_enable_timing.argtypes = [vp, C.c_int]
@@ -201,6 +205,23 @@ CONVERTERS = ("RTjpeg_yuv420rgb32", "RTjpeg_yuv420bgr32", "RTjpeg_yuv420rgb24", 
               "RTjpeg_yuv420rgb16", "RTjpeg_yuv420rgb8", "RTjpeg_yuv422rgb24")
 CONV_BPP = (4, 4, 3, 3, 2, 1, 3)
 
+# element types of rtjgpu_decode_device_chw_window, indexed by RTJ_CHW_*, and their sizes in bytes
+CHW_U8, CHW_F16, CHW_BF16, CHW_F32 = range(4)
+CHW_ESIZE = (1, 2, 2, 4)
+
+
+def normalize_coefficients(mean, std):
+    """The per-channel scale and bias of rtjgpu_decode_device_chw_window that mean torchvision's normalisation of a byte v,
+    (v / 255 - mean) / std: scale = 1 / (255 std), bias = -mean / std.  Computed in float64, rounded once to float32.
+    Returns (scale, bias), two float32 arrays of 3."""
+    mean = np.asarray(mean, dtype=np.float64).reshape(-1)
+    std = np.asarray(std, dtype=np.float64).reshape(-1)
+    if mean.shape != (3,) or std.shape != (3,):
+        raise ValueError("normalize_coefficients: mean and std take 3 values, one per channel")
+    if not (np.isfinite(mean).all() and np.isfinite(std).all()) or (std == 0).any():
+        raise ValueError("normalize_coefficients: mean and std must be finite, std nonzero")
+    return (1.0 / (255.0 * std)).astype(np.float32), (-mean / std).astype(np.float32)
+
 
 def frame_bytes(fmt: int, w: int, h: int) -> int:
     """Tight planes of one picture: YUV420 w*h*3/2, YUV422 w*h*2, 8-bit grey w*h."""
@@ -227,6 +248,16 @@ def _origins_array(origins):
     if origins is None:
         return None
     return _int_array([int(v) for xy in origins for v in xy])
+
+
+def _float3(v):
+    """3 floats -> a host float array, or NULL for None."""
+    if v is None:
+        return None
+    v = np.asarray(v, dtype=np.float32).reshape(-1)
+    if v.shape != (3,):
+        raise ValueError("3 values, one per channel, expected")
+    return (C.c_float * 3)(*[float(x) for x in v])
 
 
 def _check(rc: int, what: str) -> None:
@@ -571,6 +602,22 @@ class BatchContext:
                                                        row_pitch, frame_pitch, alpha, _ptr_array(last_yuv),
                                                        C.c_void_p(cuda_stream or 0)),
                "rtjgpu_decode_device_rgb_window")
+
+    def decode_device_chw_window(self, d_stream: int, d_desc: int, F: int, w: int, h: int, seq_first, sel, size, origins,
+                                 kind: int, dtype: int, d_out: int, mirror=None, scale=None, bias=None, carries=None,
+                                 last_yuv=None, cuda_stream: int | None = None) -> None:
+        """rtjgpu_decode_device_chw_window: the window of frame sel[k] to d_out + k * 3 * ch * cw * CHW_ESIZE[dtype] as a
+        tight [3][ch][cw] array of dtype (CHW_*), channel c byte c of kind's pixel (CONV_RGB24 / CONV_BGR24).  mirror: S flags
+        or None; scale, bias: 3 floats each or None (1 and 0); last_yuv as for decode_device_window."""
+        S = len(seq_first) - 1
+        cw, ch = size
+        mir = None if mirror is None else _int_array([1 if m else 0 for m in mirror])
+        _check(self._L.rtjgpu_decode_device_chw_window(self._h, C.c_void_p(d_stream), C.c_void_p(d_desc), F, w, h, S,
+                                                       _int_array(seq_first), _ptr_array(carries), len(sel), _int_array(sel),
+                                                       cw, ch, _origins_array(origins), mir, kind, dtype, _float3(scale),
+                                                       _float3(bias), C.c_void_p(d_out or 0), _ptr_array(last_yuv),
+                                                       C.c_void_p(cuda_stream or 0)),
+               "rtjgpu_decode_device_chw_window")
 
     def decode_host(self, stream: np.ndarray, offsets: np.ndarray, out: np.ndarray, state: State | None = None,
                     carry: np.ndarray | None = None, flags: int = 0) -> State:

@@ -11,6 +11,7 @@
 #include <cuda_runtime.h>
 
 #include <algorithm>
+#include <cmath>
 #include <cstdlib>
 #include <cstring>
 #include <new>
@@ -365,9 +366,18 @@ struct WinIn {
     const int *origins;
 };
 
+/* A window that leaves planar and typed (rtjgpu_decode_device_chw_window), next to the RgbOut that names the converter and
+ * where slot k goes (d_rgb, frame_pitch = 3 ch cw esize, row_pitch = cw esize): the element type, and per output channel a
+ * scale and a bias (host arrays, or NULL), and per sequence whether its windows are mirrored (host array, or NULL). */
+struct ChwOut {
+    int          dtype;
+    const float *scale, *bias;
+    const int   *mirror;
+};
+
 /* What a device decode is given: the batch, its sequences, which frames it wants and where they go -- planes to d_out, or
- * packed pixels (rgb != NULL), of the whole picture or of a window (win != NULL, with a selection).  rtjgpu_scan_device
- * gives the batch alone. */
+ * packed pixels (rgb != NULL), of the whole picture or of a window (win != NULL, with a selection); a window's pixels may
+ * also leave planar and typed (chw != NULL, with rgb).  rtjgpu_scan_device gives the batch alone. */
 struct DecodeCall {
     const uint8_t           *d_stream;
     const rtjgpu_frame_desc *d_desc;
@@ -378,6 +388,7 @@ struct DecodeCall {
     const WinIn             *win = nullptr;
     uint8_t                 *d_out = nullptr;
     const RgbOut            *rgb = nullptr;
+    const ChwOut            *chw = nullptr;
 
     DecodeCall(const uint8_t *d_stream, const rtjgpu_frame_desc *d_desc, int F, int w, int h, void *stream)
         : d_stream(d_stream), d_desc(d_desc), F(F), w(w), h(h), stream((cudaStream_t)stream) {}
@@ -455,6 +466,13 @@ int run_kernels(rtjgpu_ctx *ctx, Workspace *ws, const DecodeCall &c, const CallD
         a.fused_rgb = 1;
         a.d_rgb = rgb->d_rgb; a.rgb_row_pitch = rgb->row_pitch; a.rgb_frame_pitch = rgb->frame_pitch;
         a.rgb_kind = rgb->kind; a.rgb_alpha = (unsigned)rgb->alpha & 0xFFu; a.d_last_yuv = c.q.S > 1 ? nullptr : c.q.last(0);
+    }
+    if (c.chw) {
+        a.chw = 1; a.chw_dtype = c.chw->dtype;
+        for (int k = 0; k < 3; k++) {
+            a.chw_scale[k] = c.chw->scale ? c.chw->scale[k] : 1.0f;
+            a.chw_bias[k] = c.chw->bias ? c.chw->bias[k] : 0.0f;
+        }
     }
     a.d_seq = dev.seq; a.d_carries = dev.carries; a.d_last_yuvs = dev.last_yuvs;
     /* a window: K2 of the selected frames over the rows of units the windows span; then one launch over the sequences' last
@@ -693,7 +711,16 @@ int check_batch(rtjgpu_ctx *ctx, const DecodeCall &c, bool output, int *nblk)
             if (x < 0 || y < 0 || (x & 15) || (y & 1) || x > c.w - v.cw || y > c.h - v.ch) return RTJGPU_E_ARG;
         }
     }
-    if (output && c.rgb) {
+    /* the planar typed form: its converters and element types; a u8 byte is not scaled, a float one by finite numbers only */
+    if (output && c.chw) {
+        const ChwOut &o = *c.chw;
+        if (c.rgb->kind != RTJ_CONV_RGB24 && c.rgb->kind != RTJ_CONV_BGR24) return RTJGPU_E_ARG;
+        if (o.dtype < RTJ_CHW_U8 || o.dtype > RTJ_CHW_F32) return RTJGPU_E_ARG;
+        if (o.dtype == RTJ_CHW_U8 && (o.scale || o.bias)) return RTJGPU_E_ARG;
+        for (int k = 0; k < 3; k++)
+            if ((o.scale && !std::isfinite(o.scale[k])) || (o.bias && !std::isfinite(o.bias[k]))) return RTJGPU_E_ARG;
+    }
+    if (output && c.rgb && !c.chw) {                  /* (the planar form's pitches are its own, not the caller's) */
         const RgbOut &o = *c.rgb;
         const int ow = c.win ? c.win->cw : c.w, oh = c.win ? c.win->ch : c.h;     /* the picture that leaves */
         if ((o.row_pitch & 15) || (o.frame_pitch & 15) || o.row_pitch < (size_t)ow * rtj_convert_bpp(o.kind)
@@ -717,7 +744,7 @@ int decode(rtjgpu_ctx *ctx, DecodeCall c)
     if (c.rgb) {
         if (ctx->format != RTJ_YUV420) return RTJGPU_E_FORMAT;                 /* the reference's converters are yuv420 ones */
         const int k = c.rgb->kind;
-        if (k != RTJ_CONV_RGB32 && k != RTJ_CONV_BGR32 && k != RTJ_CONV_RGB24 && k != RTJ_CONV_BGR24 && k != RTJ_CONV_RGB16)
+        if (!c.chw && k != RTJ_CONV_RGB32 && k != RTJ_CONV_BGR32 && k != RTJ_CONV_RGB24 && k != RTJ_CONV_BGR24 && k != RTJ_CONV_RGB16)
             return RTJGPU_E_FORMAT;
     }
     int rc;
@@ -737,7 +764,9 @@ int decode(rtjgpu_ctx *ctx, DecodeCall c)
         /* the sequences' origins, then the jobs of the last-frame launch: each sequence's last frame that has a last_yuv */
         std::vector<uint32_t> &ww = ctx->win_words;
         ww.clear();
-        for (int s = 0; s < c.q.S; s++) ww.push_back(RTJ_WIN(c.win->origins[2 * s], c.win->origins[2 * s + 1]));
+        const int *mirror = c.chw ? c.chw->mirror : nullptr;
+        for (int s = 0; s < c.q.S; s++)
+            ww.push_back(RTJ_WIN(c.win->origins[2 * s], c.win->origins[2 * s + 1]) | (mirror && mirror[s] ? RTJ_WIN_MIRROR : 0u));
         for (int s = 0; s < c.q.S; s++)
             if (c.q.last(s)) ww.push_back(RTJ_JOB(c.q.first[s + 1] - 1, s));
     }
@@ -1366,6 +1395,29 @@ int rtjgpu_decode_device_rgb_window(rtjgpu_ctx *ctx, const uint8_t *d_stream, co
     c.sel = &s;
     c.win = &v;
     c.rgb = &o;
+    return decode(ctx, c);
+}
+
+int rtjgpu_decode_device_chw_window(rtjgpu_ctx *ctx, const uint8_t *d_stream, const rtjgpu_frame_desc *d_desc, int F, int w, int h,
+                                    int S, const int *seq_first, const uint8_t *const *carries,
+                                    int n, const int *sel, int cw, int ch, const int *origins, const int *mirror,
+                                    int kind, int dtype, const float *scale, const float *bias,
+                                    void *d_out, uint8_t *const *last_yuv, void *cuda_stream)
+{
+    if (!seq_first) return RTJGPU_E_ARG;
+    const SelIn s{n, sel};
+    const WinIn v{cw, ch, origins};
+    /* a tight [3][ch][cw] array per slot (an unknown dtype is refused by check_batch before these are used) */
+    const size_t esize = dtype == RTJ_CHW_U8 ? 1 : dtype == RTJ_CHW_F32 ? 4 : 2;
+    const size_t row = cw > 0 ? (size_t)cw * esize : 0, frame = ch > 0 ? 3 * (size_t)ch * row : 0;
+    const RgbOut o{static_cast<uint8_t *>(d_out), row, frame, kind, 0};
+    const ChwOut t{dtype, scale, bias, mirror};
+    DecodeCall c(d_stream, d_desc, F, w, h, cuda_stream);
+    c.q.S = S; c.q.first = seq_first; c.q.carries = carries; c.q.last_yuv = last_yuv;
+    c.sel = &s;
+    c.win = &v;
+    c.rgb = &o;
+    c.chw = &t;
     return decode(ctx, c);
 }
 

@@ -71,6 +71,9 @@ extern "C" {
 #define RTJ_WIN(x, y) ((uint32_t)(x) | (uint32_t)(y) << 16)
 #define RTJ_WIN_X(v) ((v) & 0xFFFFu)
 #define RTJ_WIN_Y(v) ((v) >> 16)
+/* rtjgpu_decode_device_chw_window: the sequence's windows leave mirrored left to right.  Bit 0 of x, free since x is a
+ * multiple of 16: RTJ_WIN_X(v) / 16 is the window's first unit either way. */
+#define RTJ_WIN_MIRROR 1u
 
 #define RTJ_NUM_TABLES 257
 
@@ -195,6 +198,11 @@ typedef struct rtj_launch_args {
      * launch of the sequences' last frames, a whole-picture window that leaves as planes to d_last_yuvs */
     const uint32_t          *d_win;
     int                      win_w, win_h, win_rows, win_last;
+    /* the window leaves planar and typed (rtjgpu_decode_device_chw_window; chw == 0: packed, as rgb_kind says): slot k a
+     * tight [3][win_h][win_w] array of chw_dtype (RTJ_CHW_*) at d_rgb + k * rgb_frame_pitch, rows rgb_row_pitch bytes apart.
+     * Channel c = byte c of rgb_kind's pixel (RGB24 / BGR24), stored as fadd_rn(fmul_rn(v, chw_scale[c]), chw_bias[c]) */
+    int                      chw, chw_dtype;
+    float                    chw_scale[3], chw_bias[3];
 } rtj_launch_args;
 
 int rtj_launch_scan(const rtj_launch_args *a, void *stream);          /* returns the number of launches (>0) or -cudaError */

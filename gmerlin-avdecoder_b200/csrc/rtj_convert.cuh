@@ -7,6 +7,8 @@
 #ifndef RTJ_CONVERT_CUH
 #define RTJ_CONVERT_CUH
 
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <stdint.h>
 
 #include "rtj_common.h"
@@ -83,6 +85,64 @@ __device__ __forceinline__ void row8(const uint2 yw, const Chroma (&c)[4], uint3
         reinterpret_cast<uint2 *>(o)[1] = make_uint2(wd[2], wd[3]);
         reinterpret_cast<uint2 *>(o)[2] = make_uint2(wd[4], wd[5]);
     }
+}
+
+/* The same 8 pixels as row8 computes them, clamped, one channel at a time: 8 bytes each, pixel 0 lowest */
+struct Rgb8 { uint2 r, g, b; };
+
+__device__ __forceinline__ Rgb8 rgb8(const uint2 yw, const Chroma (&c)[4])
+{
+    int R[8], G[8], B[8];
+#pragma unroll
+    for (int x = 0; x < 8; x++) {
+        const uint32_t yb = ((x < 4 ? yw.x : yw.y) >> (8 * (x & 3))) & 0xFFu;
+        const int y = ((int)yb - 16) * KY;
+        R[x] = (y + c[x >> 1].r) >> 16;
+        G[x] = (y - c[x >> 1].g) >> 16;
+        B[x] = (y + c[x >> 1].b) >> 16;
+    }
+    auto bytes8 = [](const int (&v)[8]) {
+        return make_uint2(pack_sat(v[1], v[0], pack_sat(v[3], v[2], 0u)), pack_sat(v[5], v[4], pack_sat(v[7], v[6], 0u)));
+    };
+    return Rgb8{bytes8(R), bytes8(G), bytes8(B)};
+}
+
+/* 8 bytes in reverse order: a chunk of a mirrored window */
+__device__ __forceinline__ uint2 reverse8(uint2 v)
+{
+    return make_uint2(__byte_perm(v.y, 0u, 0x0123), __byte_perm(v.x, 0u, 0x0123));
+}
+
+/* 8 elements of one channel of a planar window (rtjgpu_decode_device_chw_window) to o: the bytes v themselves (RTJ_CHW_U8,
+ * 8 bytes), or fadd_rn(fmul_rn(v, s), b) -- two roundings, never contracted -- as binary16 / bfloat16 (16 bytes) or float32
+ * (32 bytes) */
+__device__ __forceinline__ void chw8(int dtype, uint2 v, float s, float b, uint8_t *__restrict__ o)
+{
+    if (dtype == RTJ_CHW_U8) {
+        *reinterpret_cast<uint2 *>(o) = v;
+        return;
+    }
+    float t[8];
+#pragma unroll
+    for (int x = 0; x < 8; x++)
+        t[x] = __fadd_rn(__fmul_rn((float)(((x < 4 ? v.x : v.y) >> (8 * (x & 3))) & 0xFFu), s), b);
+    if (dtype == RTJ_CHW_F32) {
+        reinterpret_cast<float4 *>(o)[0] = make_float4(t[0], t[1], t[2], t[3]);
+        reinterpret_cast<float4 *>(o)[1] = make_float4(t[4], t[5], t[6], t[7]);
+        return;
+    }
+    uint32_t p[4];
+#pragma unroll
+    for (int x = 0; x < 8; x += 2) {
+        if (dtype == RTJ_CHW_F16) {
+            const __half2 hv = __floats2half2_rn(t[x], t[x + 1]);
+            p[x >> 1] = *reinterpret_cast<const uint32_t *>(&hv);
+        } else {
+            const __nv_bfloat162 bv = __floats2bfloat162_rn(t[x], t[x + 1]);
+            p[x >> 1] = *reinterpret_cast<const uint32_t *>(&bv);
+        }
+    }
+    *reinterpret_cast<uint4 *>(o) = make_uint4(p[0], p[1], p[2], p[3]);
 }
 
 } // namespace rtjcv

@@ -530,6 +530,10 @@ struct K2Params {
      * planes, or as packed pixels; 1: the window is the whole picture and leaves as planes to last_yuvs[sequence] */
     const uint32_t *win;
     int win_w, win_h, win_last;
+    /* RGB_CHW: the window leaves planar and typed to rgb (rtj_launch_args::chw): channel c of rgb_kind's pixel, as chw_dtype,
+     * scaled and offset by chw_scale[c], chw_bias[c] */
+    int chw_dtype;
+    float chw_scale[3], chw_bias[3];
 };
 
 /* The general decoder for one block that K2's sparse classes do not take (long blocks; blocks whose last writer used
@@ -597,8 +601,9 @@ constexpr int K2_PF_LINES = 12;                   /* 128-byte lines of payload a
  */
 /* RGBK: RGB_NONE = planes leave; RTJ_CONV_RGB32 .. RTJ_CONV_RGB16 = that converter fused into the store (one kernel per
  * kind: the conversion doubles the kernel's arithmetic and wants its registers); RGB_ANY = the kind is read at run time
- * (strips of very wide pictures: not worth five more kernels) */
-constexpr int RGB_NONE = -1, RGB_ANY = 99;
+ * (strips of very wide pictures: not worth five more kernels); RGB_CHW = a window that leaves planar and typed
+ * (rtjgpu_decode_device_chw_window: WIN kernels only; the channel order and the element type are read at run time) */
+constexpr int RGB_NONE = -1, RGB_ANY = 99, RGB_CHW = 100;
 
 /* RUN: a CTA works through P.run frames in turn (below); false: one frame, and none of the run's bookkeeping is compiled in */
 /* RES: a warp reserves its places in K2b's queue with one request per row (streams in which most blocks go that way: a quality
@@ -619,6 +624,8 @@ rtj_idct_kernel(const K2Params P)
     static_assert(!RGB || FMT == 0, "the fused converters are the reference's yuv420 ones");
     static_assert(!SEL || (!RUN && !RES), "a selection is decoded one frame per CTA, without K2b's reservations");
     static_assert(!WIN || (SEL && !SINGLE), "a window is a selection, decoded in strips");
+    constexpr bool CHW = RGBK == RGB_CHW;
+    static_assert(!CHW || WIN, "the planar typed form is a window's");
     constexpr bool GENERAL = RGB || WIN;                     /* HARD blocks decoded in this kernel, not queued for K2b */
     constexpr int THREADS = WARPS * 32;
     typedef Geo<FMT> G;
@@ -921,7 +928,48 @@ rtj_idct_kernel(const K2Params P)
     const int lw = G::UNIT_W * mbs;                              /* luma bytes per strip row */
     bool planes_leave = true, luma_leaves = true;
     uint8_t *last_planes = P.last_yuv;                          /* RGB: where the frame leaves as planes too, if it does */
-    if (RGB) {
+    if (CHW) {
+        /* The window's pixels as the RGB branch below makes them (RGB24 / BGR24), planar: a thread takes 8 pixels of two rows,
+         * and stores each row's three channels, 8 elements each (8-, 16- or 2 x 16-byte stores, contiguous across the warp).
+         * Mirrored, a chunk's bytes are reversed before they are converted and the chunk goes to the mirrored column. */
+        using namespace rtjcv;
+        const int chunks = lw >> 3;
+        const uint8_t *tU = tile + G::CHROMA_AT * mbs, *tV = tU + 64 * mbs;
+        const int top = my * 16 - wy;
+        const int rp0 = max(0, -top) >> 1, rp1 = min(16, P.win_h - top) >> 1;
+        const bool mirror = (worg & RTJ_WIN_MIRROR) != 0u;
+        const int dtype = P.chw_dtype;
+        const int es = dtype == RTJ_CHW_U8 ? 1 : dtype == RTJ_CHW_F32 ? 4 : 2;
+        const size_t rowp = P.rgb_row_pitch, planep = rowp * (size_t)P.win_h;
+        const int cr = P.rgb_kind == RTJ_CONV_BGR24 ? 2 : 0;        /* the channel red goes to; blue to the other end */
+        uint8_t *const base = P.rgb + (size_t)RTJ_JOB_SLOT(job) * P.rgb_frame_pitch;
+        uint8_t *const pr = base + cr * planep, *const pg = base + planep, *const pb = base + (2 - cr) * planep;
+        const float sr = P.chw_scale[cr], sg = P.chw_scale[1], sb = P.chw_scale[2 - cr];
+        const float br = P.chw_bias[cr], bg = P.chw_bias[1], bb = P.chw_bias[2 - cr];
+        const int items = (rp1 - rp0) * chunks;
+        for (int item = tid; item < items; item += THREADS) {
+            const int rp = rp0 + item / chunks, c = item - (rp - rp0) * chunks;
+            const uint2 y0 = *reinterpret_cast<const uint2 *>(tile + (2 * rp) * lw + c * 8);
+            const uint2 y1 = *reinterpret_cast<const uint2 *>(tile + (2 * rp + 1) * lw + c * 8);
+            const uint32_t ub = *reinterpret_cast<const uint32_t *>(tU + rp * (lw >> 1) + c * 4);
+            const uint32_t vb = *reinterpret_cast<const uint32_t *>(tV + rp * (lw >> 1) + c * 4);
+            Chroma ct[4];
+#pragma unroll
+            for (int k = 0; k < 4; k++) ct[k] = chroma_terms((ub >> (8 * k)) & 0xFFu, (vb >> (8 * k)) & 0xFFu);
+            const int x = (mx0 - wx) * 16 + c * 8;                  /* the chunk's first column in the window */
+            const size_t col = (size_t)(mirror ? P.win_w - 8 - x : x) * es;
+#pragma unroll
+            for (int k = 0; k < 2; k++) {
+                Rgb8 v = rgb8(k ? y1 : y0, ct);
+                if (mirror) { v.r = reverse8(v.r); v.g = reverse8(v.g); v.b = reverse8(v.b); }
+                const size_t off = (size_t)(top + 2 * rp + k) * rowp + col;   /* strip row 2 rp + k is window row top + 2 rp + k */
+                chw8(dtype, v.r, sr, br, pr + off);
+                chw8(dtype, v.g, sg, bg, pg + off);
+                chw8(dtype, v.b, sb, bb, pb + off);
+            }
+        }
+        planes_leave = false;                                   /* the last frames have a launch of their own */
+    } else if (RGB) {
         /* The strip -- 16 luma rows, 8 rows of Cb and of Cr: exactly what the reference's converters read for 16 output
          * rows (lib/RTjpeg.c:3123-3190) -- leaves as packed pixels.  A thread takes 8 pixels of two rows (one chroma row):
          * aligned 8- / 4-byte shared loads, 16- / 8-byte global stores, contiguous across the warp. */
@@ -1433,7 +1481,7 @@ cudaError_t k2_launch(K2Params &P, int grid_x, int F, cudaStream_t st)
     return e != cudaSuccess ? e : cudaGetLastError();
 }
 
-/* a window of a selection (P.win_w != 0): the strip kernels, one frame per CTA; RGBK is RGB_NONE or RGB_ANY */
+/* a window of a selection (P.win_w != 0): the strip kernels, one frame per CTA; RGBK is RGB_NONE, RGB_ANY or RGB_CHW */
 template <int FMT, int RGBK>
 cudaError_t k2_launch_win(K2Params &P, int grid_x, int njobs, cudaStream_t st)
 {
@@ -1473,6 +1521,12 @@ extern "C" int rtj_idct_init(void)
     if (e == cudaSuccess) e = k2_attrs<0, RTJ_CONV_RGB16>();
     if (e == cudaSuccess) e = k2_attrs<1, RGB_NONE>();
     if (e == cudaSuccess) e = k2_attrs<2, RGB_NONE>();
+    if (e == cudaSuccess)
+        e = cudaFuncSetAttribute(rtj_idct_kernel<false, 0, 4, RGB_CHW, false, false, true, true>,
+                                 cudaFuncAttributeMaxDynamicSharedMemorySize, (int)idct_smem_bytes(IDCT_MAX_MB, 0, 3));
+    if (e == cudaSuccess)
+        e = cudaFuncSetAttribute(rtj_idct_kernel<false, 0, 3, RGB_CHW, false, false, true, true>,
+                                 cudaFuncAttributeMaxDynamicSharedMemorySize, (int)idct_smem_bytes(IDCT_MAX_MB, 0, 3));
     if (e != cudaSuccess) return (int)e;
     int dev = 0;
     if ((e = cudaGetDevice(&dev)) != cudaSuccess) return (int)e;
@@ -1527,11 +1581,14 @@ extern "C" int rtj_launch_idct(const rtj_launch_args *a, void *stream)
     P.rgb_kind = a->rgb_kind; P.rgb_alpha = a->rgb_alpha & 0xFFu; P.last_yuv = a->d_last_yuv;
     P.seq = a->d_seq; P.carries = a->d_carries; P.last_yuvs = a->d_last_yuvs;
     P.win = a->d_win; P.win_w = a->win_w; P.win_h = a->win_h; P.win_last = a->win_last;
+    P.chw_dtype = a->chw_dtype;
+    for (int c = 0; c < 3; c++) { P.chw_scale[c] = a->chw_scale[c]; P.chw_bias[c] = a->chw_bias[c]; }
     if (a->win_w) {
         /* a window: strips cut from the window's width, over the most rows of units any sequence's window spans */
         if (!a->d_jobs || !a->d_seq || a->win_rows <= 0) return (int)cudaErrorInvalidValue;
         P.seg_mb = idct_seg_mb(RTJ_FMT_UNITS_X(fmt, a->win_w), &P.nstrips);
         const int gx = P.nstrips * a->win_rows;
+        if (a->chw && !a->win_last) return fmt == 0 ? (int)k2_launch_win<0, RGB_CHW>(P, gx, nf, st) : (int)cudaErrorInvalidValue;
         if (a->fused_rgb && !a->win_last) return fmt == 0 ? (int)k2_launch_win<0, RGB_ANY>(P, gx, nf, st) : (int)cudaErrorInvalidValue;
         return (int)(fmt == 0 ? k2_launch_win<0, RGB_NONE>(P, gx, nf, st) : fmt == 1 ? k2_launch_win<1, RGB_NONE>(P, gx, nf, st)
                                                                        : k2_launch_win<2, RGB_NONE>(P, gx, nf, st));

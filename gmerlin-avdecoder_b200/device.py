@@ -138,6 +138,53 @@ def decode_rgb_window(ctx: capi.BatchContext, b: DeviceBatch, seq_first, sel, si
     return out
 
 
+# the element types of decode_chw_window: torch dtype -> RTJ_CHW_*
+CHW_DTYPES = {torch.uint8: capi.CHW_U8, torch.float16: capi.CHW_F16, torch.bfloat16: capi.CHW_BF16,
+              torch.float32: capi.CHW_F32}
+CHW_ORDERS = {"rgb": capi.CONV_RGB24, "bgr": capi.CONV_BGR24}
+
+
+def decode_chw_window(ctx: capi.BatchContext, b: DeviceBatch, seq_first, sel, size, origins, dtype=torch.float16,
+                      mean=None, std=None, scale=None, bias=None, order: str = "rgb", mirror=None, carries=None, last=None,
+                      out: torch.Tensor | None = None, stream: torch.cuda.Stream | None = None) -> torch.Tensor:
+    """rtjgpu_decode_device_chw_window: decode_rgb_window straight to a model's input.  Frame sel[k] goes to row k of a
+    tight [n, 3, ch, cw] tensor of dtype (uint8, float16, bfloat16 or float32), channels in `order` ("rgb" or "bgr").
+    Floats are v * scale[c] + bias[c] of the byte v, two float32 roundings; mean and std (torchvision's (v / 255 - mean) /
+    std) stand for capi.normalize_coefficients(mean, std) and exclude scale and bias.  uint8 takes neither.  mirror: one
+    flag for every sequence, or S flags -- that sequence's windows mirrored left to right.  carries, last and origins as
+    for decode_window; out, if given, must be exactly the result's shape and dtype, contiguous.  YUV420 batches only."""
+    if dtype not in CHW_DTYPES:
+        raise ValueError(f"decode_chw_window: dtype {dtype} is not one of uint8, float16, bfloat16, float32")
+    if order not in CHW_ORDERS:
+        raise ValueError(f"decode_chw_window: order {order!r} is not 'rgb' or 'bgr'")
+    if (mean is None) != (std is None):
+        raise ValueError("decode_chw_window: mean and std go together")
+    if mean is not None and (scale is not None or bias is not None):
+        raise ValueError("decode_chw_window: mean/std and scale/bias exclude each other")
+    if mean is not None:
+        scale, bias = capi.normalize_coefficients(mean, std)
+    if dtype == torch.uint8 and (scale is not None or bias is not None):
+        raise ValueError("decode_chw_window: uint8 output is not scaled")
+    S = len(seq_first) - 1
+    sel, cw, ch, origins, last_ptrs = _window_args(seq_first, sel, size, origins, last)
+    if mirror is not None:
+        mirror = [bool(mirror)] * S if np.ndim(mirror) == 0 else [bool(m) for m in mirror]
+        if len(mirror) != S:
+            raise ValueError(f"decode_chw_window: {len(mirror)} mirror flags for {S} sequences")
+    shape = (len(sel), 3, ch, cw)
+    if out is not None and (out.dtype != dtype or tuple(out.shape) != shape or not out.is_contiguous()):
+        raise ValueError(f"decode_chw_window: out must be a contiguous {tuple(shape)} tensor of {dtype}")
+    st = stream if stream is not None else torch.cuda.current_stream(b.stream.device)
+    if out is None:
+        out = torch.empty(shape, dtype=dtype, device=b.stream.device)
+    ctx.set_format(b.fmt)
+    ptrs = None if carries is None else [None if c is None else c.data_ptr() for c in carries]
+    ctx.decode_device_chw_window(b.stream.data_ptr(), b.desc.data_ptr(), b.F, b.w, b.h, list(seq_first), sel, (cw, ch),
+                                 origins, CHW_ORDERS[order], CHW_DTYPES[dtype], out.data_ptr() if len(sel) else None,
+                                 mirror, scale, bias, ptrs, last_ptrs, st.cuda_stream)
+    return out
+
+
 def encode_sequences(ctx: capi.BatchContext, pictures, encoders, w: int, h: int, fmt: int = 0,
                      stream: torch.cuda.Stream | None = None):
     """rtjgpu_encode_device_seq: pictures a list of S uint8 device tensors (or views), each one sequence's consecutive

@@ -46,6 +46,12 @@ typedef void RTjpeg_t;
 #define RTJ_CONV_RGB8         5   /* RTjpeg_yuv420rgb8, :3477: the luma plane */
 #define RTJ_CONV_YUV422_RGB24 6   /* RTjpeg_yuv422rgb24, :3077 */
 
+/* Element types of rtjgpu_decode_device_chw_window's planar output. */
+#define RTJ_CHW_U8   0            /* the converter's byte */
+#define RTJ_CHW_F16  1            /* IEEE binary16 */
+#define RTJ_CHW_BF16 2            /* bfloat16 */
+#define RTJ_CHW_F32  3            /* IEEE binary32 */
+
 /* Fixed packet header length, include/RTjpeg.h:139 (RTJPEG_HEADER_SIZE). */
 #define RTJPEG_B200_HEADER_BYTES 12
 
@@ -419,6 +425,23 @@ int  rtjgpu_decode_device_rgb_window(rtjgpu_ctx *ctx, const uint8_t *d_stream, c
                                      int n, const int *sel, int cw, int ch, const int *origins,
                                      int kind, uint8_t *d_rgb, size_t row_pitch, size_t frame_pitch, int alpha,
                                      uint8_t *const *last_yuv, void *cuda_stream);
+/* STRAIGHT TO A MODEL'S INPUT.  The batch, selection, window, origins, carries and last_yuv of rtjgpu_decode_device_rgb_window,
+ * with its rules and error codes; what leaves is planar and typed.  Slot k is a tight [3][ch][cw] array of dtype (RTJ_CHW_U8,
+ * F16, BF16 or F32: 1, 2, 2 or 4 bytes an element) at d_out + k * 3 * ch * cw * esize; d_out 16-byte aligned, NULL only when
+ * n = 0.  kind is RTJ_CONV_RGB24 or RTJ_CONV_BGR24: channel c is byte c of that converter's pixel, v (0..255), bit for bit
+ * what rtjgpu_decode_device_rgb_window writes.  RTJ_CHW_U8 stores v, and scale and bias must be NULL.  The float types store
+ * t = fadd_rn(fmul_rn((float)v, scale[c]), bias[c]) -- two float32 roundings, no FMA -- as float32, or rounded to nearest even
+ * to binary16 or bfloat16 (overflow to +-inf and subnormals as that rounding gives them).  scale and bias are HOST arrays of 3
+ * floats indexed by output channel, read before the call returns; NULL means 1 and 0.  mirror is a HOST array of S ints, or
+ * NULL: mirror[s] != 0 mirrors every window of sequence s left to right (output column j is window column cw - 1 - j; the
+ * origin still says where the window lies).  RTJGPU_E_ARG also for a dtype or kind other than these, a scale or bias on
+ * RTJ_CHW_U8, a scale or bias that is not finite, or a misaligned d_out; RTJGPU_E_FORMAT on a context that is not RTJ_YUV420.
+ * Asynchronous on cuda_stream. */
+int  rtjgpu_decode_device_chw_window(rtjgpu_ctx *ctx, const uint8_t *d_stream, const rtjgpu_frame_desc *d_desc, int F, int w, int h,
+                                     int S, const int *seq_first, const uint8_t *const *carries,
+                                     int n, const int *sel, int cw, int ch, const int *origins, const int *mirror,
+                                     int kind, int dtype, const float *scale, const float *bias,
+                                     void *d_out, uint8_t *const *last_yuv, void *cuda_stream);
 
 /* Host-buffer decode: packets in host memory in, frames in host memory out.
  * The batch is cut into chunks that move through pinned staging buffers with
