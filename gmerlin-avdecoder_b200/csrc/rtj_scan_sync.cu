@@ -322,17 +322,26 @@ __device__ __noinline__ bool walk_repair(const SySeg sg, uint16_t *bits16, int p
 }
 
 /* The 32-bit entry of a block (rtj_common.h): head = its first four bytes (DC, token 1, 2, 3), last = its last byte,
- * dl = its length, off = its offset in the payload. */
+ * dl = its length, off = its offset in the payload.  The entry loop makes some 76 of them per lane and frame, so every
+ * instruction here counts: the kernel is bound by the ALU pipe. */
 __device__ __forceinline__ uint32_t sy_entry(uint32_t head, uint32_t last, int dl, int off, int bt8 = 0)
 {
-    /* positions >= eob are zero: a final run of n zeros ends at 64, so it starts at 64 - n (bt8 = 63: no tokens at all) */
-    const int eob = bt8 >= 63 ? 64 : (last - 64u) < 64u ? max(127 - (int)last, dl - 1) : 64;
-    const uint32_t t1 = (head >> 8) & 0xFFu, t2 = (head >> 16) & 0xFFu;
-    const uint32_t c1 = (eob >= 2 && (t1 - 64u) >= 64u) ? t1 : 0u;
-    const uint32_t c2 = (eob >= 3 && (t2 - 64u) >= 64u) ? t2 : 0u;
-    const uint32_t e_inl = RTJ_ENT_INLINE_BIT | (head & 0xFFu) | (c1 << 8) | (c2 << 16);
+    /* positions >= eob are zero: a final run token (64..127) of n zeros ends at 64, so it starts at 64 - n = 127 - last;
+     * any other last byte: 64 (bt8 = 63: no tokens at all).  Taken as unsigned, 127 - last is 0..63 for a run token, 64..127
+     * for a byte below 64 and above 2^31 for one above 127, so one clamp does the choice (dl - 1 <= 63: a block is at most
+     * 64 bytes) */
+    uint32_t eob = min(max(127u - last, (uint32_t)(dl - 1)), 64u);
+    if (bt8 >= 63) eob = 64u;
+    /* inline (eob <= 3): the DC, and tokens 1 and 2 where they lie in front of eob and are not run tokens.  Byte-wise, bit 7
+     * of x says "drop this byte": in bytes 1 and 2, ~head & (head << 1) marks a token 01xxxxxx, and 0x81 - eob / 0x82 - eob
+     * (no borrow for eob <= 3) one at or behind eob; byte 0 reads 0x80.  PRMT spreads those bits over their bytes
+     * (selector nibbles 9, A: sign of byte 1, 2; 8: byte 0's, dropping token 3; 4: zero, keeping the DC). */
+    const uint32_t x = (~head & (head << 1)) | (0x00828180u - eob * 0x00010100u);
+    uint32_t drop;
+    asm("prmt.b32 %0, %1, 0, 0x8A94;" : "=r"(drop) : "r"(x));
+    const uint32_t e_inl = RTJ_ENT_INLINE_BIT | (head & ~drop);
     const uint32_t e_gen = RTJ_ENT(off, eob);
-    return (head & 0xFFu) == 0xFFu ? RTJ_ENT_SKIP : (bt8 == 0 && eob <= 3 ? e_inl : e_gen);      /* 0xFF: a skipped block */
+    return (head & 0xFFu) == 0xFFu ? RTJ_ENT_SKIP : (bt8 == 0 && eob <= 3u ? e_inl : e_gen);      /* 0xFF: a skipped block */
 }
 
 } // namespace
@@ -508,10 +517,19 @@ rtj_scan_sync_kernel(const uint8_t *__restrict__ stream, const rtjgpu_frame_desc
 
         /* ---- emit: the list of starts (every lane its chunk's), then one block per thread ---- */
         const int nemit = min(total, nblk - nb0);
-        int myskips = 0, lastend = -1;
+        int myskips = 0;
         const uint32_t *gw = reinterpret_cast<const uint32_t *>(gbase + seg0);
         const uint8_t *gb = gbase + seg0;
+        const int offb = seg0 - mis;                                   /* a block's offset in the payload less its start */
+#ifdef SY_AB_COUNT_ONLY
+        /* (A/B builds only: the kernel stops after the count -- no list of starts, no entries but a harmless one per block,
+         * stored as the entry loop stores them -- to time what the emit stage costs) */
+        for (int b = tid; b < nemit; b += SY_THREADS) out[nb0 + b] = RTJ_ENT(0, 1);
+        if (tid == 0) sh.consumed = len;
+        for (int lo = 0; lo < 0; lo += SY_STAGE) {
+#else
         for (int lo = 0; lo < nemit; lo += SY_STAGE) {
+#endif
             const int n = min(SY_STAGE, nemit - lo);
             {
                 /* One start per turn, the same instructions for every lane whatever its words hold (nothing to diverge on):
@@ -537,38 +555,45 @@ rtj_scan_sync_kernel(const uint8_t *__restrict__ stream, const rtjgpu_frame_desc
             }
             if (tid == 0 && lo + n == total) sh.starts[n] = (uint16_t)sh.sentinel;
             __syncthreads();
+            /* the payload read so far ends where the list's last block ends: starts[n] (the sentinel, or the start behind it) */
+            if (tid == 0 && lo + n == nemit) sh.consumed = max(sh.consumed, offb + (int)sh.starts[n]);
             /* four blocks a thread and turn: the loads of all four are under way before any is used (the payload comes
              * from L2 by now: several hundred clocks) */
             uint32_t *op = out + nb0 + lo;
             constexpr int U = 4;
-            for (int k = tid; k < n; k += U * SY_THREADS) {
+            /* whole: all four blocks lie in the list (every turn but a thread's last) -- no clamps, no tests */
+            auto emit4 = [&](const int k, const bool whole) {
                 int qq[U], nx[U];
                 uint32_t h0[U], h1[U], lb[U];
 #pragma unroll
                 for (int u = 0; u < U; u++) {
-                    const int ku = min(k + u * SY_THREADS, n - 1);
+                    const int ku = whole || u == 0 ? k + u * SY_THREADS : min(k + u * SY_THREADS, n - 1);
                     qq[u] = sh.starts[ku];
                     nx[u] = sh.starts[ku + 1];
                 }
 #pragma unroll
                 for (int u = 0; u < U; u++) {
-                    const uint32_t *wp = gw + (qq[u] >> 2);
+                    const uint32_t *wp = gw + ((unsigned)qq[u] >> 2);
                     h0[u] = __ldg(wp);
                     h1[u] = __ldg(wp + 1);
-                    lb[u] = __ldg(gb + nx[u] - 1);
+                    lb[u] = __ldg(gb + (unsigned)nx[u] - 1);
                 }
 #pragma unroll
                 for (int u = 0; u < U; u++) {
                     /* raw prefix: the block's place in its unit tells its plane, and that the prefix's length */
                     const int bt8 = RAW ? ((nb0 + lo + k + u * SY_THREADS) % unit < unit_luma ? lb8 : cb8) : 0;
-                    const uint32_t e = sy_entry(__funnelshift_r(h0[u], h1[u], (unsigned)(qq[u] & 3) * 8), lb[u], nx[u] - qq[u], seg0 + qq[u] - mis, bt8);
-                    if (k + u * SY_THREADS < n) {
+                    /* (the funnel shift takes its count modulo 32: qq * 8 is (qq & 3) * 8) */
+                    const uint32_t head = __funnelshift_r(h0[u], h1[u], (unsigned)qq[u] * 8u);
+                    const uint32_t e = sy_entry(head, lb[u], nx[u] - qq[u], qq[u] + offb, bt8);
+                    if (whole || k + u * SY_THREADS < n) {
                         op[k + u * SY_THREADS] = e;
-                        myskips += e == RTJ_ENT_SKIP ? 1 : 0;
-                        lastend = max(lastend, nx[u]);
+                        if ((head & 0xFFu) == 0xFFu) myskips++;                    /* e == RTJ_ENT_SKIP */
                     }
                 }
-            }
+            };
+            int k = tid;
+            for (; k + (U - 1) * SY_THREADS < n; k += U * SY_THREADS) emit4(k, true);
+            if (k < n) emit4(k, false);
             /* the payload's last bytes: a block that starts on one of the last three, or that is cut short, must see 0x7F
              * behind the payload, not what follows the packet in memory -- at most the list's last four blocks */
             if (lo + n == total && lim < climit + SY_LA) {
@@ -585,7 +610,7 @@ rtj_scan_sync_kernel(const uint8_t *__restrict__ stream, const rtjgpu_frame_desc
                             head = (head & m) | (0x7F7F7F7Fu & ~m);
                         }
                         if (nx > lim) last = 0x7Fu;                                    /* the last block, cut short */
-                        op[k] = sy_entry(head, last, nx - qq, seg0 + qq - mis, RAW ? ((nb0 + lo + k) % unit < unit_luma ? lb8 : cb8) : 0);
+                        op[k] = sy_entry(head, last, nx - qq, qq + offb, RAW ? ((nb0 + lo + k) % unit < unit_luma ? lb8 : cb8) : 0);
                     }
                 }
             }
@@ -593,14 +618,8 @@ rtj_scan_sync_kernel(const uint8_t *__restrict__ stream, const rtjgpu_frame_desc
         }
         {
 #pragma unroll
-            for (int o = 16; o; o >>= 1) {
-                myskips += __shfl_xor_sync(FULL, myskips, o);
-                lastend = max(lastend, __shfl_xor_sync(FULL, lastend, o));
-            }
-            if (lane == 0) {
-                if (myskips) atomicAdd(&sh.skips, myskips);
-                if (lastend >= 0) atomicMax(&sh.consumed, seg0 + lastend - mis);
-            }
+            for (int o = 16; o; o >>= 1) myskips += __shfl_xor_sync(FULL, myskips, o);
+            if (lane == 0 && myskips) atomicAdd(&sh.skips, myskips);
             if (tid == 0) sh.nb = nb0 + total;
         }
         __syncthreads();
